@@ -7,16 +7,18 @@ of synthetic test queries with the fitted model resident in HBM.  The default wo
 BASELINE.json names for the 1/2/4/8-GPU metric and the N = 32k fit): 32 768 train rows, 256-dim encodings,
 depth-3 NNGP, 131 072 test rows per GPU (1M / 8).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c5] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c5] [--impl reference] [--dump-outputs DIR]
 
 N>1 is launched by torchrun (one rank per GPU, NCCL): rank 0 fits, the fitted state is broadcast once (packed
 lower triangle, nngp_b200.dist.broadcast_fit), each rank predicts its own shard of test rows (weak scaling:
 per-GPU rows fixed), no data-path collective.  After that timed region rank 0 also measures the IN-PROCESS
 multi-GPU path (one handle with n_gpus = N: peer-to-peer replication + row split behind the same C-ABI call the
 reference's single-process callers make) and reports it under "in_process".
-Rank 0 prints ONE JSON line.  `--impl reference` times the CPU restatement of the reference path
-(oracle/nngp_oracle.py: numpy/scipy -> OpenBLAS/LAPACK, the library class jaxlib calls) on all the box's host
-cores; jax / neural-tangents are not installable, so no `oracle/_ref` exists (DESIGN.md).
+Rank 0 prints ONE JSON line.  `--dump-outputs DIR` also writes what the last timed step returned (posterior mean and
+variance of every rank's test rows, in rank order) as float64 DIR/mean.npy and DIR/var.npy.  `--impl reference` times
+the CPU restatement of the reference path (oracle/nngp_oracle.py: numpy/scipy -> OpenBLAS/LAPACK, the library class
+jaxlib calls) on all the box's host cores; jax / neural-tangents are not installable, so no `oracle/_ref` exists
+(DESIGN.md).
 """
 from __future__ import annotations
 
@@ -65,7 +67,27 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--slices", type=int, default=7, help="digit planes of the int8 variance side record (0 = skip it)")
     ap.add_argument("--no-extras", action="store_true", help="skip the C2 side record / fit_n32k / in-process multi-GPU legs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the posterior mean and variance of the last timed step to DIR/mean.npy, DIR/var.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_MAX_ROWS = 1 << 21     # 2 float64 arrays of at most 2M rows: 32 MiB per dump
+
+
+def dump_outputs(out_dir: str, mean: np.ndarray, var: np.ndarray) -> None:
+    """float64 mean.npy / var.npy of one timed step, in test-row order.  The inputs are seeded, so two builds run with
+    the same arguments can be compared output for output.  Above DUMP_MAX_ROWS rows the same fixed, seeded sample of
+    rows (ascending) is written for every run."""
+    if mean.shape[0] > DUMP_MAX_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(mean.shape[0], DUMP_MAX_ROWS, replace=False))
+        mean, var = mean[rows], var[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "mean.npy"), np.ascontiguousarray(mean, dtype=np.float64))
+    np.save(os.path.join(out_dir, "var.npy"), np.ascontiguousarray(var, dtype=np.float64))
 
 
 def make_config(workload: str, world: int) -> dict:
@@ -154,8 +176,10 @@ def run_reference(args):
     times = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        fit.predict(xte)
+        mean, var = fit.predict(xte)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, mean, var)
     sec = sum(times) / len(times)
     val = rows / sec
     sample = (f"oracle (numpy/scipy -> OpenBLAS, {blas_threads()} BLAS threads, {oracle.THREADS} threads for the "
@@ -364,7 +388,17 @@ def run_b200(args):
 
     kept = {}
     ms_total, ms_e2e, e2e_steps, st, st_e2e, clocks = _time_predict(torch, dist, world, h, local, xte_host, args.steps, warmup,
-                                                                    sample_clocks=(rank == 0), keep=kept if rank == 0 else None)
+                                                                    sample_clocks=(rank == 0),
+                                                                    keep=kept if rank == 0 or args.dump_outputs else None)
+    if args.dump_outputs:
+        outs = [kept["mean"], kept["var"]]
+        if world > 1:                     # every rank's shard of test rows, in rank order
+            for i, a in enumerate(outs):
+                parts = [torch.empty(t_rank, dtype=torch.float64, device="cuda") for _ in range(world)]
+                dist.all_gather(parts, torch.from_numpy(a).cuda())
+                outs[i] = torch.cat(parts).cpu().numpy()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, *outs)
 
     sliced = None
     if args.slices > 0 and not args.no_extras:

@@ -1,16 +1,19 @@
 """CPU: the reference arm of bench.py (the CPU restatement timed as the baseline) honours the output contract:
-exactly one JSON line on stdout with the agreed keys.  The B200 arm needs a GPU and is exercised by the driver."""
+exactly one JSON line on stdout with the agreed keys.  One GPU test runs the B200 arm at C2 and checks what it dumps."""
 import json
 import subprocess
 import sys
 from pathlib import Path
 
+import numpy as np
+import pytest
+
 ROOT = Path(__file__).resolve().parents[1]
 
 
-def test_reference_arm_prints_one_json_line():
+def test_reference_arm_prints_one_json_line(tmp_path):
     r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
-                        "--workload", "c2"],
+                        "--workload", "c2", "--dump-outputs", str(tmp_path)],
                        capture_output=True, text=True, timeout=600, cwd=str(ROOT))
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
@@ -24,6 +27,29 @@ def test_reference_arm_prints_one_json_line():
     assert cb["blas_threads"] in (-1, cb["cores"]) and cb["rows_per_step"] == 2048
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
     assert e2e["value"] == d["value"] and e2e["h2d_bytes_per_step"] == 0 and e2e["d2h_bytes_per_step"] == 0
+    mean, var = np.load(tmp_path / "mean.npy"), np.load(tmp_path / "var.npy")
+    assert mean.dtype == var.dtype == np.float64 and mean.shape == var.shape == (2048,)
+    assert np.all(np.isfinite(mean)) and np.all(var > 0)
+
+
+@pytest.mark.gpu
+def test_b200_arm_dumps_the_last_timed_step(tmp_path):
+    """--dump-outputs writes what the timed path returned: the posterior of the seeded C2 test rows, bit for bit what a
+    fresh handle predicts for them; --steps sets the number of timed steps."""
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--workload", "c2", "--steps", "2", "--warmup", "1",
+                        "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600, cwd=str(ROOT))
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads(r.stdout)
+    assert d["steps"] == 2 and d["config"]["test_rows_per_gpu"] == 65536
+    mean, var = np.load(tmp_path / "mean.npy"), np.load(tmp_path / "var.npy")
+    assert mean.dtype == var.dtype == np.float64 and mean.shape == var.shape == (65536,)
+    from nngp_b200 import _lib, synth
+    x = synth.encodings(8192, 128, 1)
+    h = _lib.Handle(depth=2, diag_reg=1e-3)
+    h.fit(x, synth.labels(x))
+    m, v = h.predict(synth.encodings(65536, 128, 2))
+    assert np.array_equal(mean, m) and np.array_equal(var, v)
 
 
 def test_reference_arm_keeps_all_blas_threads_under_torchrun_env():
