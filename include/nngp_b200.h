@@ -143,6 +143,11 @@ NNGP_API void* nngp_get_stream(nngp_handle* h);
  * live via predict_fn: train.py:157-158, estimator.py:66-67.
  * [nt: stax._inputs_to_kernel -> Dense -> Relu(ABRelu 0,1; arctan2 form) -> Dense]
  * x1: M x D, x2: N2 x D (NULL => x2 = x1, N2 ignored), k_out: M x N2.
+ *
+ * Accepted input range (nngp_kernel, nngp_fit, nngp_append_fit, nngp_predict): every element finite, and every
+ * row's layer-0 diagonal q = sigma_w^2 |x|^2 / D + sigma_b^2 below 2^512, so that q q' is a finite double;
+ * anything else is NNGP_EINVAL.  There is no lower bound: rows down to the subnormal range (and zero rows) are
+ * accepted, but an entry whose q, q q' or k^2 is subnormal carries fewer significant bits.
  */
 NNGP_API int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2_or_null, int64_t N2,
                 int64_t D, double* k_out);

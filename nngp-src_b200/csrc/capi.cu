@@ -983,6 +983,14 @@ int check_finite_async(nngp_handle* h, const double* x, int64_t ld, int64_t rows
   return NNGP_OK;
 }
 
+// flags[1] after check_finite_async (bit 0) and row_sqnorm_kernel with range_flag (bit 1) -> the caller's error
+int input_error(nngp_handle* h, int flag, const char* who, const char* what) {
+  if (flag & 1) return fail(h, NNGP_EINVAL, "%s: non-finite value in %s", who, what);
+  return fail(h, NNGP_EINVAL,
+              "%s: %s out of range: a row's layer-0 kernel diagonal sigma_w^2 |x|^2 / D + sigma_b^2 reaches 2^512 "
+              "(the kernel needs q q' < 2^1024)", who, what);
+}
+
 int bind_device(nngp_handle* h) {
   CK(cudaSetDevice(h->device));
   return NNGP_OK;
@@ -1414,7 +1422,7 @@ int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2, i
   CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
   CKR(upload_matrix(h, x1, M, D, h->ka.as<double>(), ldx));
   CKR(check_finite_async(h, h->ka.as<double>(), ldx, M, D));
-  row_sqnorm_kernel<<<(unsigned)((M * 32 + 255) / 256), 256, 0, h->stream>>>(h->ka.as<double>(), ldx, (int)M, (int)D, sw2, sb2, h->kqa.as<double>());
+  row_sqnorm_kernel<<<(unsigned)((M * 32 + 255) / 256), 256, 0, h->stream>>>(h->ka.as<double>(), ldx, (int)M, (int)D, sw2, sb2, h->kqa.as<double>(), h->flags.as<int>() + 1);
   h->st.kernel_launches++;
   const double* bptr = h->ka.as<double>();
   const double* qb = h->kqa.as<double>();
@@ -1423,7 +1431,7 @@ int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2, i
     CKR(ensure(h, h->kqb, (size_t)Nn * 8));
     CKR(upload_matrix(h, x2, Nn, D, h->kb.as<double>(), ldx));
     CKR(check_finite_async(h, h->kb.as<double>(), ldx, Nn, D));
-    row_sqnorm_kernel<<<(unsigned)((Nn * 32 + 255) / 256), 256, 0, h->stream>>>(h->kb.as<double>(), ldx, (int)Nn, (int)D, sw2, sb2, h->kqb.as<double>());
+    row_sqnorm_kernel<<<(unsigned)((Nn * 32 + 255) / 256), 256, 0, h->stream>>>(h->kb.as<double>(), ldx, (int)Nn, (int)D, sw2, sb2, h->kqb.as<double>(), h->flags.as<int>() + 1);
     h->st.kernel_launches++;
     bptr = h->kb.as<double>();
     qb = h->kqb.as<double>();
@@ -1442,7 +1450,7 @@ int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2, i
   CK(cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   flush_class_events(h);
-  if (flags[1]) return fail(h, NNGP_EINVAL, "nngp_kernel: non-finite value in the inputs");
+  if (flags[1]) return input_error(h, flags[1], "nngp_kernel", "the inputs");
   return NNGP_OK;
 }
 
@@ -1479,7 +1487,7 @@ static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train
   CKR(check_finite_async(h, alpha, 1, N, 1));
 
   StageTimer t_gram(h, &h->st.fit_gram_ms);
-  row_sqnorm_kernel<<<(unsigned)((N * 32 + 255) / 256), 256, 0, h->stream>>>(X, h->ldx, (int)N, (int)D, sw2, sb2, q);
+  row_sqnorm_kernel<<<(unsigned)((N * 32 + 255) / 256), 256, 0, h->stream>>>(X, h->ldx, (int)N, (int)D, sw2, sb2, q, h->flags.as<int>() + 1);
   h->st.kernel_launches++;
   const bool ntk = h->cfg.kernel_type == 1;
   if (!ntk) {
@@ -1524,7 +1532,7 @@ static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train
   CK(cudaStreamSynchronize(h->stream));
   t_total.collect(); t_h2d.collect(); t_gram.collect(); t_chol.collect(); t_solve.collect();
   flush_class_events(h);
-  if (flags[1]) return fail(h, NNGP_EINVAL, "nngp_fit: non-finite value in x_train / y_train");
+  if (flags[1]) return input_error(h, flags[1], "nngp_fit", "x_train / y_train");
   if (flags[0])
     return fail(h, NNGP_ENOTPD, "nngp_fit: K + lambda*I is not positive definite (pivot %d of %lld, lambda=%.6g)",
                 flags[0] - 1, (long long)N, h->lambda);
@@ -1734,7 +1742,7 @@ static int append_incremental(nngp_handle* h, int64_t M) {
   CK(cudaMemcpyAsync(h->y.p, h->app_y.p, (size_t)Nn * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
   CKR(check_finite_async(h, X + N * h->ldx, h->ldx, M, D));
   CKR(check_finite_async(h, h->y.as<double>() + N, 1, M, 1));
-  row_sqnorm_kernel<<<(unsigned)((Nn * 32 + 255) / 256), 256, 0, h->stream>>>(X, h->ldx, (int)Nn, (int)D, sw2, sb2, q);
+  row_sqnorm_kernel<<<(unsigned)((Nn * 32 + 255) / 256), 256, 0, h->stream>>>(X, h->ldx, (int)Nn, (int)D, sw2, sb2, q, h->flags.as<int>() + 1);
   h->st.kernel_launches++;
 
   StageTimer t_gram(h, &h->st.fit_gram_ms);
@@ -1776,7 +1784,7 @@ static int append_incremental(nngp_handle* h, int64_t M) {
   CK(cudaStreamSynchronize(h->stream));
   t_total.collect(); t_gram.collect(); t_chol.collect(); t_solve.collect();
   flush_class_events(h);
-  if (flags[1]) { drop_fit(h); return fail(h, NNGP_EINVAL, "nngp_append_fit: non-finite value in x_new / y_new"); }
+  if (flags[1]) { drop_fit(h); return input_error(h, flags[1], "nngp_append_fit", "x_new / y_new"); }
   if (flags[0]) {
     drop_fit(h);
     return fail(h, NNGP_ENOTPD, "nngp_append_fit: the extended K + lambda*I is not positive definite (pivot %lld of %lld)",
@@ -1923,7 +1931,7 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
       CKR(check_finite_async(h, xt + c0 * ldx, ldx, cr, D));
       double* qt_c = h->qt.as<double>() + c0;
       double* mp_c = h->mean_partial.as<double>() + c0 * 2 * col_tiles;
-      row_sqnorm_kernel<<<(unsigned)((cr * 32 + 255) / 256), 256, 0, h->stream>>>(xt + c0 * ldx, ldx, (int)cr, (int)D, sw2, sb2, qt_c);
+      row_sqnorm_kernel<<<(unsigned)((cr * 32 + 255) / 256), 256, 0, h->stream>>>(xt + c0 * ldx, ldx, (int)cr, (int)D, sw2, sb2, qt_c, h->flags.as<int>() + 1);
       h->st.kernel_launches++;
       CKR(run_gram(h, xt + c0 * ldx, ldx, cr, qt_c, h->X.as<double>(), ldx, N, h->q.as<double>(), D, blk + c0 * ldl, ldl, 0,
                    (ntk && var_out) ? h->blk2.as<double>() + c0 * ldl : nullptr, h->alpha.as<double>(), mp_c));
@@ -1991,7 +1999,7 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
     h->ev_pool.push_back(sp.first); h->ev_pool.push_back(sp.second);
   }
   flush_class_events(h);
-  if (flags[1]) return fail(h, NNGP_EINVAL, "nngp_predict: non-finite value in x_test");
+  if (flags[1]) return input_error(h, flags[1], "nngp_predict", "x_test");
   h->st.queries += T;
   return NNGP_OK;
 }

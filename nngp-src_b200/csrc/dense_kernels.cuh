@@ -26,8 +26,10 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // q[r] = sw2 * sum_j x[r][j]^2 / D + sb2 ; one warp per row.
+// range_flag (optional): |= 2 when some q >= 2^512 (or overflows): the Gram epilogue forms q q', which must stay finite.
+constexpr double Q_LIMIT = 0x1p+512;
 __global__ void row_sqnorm_kernel(const double* __restrict__ x, long long ldx, int rows, int D, double sw2,
-                                  double sb2, double* __restrict__ q) {
+                                  double sb2, double* __restrict__ q, int* __restrict__ range_flag = nullptr) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp >= rows) return;
@@ -38,7 +40,11 @@ __global__ void row_sqnorm_kernel(const double* __restrict__ x, long long ldx, i
     s = fma(v, v, s);
   }
   s = warp_sum(s);
-  if (lane == 0) q[warp] = sw2 * (s / (double)D) + sb2;
+  if (lane == 0) {
+    const double v = sw2 * (s / (double)D) + sb2;
+    q[warp] = v;
+    if (range_flag && !(v < Q_LIMIT)) atomicOr(range_flag, 2);
+  }
 }
 
 // kss[r] = layer-(depth-1) diagonal: q <- sw2_s*q/2 + sb2_s for the Dense layer that follows arc-cosine step s.
@@ -859,7 +865,7 @@ __global__ void state_pack_kernel(StatePackView v, long long offset, long long c
   }
 }
 
-// finite check: *flag |= any non-finite in x (rows x cols, ld)
+// finite check: *flag |= 1 for any non-finite in x (rows x cols, ld)
 __global__ void finite_check_kernel(const double* __restrict__ x, long long ld, long long rows, int cols,
                                     int* __restrict__ flag) {
   const long long total = rows * cols;

@@ -147,6 +147,8 @@ __device__ __forceinline__ double rcp_newton(double x) {
 // max(x, 0) for finite x through the sign bit (integer pipe); -0 and negative rounding residue become +0
 __device__ __forceinline__ double clamp_nonneg(double x) { return (__double2hiint(x) < 0) ? 0.0 : x; }
 
+// GUARD = false: only for max(s^2, k^2) in [2^-1022, 2^1022) (see gram_epilogue), where both versions agree bitwise.
+template <bool GUARD>
 __device__ __forceinline__ double atan2_pos(double s, double s2, double k) {
   constexpr double C[21] = {
     1.0,
@@ -176,9 +178,21 @@ __device__ __forceinline__ double atan2_pos(double s, double s2, double k) {
   // k is its top bit): a DSETP would queue on the FP64 pipe this epilogue shares with the co-resident CTA's DMMAs.
   const double a = fabs(k);
   const double a2 = k * k;
-  const bool s_bigger = __double_as_longlong(s2) > __double_as_longlong(a2);
-  const double mx2 = s_bigger ? s2 : a2;
-  const double t = (s * a) * rcp_newton(mx2);
+  bool s_bigger = __double_as_longlong(s2) > __double_as_longlong(a2);
+  double mx2 = s_bigger ? s2 : a2;
+  double sa = s * a;
+  // rcp.approx.ftz flushes a subnormal input (seed +inf -> NaN after Newton) and a subnormal result (t -> 0): outside
+  // mx2 in [2^-1022, 2^1022) -- biased exponent field 1..2044, tested on the integer pipe -- s and |k| are first scaled
+  // by 2^+-600 (t = min/max does not change), which brings max(s, |k|) from anywhere in [2^-1074, 2^1024) into
+  // [2^-474, 2^424].  s2 / a2 are then also unreliable (underflow), so the larger side is decided on s, |k| themselves.
+  if (GUARD && (unsigned)(__double2hiint(mx2) >> 20) - 1u >= 2044u) {
+    const double f = (__double2hiint(mx2) < 0x00100000) ? 0x1p+600 : 0x1p-600;
+    const double sf = s * f, af = a * f;
+    s_bigger = __double_as_longlong(sf) > __double_as_longlong(af);
+    mx2 = s_bigger ? sf * sf : af * af;
+    sa = sf * af;
+  }
+  const double t = sa * rcp_newton(mx2);
   const double u = t * t;
   const double w = u * u;
   double pe = C[20], po = C[19];
@@ -189,18 +203,20 @@ __device__ __forceinline__ double atan2_pos(double s, double s2, double k) {
   const double at = t * fma(u, po, pe);
   const double th0 = s_bigger ? (half_pi - at) : at;
   const double th = (__double2hiint(k) < 0) ? (pi - th0) : th0;
-  return (__double_as_longlong(mx2) == 0LL) ? half_pi : th;
+  // s == k == 0 on the bit patterns (s >= +0; the shift drops the sign of k): k^2 can underflow while k != 0
+  return ((__double_as_longlong(s) | (__double_as_longlong(k) << 1)) == 0LL) ? half_pi : th;
 }
 
 // One ReLU arc-cosine step followed by the next Dense layer's affine map
 // (SURVEY Appendix A.1; [nt 0.6.1 stax.ABRelu(a=0,b=1) nngp_ntk_fn + stax.Dense _affine]):
 //   s = sqrt(max(q1 q2 - k^2, 0)); theta = atan2(s, k) (pi/2 when s == k == 0)
 //   k' = sw2 * ( s/(2 pi) + (1/2 - theta/(2 pi)) k ) + sb2
+template <bool GUARD>
 __device__ __forceinline__ double arccos_step(double k, double q1, double q2, double sw2, double sb2) {
   const double inv_2pi = 0.15915494309189533577;
   double s2 = clamp_nonneg(q1 * q2 - k * k);
   double s = sqrt(s2);
-  double theta = atan2_pos(s, s2, k);
+  double theta = atan2_pos<GUARD>(s, s2, k);
   double dot_sigma = 0.5 - inv_2pi * theta;
   double r = inv_2pi * s + dot_sigma * k;
   return sw2 * r + sb2;
@@ -209,11 +225,12 @@ __device__ __forceinline__ double arccos_step(double k, double q1, double q2, do
 
 // Same step, also advancing the NTK:  ntk' = k' + sw2 * (ntk * kdot),  kdot = 1/2 - theta/(2 pi)
 // (SURVEY Appendix A.5; [nt: Relu `ntk *= dot_sigma`, Dense `ntk = nngp + W_std^2 * ntk`]).
+template <bool GUARD>
 __device__ __forceinline__ void arccos_step_ntk(double& k, double& ntk, double q1, double q2, double sw2, double sb2) {
   const double inv_2pi = 0.15915494309189533577;
   double s2 = clamp_nonneg(q1 * q2 - k * k);
   double s = sqrt(s2);
-  double theta = atan2_pos(s, s2, k);
+  double theta = atan2_pos<GUARD>(s, s2, k);
   double dot_sigma = 0.5 - inv_2pi * theta;
   double r = inv_2pi * s + dot_sigma * k;
   k = sw2 * r + sb2;
@@ -345,6 +362,25 @@ __device__ __forceinline__ void mma_mainloop(double (&acc)[4][4][2], const TileS
 //     accumulator tiles through shared memory to 8 epilogue warps -- 0.45 / 0.50 (0.47 / 0.52 with 8 entries in flight
 //     per thread): the register file caps the CTA at 16 warps, and 8 warps cannot keep enough of the epilogue's
 //     dependent FP64 chains in flight; the epilogue becomes the longer side.
+// Whether atan2_pos may skip its range guard for all W entries of a group: with q1 in [2^e1, 2^(e1+1)) and q2 in
+// [2^e2, 2^(e2+1)), max(s^2, k^2) lies in [q1 q2 / 2, q1 q2] (s^2 + k^2 = q1 q2, up to rounding), so
+// e1 + e2 in [-1020, 1019] keeps it inside [2^-1022, 2^1022).  That needs q1 and q2 to be normal doubles: a zero or
+// subnormal q (a row whose |x|^2 / D underflowed) no longer bounds k, whose own products did not underflow.
+// Exponents only: integer pipe.  The guarded version costs a branch per entry, which splits the W independent chains
+// the scheduler interleaves (-3..5 % Gram throughput), so it only runs for groups that need it (zero rows, inputs
+// near the ends of the FP64 range).
+template <int W>
+__device__ __forceinline__ bool q_in_range(double q1, const double (&q2)[W]) {
+  const int e1 = __double2hiint(q1) >> 20;   // biased exponent fields (q >= 0): 1..2046 for a normal double
+  bool ok = (unsigned)(e1 - 1) < 2046u;
+#pragma unroll
+  for (int j = 0; j < W; ++j) {
+    const int e2 = __double2hiint(q2[j]) >> 20;
+    ok &= ((unsigned)(e2 - 1) < 2046u) & ((unsigned)(e1 + e2 - (2046 - 1020)) <= 2039u);
+  }
+  return ok;
+}
+
 #ifndef NNGP_GRAM_ILP
 #define NNGP_GRAM_ILP 4   // entries advanced through the layers together (2, 4 or 8): independent dependency chains
 #endif                    // (sqrt, reciprocal, two Horner halves each) for the scheduler to interleave; 8 spills
@@ -374,8 +410,13 @@ __device__ __forceinline__ void gram_epilogue(const double (&acc)[4][4][2], cons
           for (int s = 0; s < p.steps; ++s) {
             const int li = s < GEMM_MAX_LAYERS ? s : GEMM_MAX_LAYERS - 1;
             const double sw2 = p.lsw2[li], sb2 = p.lsb2[li];
+            if (q_in_range<W>(qa, qb)) {
 #pragma unroll
-            for (int j = 0; j < W; ++j) k[j] = arccos_step(k[j], qa, qb[j], sw2, sb2);
+              for (int j = 0; j < W; ++j) k[j] = arccos_step<false>(k[j], qa, qb[j], sw2, sb2);
+            } else {
+#pragma unroll
+              for (int j = 0; j < W; ++j) k[j] = arccos_step<true>(k[j], qa, qb[j], sw2, sb2);
+            }
             if (s + 1 < p.steps) {              // the diagonals of the next layer (not needed after the last one)
 #pragma unroll
               for (int j = 0; j < W; ++j) qb[j] = sw2 * (0.5 * qb[j]) + sb2;
@@ -389,8 +430,13 @@ __device__ __forceinline__ void gram_epilogue(const double (&acc)[4][4][2], cons
           for (int s = 0; s < p.steps; ++s) {
             const int li = s < GEMM_MAX_LAYERS ? s : GEMM_MAX_LAYERS - 1;
             const double sw2 = p.lsw2[li], sb2 = p.lsb2[li];
+            if (q_in_range<W>(qa, qb)) {
 #pragma unroll
-            for (int j = 0; j < W; ++j) arccos_step_ntk(k[j], n[j], qa, qb[j], sw2, sb2);
+              for (int j = 0; j < W; ++j) arccos_step_ntk<false>(k[j], n[j], qa, qb[j], sw2, sb2);
+            } else {
+#pragma unroll
+              for (int j = 0; j < W; ++j) arccos_step_ntk<true>(k[j], n[j], qa, qb[j], sw2, sb2);
+            }
             if (s + 1 < p.steps) {
 #pragma unroll
               for (int j = 0; j < W; ++j) qb[j] = sw2 * (0.5 * qb[j]) + sb2;

@@ -149,8 +149,9 @@ def test_active_sampling_restatement():
 
 
 def test_device_atan2_algorithm_in_numpy():
-    """The Gram epilogue's atan2_pos (csrc/gemm_nt.cuh) restated in numpy with the SAME coefficients (parsed from
-    the source): <= 1 ulp-level agreement with libm and with 40-digit mpmath, incl. the axes and the origin."""
+    """The Gram epilogue's atan2_pos (csrc/gemm_nt.cuh) restated in numpy with the SAME coefficients and range guard
+    (parsed from the source) and the flush-to-zero semantics of rcp.approx.ftz.f64: <= 2 ulp of theta against libm and
+    40-digit mpmath over the whole double range of s and k, incl. subnormals, the axes and the origin."""
     import re
     from pathlib import Path
     import mpmath as mp
@@ -159,16 +160,40 @@ def test_device_atan2_algorithm_in_numpy():
     body = body[:body.index("};")]
     coef = [float(v) for v in re.findall(r"-?\d+\.\d+(?:e-?\d+)?", body.split("{", 1)[1])]
     assert len(coef) == 21 and coef[0] == 1.0
+    # the range guard in front of the reciprocal: biased exponent field of max(s^2, k^2) outside 1..hi, scale 2^+-e
+    guard = re.search(r"__double2hiint\(mx2\) >> 20\) - 1u >= (\d+)u\).*?\? 0x1p\+(\d+) : 0x1p-(\d+);", src, re.S)
+    assert guard, "atan2_pos: range guard of the reciprocal not found"
+    hi, e_up, e_dn = (int(v) for v in guard.groups())
+    assert (hi, e_up) == (2044, e_dn)     # [2^-1022, 2^1022): the reciprocal and its result are normal doubles
 
-    def atan2_pos(s, k):
-        # min/max = s |k| / max(s^2, k^2) (reciprocal + product instead of a division; the device computes the
-        # reciprocal with a MUFU seed + two Newton steps, <= 1 ulp from the correctly rounded one used here),
+    tiny = 2.0 ** -1022
+
+    def rcp_newton(x):
+        # rcp.approx.ftz.f64: a subnormal input and a subnormal result are flushed to zero (input 0 -> +inf); the seed
+        # is correctly rounded here (the MUFU seed is ~20 bits, the two Newton steps make up the difference: <= 1 ulp)
+        r = 1.0 / np.where(x < tiny, 0.0, x)
+        r = np.where(r < tiny, 0.0, r)
+        for _ in range(2):
+            r = r * (1.0 - x * r) + r
+        return r
+
+    def atan2_pos(s, k, guarded=True):
+        # min/max = s |k| / max(s^2, k^2) (reciprocal + product instead of a division),
         # P(u) = Pe(u^2) + u Po(u^2): two Horner chains of 10
         a = np.abs(k)
         s2, a2 = s * s, k * k
-        mx2 = np.maximum(s2, a2)
-        with np.errstate(invalid="ignore", divide="ignore"):
-            t = (s * a) * (1.0 / mx2)
+        sbig = s2 > a2
+        mx2 = np.where(sbig, s2, a2)
+        sc = s
+        if guarded:
+            field = (mx2.view(np.int64) >> 52) & 0x7FF
+            rare = (field < 1) | (field > hi)
+            f = np.where(field < 1, 2.0 ** e_up, 2.0 ** -e_dn)
+            sc = np.where(rare, s * f, s)
+            a = np.where(rare, a * f, a)
+            sbig = np.where(rare, sc > a, sbig)
+            mx2 = np.where(rare, np.where(sbig, sc * sc, a * a), mx2)
+        t = (sc * a) * rcp_newton(mx2)
         u = t * t
         w = u * u
         pe = np.full_like(u, coef[20])
@@ -178,21 +203,90 @@ def test_device_atan2_algorithm_in_numpy():
         for c in coef[17::-2]:
             po = po * w + c
         at = t * (u * po + pe)
-        th0 = np.where(s2 > a2, np.pi / 2 - at, at)
-        th = np.where(k < 0, np.pi - th0, th0)
-        return np.where(mx2 == 0, np.pi / 2, th)
+        th0 = np.where(sbig, np.pi / 2 - at, at)
+        th = np.where(np.signbit(k), np.pi - th0, th0)
+        if not guarded:
+            return np.where(mx2 == 0, np.pi / 2, th)
+        return np.where((s == 0) & (k == 0), np.pi / 2, th)
+
+    def ref_of(s, k):
+        r = np.arctan2(s, k)
+        r[(s == 0) & (k == 0)] = np.pi / 2
+        return r
 
     rng = np.random.default_rng(1)
-    # magnitudes a kernel value can take (the squares must stay inside the FP64 range)
-    s = np.abs(rng.standard_normal(200000)) * 10 ** rng.uniform(-12, 9, 200000)
-    k = rng.standard_normal(200000) * 10 ** rng.uniform(-12, 9, 200000)
-    s[:500] = 0.0; k[500:1000] = 0.0; s[1000] = k[1000] = 0.0; k[1001:1500] = s[1001:1500]
-    ref = np.arctan2(s, k)
-    ref[(s == 0) & (k == 0)] = np.pi / 2
-    assert np.max(np.abs(atan2_pos(s, k) - ref)) <= 9e-16            # <= 2 ulp of theta in [0, pi]
-    mp.mp.dps = 40
-    hi = np.array([float(mp.atan2(mp.mpf(float(a)), mp.mpf(float(b)))) for a, b in zip(s[2000:4000], k[2000:4000])])
-    assert np.max(np.abs(atan2_pos(s[2000:4000], k[2000:4000]) - hi)) <= 9e-16
+    with np.errstate(all="ignore"):
+        # magnitudes of a kernel value in ordinary use
+        s = np.abs(rng.standard_normal(200000)) * 10 ** rng.uniform(-12, 9, 200000)
+        k = rng.standard_normal(200000) * 10 ** rng.uniform(-12, 9, 200000)
+        s[:500] = 0.0; k[500:1000] = 0.0; s[1000] = k[1000] = 0.0; k[1001:1500] = s[1001:1500]
+        k[1500:1600] = -0.0
+        assert np.max(np.abs(atan2_pos(s, k) - ref_of(s, k))) <= 9e-16            # <= 2 ulp of theta in [0, pi]
+        # ... which the guard leaves bitwise alone (mx2 inside [2^-1022, 2^1022) there)
+        assert np.array_equal(atan2_pos(s, k), atan2_pos(s, k, guarded=False))
+        mp.mp.dps = 40
+        hi_ = np.array([float(mp.atan2(mp.mpf(float(a)), mp.mpf(float(b)))) for a, b in zip(s[2000:4000], k[2000:4000])])
+        assert np.max(np.abs(atan2_pos(s[2000:4000], k[2000:4000]) - hi_)) <= 9e-16
+
+        # the whole double range: exponents of s and |k| swept independently over [-1074, 1023], subnormals included
+        n = 300000
+        es, ek = rng.integers(-1074, 1024, n), rng.integers(-1074, 1024, n)
+        es[:2000] = ek[:2000] + rng.integers(-3, 4, 2000)               # comparable magnitudes: theta away from the axes
+        es[150:250] = ek[150:250] = 511                                  # max(s^2, k^2) in [2^1022, 2^1024)
+        s = np.ldexp(rng.uniform(1.0, 2.0, n), es)
+        k = np.ldexp(rng.uniform(1.0, 2.0, n), ek) * rng.choice([-1.0, 1.0], n)
+        s[:50] = 0.0; k[50:100] = 0.0; k[100:150] = -0.0
+        ref = ref_of(s, k)
+        got = atan2_pos(s, k)
+        assert np.all(np.isfinite(got))
+        assert np.max(np.abs(got - ref)) <= 9e-16
+        hi_ = np.array([float(mp.atan2(mp.mpf(float(a)), mp.mpf(float(b)))) for a, b in zip(s[:2000], k[:2000])])
+        assert np.max(np.abs(got[:2000] - hi_)) <= 9e-16
+        # without the guard the flush-to-zero reciprocal breaks exactly there (defects the guard exists for):
+        bare = atan2_pos(s, k, guarded=False)
+        mx = np.maximum(s, np.abs(k))
+        sub = (mx < 2.0 ** -511) & (mx > 0)
+        assert np.any(np.isnan(bare[sub]) & (np.maximum(s * s, k * k)[sub] > 0))      # subnormal max(s^2, k^2): NaN
+        assert np.any(np.abs(bare[sub] - ref[sub]) == np.pi / 2)                     # k^2 underflows: pi/2, not 0 / pi
+        big = (mx >= 2.0 ** 511) & (mx < 2.0 ** 512)                                  # (q < 2^512 keeps |k|, s there)
+        assert np.max(np.abs(bare[big] - ref[big])) > 0.1                             # 1/mx2 flushed: t = 0
+    # gram_epilogue skips the guard (atan2_pos<false>) when q1 and q2 are normal doubles whose exponents sum to
+    # [lo, hi]: then max(s^2, k^2) is inside [2^-1022, 2^1022), even with |k| a little above sqrt(q1 q2) from rounding
+    gate = re.search(r"ok &= \(\(unsigned\)\(e2 - 1\) < (\d+)u\) & \(\(unsigned\)\(e1 \+ e2 - \(2046 - (\d+)\)\) <= (\d+)u\)",
+                     src)
+    assert gate, "gram_epilogue: exponent gate of the unguarded path not found"
+    assert re.search(r"bool ok = \(unsigned\)\(e1 - 1\) < %su;" % gate.group(1), src)
+    n_normal, lo = int(gate.group(1)), -int(gate.group(2))
+    hi_e = lo + int(gate.group(3))
+    assert (n_normal, lo, hi_e) == (2046, -1020, 1019)
+
+    def fast(q1, q2):      # the gate, on the biased exponent fields like the device
+        f1, f2 = (np.asarray(q1).view(np.int64) >> 52) & 0x7FF, (np.asarray(q2).view(np.int64) >> 52) & 0x7FF
+        return (f1 >= 1) & (f1 <= n_normal) & (f2 >= 1) & (f2 <= n_normal) & (f1 + f2 - 2046 >= lo) & (f1 + f2 - 2046 <= hi_e)
+
+    n = 200000
+    e1 = rng.integers(-1022, 1023, n)
+    e2 = np.where(rng.random(n) < 0.5, lo, hi_e) - e1
+    ok = (e2 >= -1022) & (e2 <= 1022)
+    q1 = np.ldexp(rng.uniform(1.0, 2.0, n)[ok], e1[ok])
+    q2 = np.ldexp(rng.uniform(1.0, 2.0, n)[ok], e2[ok])
+    assert np.all(fast(q1, q2))
+    kk = np.sqrt(q1) * np.sqrt(q2) * rng.uniform(-1.0 - 8 * 2.0 ** -52, 1.0 + 8 * 2.0 ** -52, q1.size)
+    mx2 = np.maximum(np.maximum(q1 * q2 - kk * kk, 0.0), kk * kk)
+    assert np.all((mx2 >= 2.0 ** -1022) & (mx2 < 2.0 ** 1022))
+    # a row whose q underflowed (to 0 or a subnormal) no longer bounds k: x = (3, 1) 2^-540 against y = (2, -0.5) 2^20
+    # has q_x = 0 but k = 2.75 2^-520, k^2 subnormal -- such groups must take the guarded path
+    for ex in (-540, -530):
+        x, y = np.ldexp(np.array([3.0, 1.0]), ex), np.ldexp(np.array([2.0, -0.5]), 20)
+        qx, qy = x @ x / 2, y @ y / 2
+        assert not fast(qx, qy) and not fast(qy, qx) and not fast(0.0, 1.0) and not fast(np.inf, 1.0)
+    # a pair from the kernel's own domain: x = (3, 1) 2^-530, y = (2, -0.5): k, s ~ 2^-530, k^2 and s^2 subnormal
+    x, y = np.ldexp(np.array([3.0, 1.0]), -530), np.array([2.0, -0.5])
+    kk, q1, q2 = x @ y / 2, x @ x / 2, y @ y / 2
+    ss = np.sqrt(np.array([max(q1 * q2 - kk * kk, 0.0)]))
+    with np.errstate(all="ignore"):
+        assert np.isnan(atan2_pos(ss, np.array([kk]), guarded=False)[0])
+    assert abs(atan2_pos(ss, np.array([kk]))[0] - np.arctan2(ss[0], kk)) < 1e-3
 
 
 @pytest.mark.parametrize("case", ["layers_d2", "layers_d3"])
