@@ -29,9 +29,6 @@
 
 using namespace nngp;
 
-// (the fused panel kernel may ask for more shared memory than it uses, to keep an SM to itself: potrf_panel_fused)
-constexpr int PANEL_SMEM_MAX = 200 * 1024;
-
 namespace {
 
 thread_local std::string g_create_error;
@@ -348,42 +345,22 @@ int run_gemm_rowdot(nngp_handle* h, const double* V, int64_t ldv, int64_t rows, 
 
 // ---- blocked Cholesky (lower, in place, row-major) ----------------------------------------------
 // Right-looking over W-wide outer panels (trailing SYRK with K = W on the DMMA core), left-looking
-// over the 64-wide sub-panels inside a panel (potf2 on the diagonal block, one-thread-per-row
-// forward substitution for the block column below it).
+// over the 64-wide sub-panels inside a panel (potrf_panel).
 // Outer panel width: 256 keeps the panel chain short for small N; for larger N the trailing SYRK
 // dominates and K = 512 runs closer to the DMMA peak (measured at N = 32768: 394 / 378 / 371 ms for
-// W = 256 / 384 / 512; at N = 8192: 13.8 / 14.5 / 15.2 ms).  NNGP_CHOL_W overrides.
+// W = 256 / 384 / 512; at N = 8192: 13.8 / 14.5 / 15.2 ms).
 int chol_outer_width(int64_t N) {
-  static int forced = [] {
-    const char* e = getenv("NNGP_CHOL_W");
-    int v = e ? atoi(e) : 0;
-    return v >= NB ? (v / NB) * NB : 0;
-  }();
-  if (forced) return forced;
   // (with the fused panel kernel: N = 4096 3.44 vs 3.54 ms, N = 8192 9.67 vs 9.96 ms for W = 512 vs 256;
   //  N = 32768: 356.0 / 353.9 / 352.0 ms for W = 512 / 768 / 1024)
   return N >= 24576 ? 1024 : (N >= 4096 ? 512 : 256);
 }
 
-// `R` = N + extra rows riding along below the matrix (see run_potrf).
-// Per 64-wide sub-panel: (1) left-looking update from the panel's earlier columns (DMMA), (2) potf2_64: Cholesky of
-// the diagonal block AND its inverse W = inv(L_JJ) in one one-CTA launch, (3) the block column below it,
-// X L_JJ^T = B  ->  X = B W^T, as a K = 64 product on the tensor pipe (gemm_nt_kernel<EPI_DIAG>, in place: a CTA reads
-// its own 128 x 64 tile completely before it stores it).  Step (3) used to be a one-thread-per-row substitution on
-// the FP64 CUDA cores (23 us per sub-panel on the critical path of the panel chain; NNGP_PANEL_SOLVE=fma brings
-// it back for A/B runs).  `Winv` receives the inverses, block J at rows [64 J, 64 J + 64) of a 64-wide matrix.
-bool panel_solve_fma() {
-  static const bool v = [] { const char* e = getenv("NNGP_PANEL_SOLVE"); return e && !strcmp(e, "fma"); }();
-  return v;
-}
-
-// The whole panel as one persistent kernel (potrf_panel.cuh); NNGP_PANEL=steps selects the launch-per-step chain below.
-bool panel_fused() {
-  static const bool v = [] { const char* e = getenv("NNGP_PANEL"); return !(e && !strcmp(e, "steps")); }();
-  return v;
-}
-
-int potrf_panel_fused(nngp_handle* h, double* A, int64_t ld, int64_t N, int64_t R, int64_t j0, int64_t w, double* Winv) {
+// One outer panel, columns [j0, j0 + w) of the rows from j0 down to `R` = N + extra rows riding along below the
+// matrix (see run_potrf), as one persistent kernel (potrf_panel.cuh).  Per 64-wide sub-panel: the left-looking
+// update from the panel's earlier columns, potf2_64_block (Cholesky of the diagonal block AND its inverse
+// W = inv(L_JJ)), and the block column below it, X L_JJ^T = B  ->  X = B W^T, as a K = 64 product on the tensor pipe.
+// `Winv` receives the inverses, block J at rows [64 J, 64 J + 64) of a 64-wide matrix.
+int potrf_panel(nngp_handle* h, double* A, int64_t ld, int64_t N, int64_t R, int64_t j0, int64_t w, double* Winv) {
   PanelParams p{};
   p.A = A; p.ld = ld; p.j0 = (int)j0; p.rows = (int)(R - j0); p.ncols = (int)w;
   p.row_tiles = (int)((R - j0 + GEMM_BM - 1) / GEMM_BM);
@@ -402,18 +379,12 @@ int potrf_panel_fused(nngp_handle* h, double* A, int64_t ld, int64_t N, int64_t 
   // Grid: a few CTAs per row tile, but no more than a quarter of the GPU's CTA slots.  The kernel's CTAs spend most of
   // their life waiting for the owner's potf2; every slot they hold is a slot the trailing update running beside
   // them (look-ahead) cannot use -- with 2 x #SMs spinning CTAs the overlap was gone (measured: 11.0 ms at N = 8192,
-  // no better than the launch-per-step chain).  NNGP_PANEL_GRID overrides (A/B runs).
-  static const int forced_grid = [] { const char* e = getenv("NNGP_PANEL_GRID"); return e ? atoi(e) : 0; }();
+  // no better than the launch-per-step chain this kernel replaced).
   const long long total = (long long)p.row_tiles * p.col_blocks;
   // (3 CTAs per row tile: the extra ones claim the row tile's NEXT column blocks early and work through the k-tiles
   //  that already exist while the owner is still factoring -- N = 4096: 3.45 -> 3.28 ms, 8192: 9.65 -> 9.50 ms)
-  static const int grid_mult = [] { const char* e = getenv("NNGP_PANEL_GRID_MULT"); return e ? std::max(1, atoi(e)) : 3; }();
-  int grid = (int)std::min<long long>((long long)p.row_tiles * grid_mult, h->sm_count / 2);
-  if (forced_grid > 0) grid = forced_grid;
+  int grid = (int)std::min<long long>((long long)p.row_tiles * 3, h->sm_count / 2);
   grid = (int)std::max<long long>(1, std::min<long long>(grid, total));
-  static const int forced_smem = [] { const char* e = getenv("NNGP_PANEL_SMEM"); return e ? atoi(e) : -1; }();
-  int panel_smem = TF_SMEM_BYTES;
-  if (forced_smem >= 0) panel_smem = std::min(std::max(panel_smem, forced_smem), PANEL_SMEM_MAX);
   // NNGP_PANEL_TRACE=1 (diagnostics): time stamps of the owner items of every panel -> stderr (synchronises!)
 #ifdef NNGP_PANEL_TRACE
   static const bool trace = [] { const char* e = getenv("NNGP_PANEL_TRACE"); return e && atoi(e) > 0; }();
@@ -426,7 +397,7 @@ int potrf_panel_fused(nngp_handle* h, double* A, int64_t ld, int64_t N, int64_t 
     CK(cudaMemsetAsync(tr_d, 0, (size_t)p.col_blocks * 18 * sizeof(unsigned long long), h->cur));
     p.trace = tr_d;
   }
-  potrf_panel_kernel<<<grid, GEMM_THREADS, panel_smem, h->cur>>>(tmA, tmL, tmW, p);
+  potrf_panel_kernel<<<grid, GEMM_THREADS, TF_SMEM_BYTES, h->cur>>>(tmA, tmL, tmW, p);
   CK(cudaGetLastError());
   h->st.kernel_launches++;
   if (trace) {
@@ -450,42 +421,12 @@ int potrf_panel_fused(nngp_handle* h, double* A, int64_t ld, int64_t N, int64_t 
   return NNGP_OK;
 }
 
-int potrf_panel(nngp_handle* h, double* A, int64_t ld, int64_t N, int64_t R, int64_t j0, int64_t w, double* Winv) {
-  if (panel_fused()) return potrf_panel_fused(h, A, ld, N, R, j0, w, Winv);
-  int* info = h->flags.as<int>();
-  MatView Av{A, R, N, ld}, Wv{Winv, round_up(N, NB), NB, NB};
-  for (int64_t s0 = j0; s0 < j0 + w; s0 += NB) {
-    const int64_t nb = std::min<int64_t>(NB, N - s0);
-    if (s0 > j0)  // A[s0:R, s0:s0+nb] -= A[s0:R, j0:s0] * A[s0:s0+nb, j0:s0]^T
-      CKR(run_gemm_sub(h, Av, s0, j0, Av, s0, j0, R - s0, nb, s0 - j0, A + s0 * ld + s0, ld, 0));
-    potf2_64_kernel<<<1, POTF2_THREADS, 0, h->cur>>>(A + s0 * ld + s0, ld, (int)nb, (int)s0, info, Winv + s0 * NB);
-    h->st.kernel_launches++;
-    const int64_t below = R - s0 - nb;
-    if (below > 0) {
-      if (panel_solve_fma()) {
-        const int grid = (int)((below + TRSM_ROWS - 1) / TRSM_ROWS);
-        trsm_rows_64_kernel<<<grid, TRSM_ROWS, TRSM_SMEM_BYTES, h->cur>>>(A + (s0 + nb) * ld + s0, ld, (int)below,
-                                                                         A + s0 * ld + s0, ld, (int)nb);
-        h->st.kernel_launches++;
-      } else {
-        GemmParams p{};
-        p.M = (int)below; p.N = (int)nb; p.ktiles = NB / GEMM_BK;
-        p.C = A + (s0 + nb) * ld + s0; p.ldc = ld;
-        p.var = nullptr; p.J = 0; p.col_blocks = 1;
-        CKR(launch_gemm<EPI_DIAG>(h, Av, (int)(s0 + nb), (int)s0, Wv, (int)s0, 0, p));
-      }
-    }
-  }
-  return NNGP_OK;
-}
-
 // Blocked right-looking Cholesky.  The trailing update of outer step j is split into (A) the columns of the NEXT
 // panel and (B) the rest.
 // Look-ahead (on by default, NNGP_CHOL_LOOKAHEAD=0 disables it): as soon as (A) is done the next panel is factored
 // on a high-priority stream while (B) keeps the tensor pipes busy on the main stream (-6 % fit time at N = 32768,
 // -30 % at N = 8192).  The two streams touch disjoint column ranges, so the factor is bitwise the same with and
-// without it (tests/test_gpu_parity.py, tools/determinism_check.py).  NNGP_LA_MODE=2 keeps the two-stream schedule
-// but removes the overlap (debugging aid, see DESIGN.md 5.3).
+// without it (tests/test_gpu_parity.py, tools/determinism_check.py).
 // `extra` rows stored below the matrix (rows N..N+extra-1, N columns each) are carried through every
 // panel solve and trailing update: on exit they hold  E L^-T.  The fit puts y^T there, so the forward
 // substitution z = L^-1 y of the alpha solve costs nothing extra (one more row in GEMMs already running).
@@ -496,7 +437,6 @@ int run_potrf(nngp_handle* h, double* A, int64_t ld, int64_t N, int64_t extra, d
   // counters / flags of the fused panel kernel, sized once so that nothing is (re)allocated between the panels
   CKR(ensure(h, h->panel_sync, (size_t)(2 + (R + GEMM_BM - 1) / GEMM_BM + (W + NB - 1) / NB) * sizeof(int)));
   const bool lookahead = h->panel_stream != nullptr && N > 2 * W;
-  static const int la_mode = [] { const char* e = getenv("NNGP_LA_MODE"); return e ? atoi(e) : 1; }();
   cudaEvent_t ev_cols = get_event(h), ev_panel = get_event(h);
   auto edge = [&](cudaEvent_t e, cudaStream_t from, cudaStream_t to) -> cudaError_t {
     cudaError_t r = cudaEventRecord(e, from);
@@ -529,12 +469,11 @@ int run_potrf(nngp_handle* h, double* A, int64_t ld, int64_t N, int64_t extra, d
     rc = run_gemm_sub(h, Av, t0, j0, Av, t0, j0, R - t0, w2, w, A + t0 * ld + t0, ld, 1);
     span_end();
     if (rc != NNGP_OK) break;
-    if (lookahead && la_mode != 2 && ce == cudaSuccess) ce = edge(ev_cols, h->stream, h->panel_stream);
+    if (lookahead && ce == cudaSuccess) ce = edge(ev_cols, h->stream, h->panel_stream);
     // (B) the rest of the trailing matrix: A[t1:R, t1:N] (lower) -= A[t1:R, j0:t0] * A[t1:N, j0:t0]^T
     span_begin("B", j0);
     if (t1 < N) rc = run_gemm_sub(h, Av, t1, j0, Av, t1, j0, R - t1, N - t1, w, A + t1 * ld + t1, ld, 1);
     span_end();
-    if (lookahead && la_mode == 2 && ce == cudaSuccess) ce = edge(ev_cols, h->stream, h->panel_stream);  // no overlap
   }
   if (lookahead && ce == cudaSuccess) ce = edge(ev_panel, h->panel_stream, h->stream);  // join
   h->cur = h->stream;
@@ -793,65 +732,44 @@ int launch_sliced(nngp_handle* h, const int8_t* qa, int64_t ra, const double* sa
   p.ra = ra; p.rb = rb; p.rscale = sa; p.cscale = sw; p.vpart = vpart; p.V = V; p.ldv = ldv;
   if ((int64_t)s * ra >= (1LL << 31) || (int64_t)s * rb >= (1LL << 31))
     return fail(h, NNGP_EINVAL, "internal: digit-plane row range too large");
-  static const int grid_env = [] { const char* e = getenv("NNGP_SLICED_GRID"); return e ? atoi(e) : 0; }();
-  static const int rt_env = [] { const char* e = getenv("NNGP_SLICED_RT"); return e ? atoi(e) : 0; }();
-  static const int cl_env = [] { const char* e = getenv("NNGP_SLICED_CLUSTER"); return e ? atoi(e) : SL_CLUSTER_DEFAULT; }();
-  static const int sync_env = [] { const char* e = getenv("NNGP_SLICED_SYNC"); return e ? atoi(e) : SL_SYNC_DEFAULT; }();
-  // two row tiles per CTA tile: 32 KiB of operands per MMA set instead of 48.  (Single row tiles -- twice as many,
-  // lighter tiles -- were measured for small batches and lose: 1024 rows at N = 8192 take 1.82 ms instead of 1.55 ms,
-  // the kernel is bound by bytes per MAC even there.  NNGP_SLICED_RT=1 keeps the variant for A/B runs.)
-  p.rt = rt_env == 1 ? 1 : 2;
+  // Two row tiles per CTA tile (SL_RT): 32 KiB of operands per MMA set instead of 48.  (Single row tiles -- twice as
+  // many, lighter tiles -- were measured for small batches and lose: 1024 rows at N = 8192 take 1.82 ms instead of
+  // 1.55 ms, the kernel is bound by bytes per MAC even there.)
+  const int64_t tiles = (int64_t)((p.row_tiles + SL_RT - 1) / SL_RT) * p.col_tiles;
+  const int grid = (int)std::min<int64_t>((h->sm_count / SL_SUPER) * SL_SUPER, tiles);   // CTAs 4k..4k+3 share K_* row tiles
+  CKR(ensure(h, h->slscratch, (size_t)grid * SL_RT * SL_BM * SL_BN * sizeof(double)));
+  p.scratch = h->slscratch.as<double>();
   CUtensorMap tmA, tmB;
   CKR(get_tmap_u8(h, qa, (uint64_t)s * ra, (uint64_t)ldq, SL_RT * SL_BM, &tmA));
-  // One attempt per cluster size: 2 (W stages multicast inside CTA pairs) falls back to 1 when the driver cannot place
-  // the clusters; inside an attempt the wave re-alignment (cooperative launch: every CTA resident) falls back to
-  // free-running CTAs when the grid cannot be co-scheduled (another context holds SMs).
+  CKR(get_tmap_u8(h, qw, (uint64_t)s * rb, (uint64_t)ldq, SL_BN, &tmB));
+  CK(cudaFuncSetAttribute(sliced_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SL_SMEM_BYTES));   // (per device)
+  cudaLaunchConfig_t lc = {};
+  cudaLaunchAttribute coop;
+  coop.id = cudaLaunchAttributeCooperative;
+  coop.val.cooperative = 1;
+  lc.gridDim = dim3((unsigned)grid); lc.blockDim = dim3(SL_THREADS); lc.dynamicSmemBytes = SL_SMEM_BYTES;
+  lc.stream = h->stream;
+  // The wave re-alignment (wave_barrier, one counter per round of tiles) needs every CTA resident: a cooperative
+  // launch.  With a single round there is nothing to re-align, and when the grid cannot be co-scheduled (another
+  // context holds SMs) the launch is refused: then the CTAs run free.
+  const int64_t rounds = (tiles + grid - 1) / grid;
   bool launched = false;
-  for (int cl = (cl_env == 2 ? 2 : 1); cl >= 1 && !launched; --cl) {
-    p.cl = cl;
-    const int64_t pairs = ((p.row_tiles + p.rt - 1) / p.rt + cl - 1) / cl * cl;
-    const int64_t tiles = pairs * p.col_tiles;
-    int grid = grid_env > 0 ? grid_env : (h->sm_count / SL_SUPER) * SL_SUPER;   // CTAs 4k..4k+3 (cl = 2: 8k..8k+7) share K_* row tiles
-    const void* fn = cl == 2 ? (const void*)sliced_gemm_kernel<2> : (const void*)sliced_gemm_kernel<1>;
-    CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, SL_SMEM_BYTES));   // (per device)
-    cudaLaunchConfig_t lc = {};
-    cudaLaunchAttribute attrs[2];
-    lc.blockDim = dim3(SL_THREADS); lc.dynamicSmemBytes = SL_SMEM_BYTES; lc.stream = h->stream; lc.attrs = attrs;
-    if (cl == 2) {
-      attrs[0].id = cudaLaunchAttributeClusterDimension;
-      attrs[0].val.clusterDim.x = 2; attrs[0].val.clusterDim.y = 1; attrs[0].val.clusterDim.z = 1;
-      lc.numAttrs = 1;
-      lc.gridDim = dim3((unsigned)(grid / 2 * 2));
-      int nclusters = 0;
-      if (cudaOccupancyMaxActiveClusters(&nclusters, fn, &lc) != cudaSuccess || nclusters < 1) { cudaGetLastError(); continue; }
-      grid = std::min(grid, 2 * nclusters) / SL_SUPER * SL_SUPER;
-      if (grid < 2) continue;
-    }
-    grid = (int)std::min<int64_t>(grid, tiles);
-    CKR(ensure(h, h->slscratch, (size_t)grid * SL_RT * SL_BM * SL_BN * sizeof(double)));
-    p.scratch = h->slscratch.as<double>();
-    CKR(get_tmap_u8(h, qw, (uint64_t)s * rb, (uint64_t)ldq, SL_BN / cl, &tmB));
-    const int64_t rounds = (tiles + grid - 1) / grid;
-    lc.gridDim = dim3((unsigned)grid);
-    for (int sync = ((sync_env == 1 || sync_env == 2) && rounds >= 2 ? sync_env : 0); !launched; sync = 0) {
-      p.sync_mode = sync; p.wave_sync = nullptr;
-      lc.numAttrs = cl == 2 ? 1 : 0;
-      if (sync) {
-        const size_t nsync = (size_t)rounds * (sync == 2 ? s : 1);
-        CKR(ensure(h, h->slsync, nsync * sizeof(int)));
-        CK(cudaMemsetAsync(h->slsync.p, 0, nsync * sizeof(int), h->stream));
-        p.wave_sync = h->slsync.as<int>();
-        attrs[lc.numAttrs].id = cudaLaunchAttributeCooperative;
-        attrs[lc.numAttrs].val.cooperative = 1;
-        lc.numAttrs++;
-      }
-      const cudaError_t le = cl == 2 ? cudaLaunchKernelEx(&lc, sliced_gemm_kernel<2>, tmA, tmB, p)
-                                     : cudaLaunchKernelEx(&lc, sliced_gemm_kernel<1>, tmA, tmB, p);
-      if (le == cudaSuccess) launched = true;
-      else { cudaGetLastError(); if (!sync || cl == 2) break; }   // (clusters without re-alignment are not worth keeping: try cl = 1)
+  if (rounds >= 2) {
+    CKR(ensure(h, h->slsync, (size_t)rounds * sizeof(int)));
+    CK(cudaMemsetAsync(h->slsync.p, 0, (size_t)rounds * sizeof(int), h->stream));
+    p.wave_sync = h->slsync.as<int>();
+    lc.attrs = &coop; lc.numAttrs = 1;
+    launched = cudaLaunchKernelEx(&lc, sliced_gemm_kernel, tmA, tmB, p) == cudaSuccess;
+    if (!launched) cudaGetLastError();
+  }
+  if (!launched) {
+    p.wave_sync = nullptr;
+    lc.attrs = nullptr; lc.numAttrs = 0;
+    if (cudaLaunchKernelEx(&lc, sliced_gemm_kernel, tmA, tmB, p) != cudaSuccess) {
+      cudaGetLastError();
+      return fail(h, NNGP_ECUDA, "sliced_gemm_kernel could not be launched");
     }
   }
-  if (!launched) return fail(h, NNGP_ECUDA, "sliced_gemm_kernel could not be launched");
   CK(cudaGetLastError());
   h->st.kernel_launches++;
   h->st.sliced_macs += sliced_macs(p.row_tiles, p.col_tiles, K, tri, s, skip_weak);
@@ -874,14 +792,9 @@ int build_w_planes(nngp_handle* h) {
   return NNGP_OK;
 }
 
-// The variance path drops the plane pair (s-1, 0) (SlicedParams::skip_weak); NNGP_SLICED_KEEP_ALL_PAIRS=1 keeps it.
-static int sliced_skip_weak() {
-  static const int keep = [] { const char* e = getenv("NNGP_SLICED_KEEP_ALL_PAIRS"); return e ? atoi(e) : 0; }();
-  return keep ? 0 : 1;
-}
-
 // var[r] = kss[r] - |K_*[r,:] W^T|^2 with the product on the int8 tensor cores, in row sub-blocks whose planes fit
-// 16 GiB (whole waves of 37 row tiles x 4 column tiles, so that the static tile order stays balanced)
+// 16 GiB (whole waves of 37 row tiles x 4 column tiles, so that the static tile order stays balanced).  The plane
+// pair (s-1, 0) is dropped (SlicedParams::skip_weak).
 int run_sliced_variance(nngp_handle* h, const double* B, int64_t ldb, int64_t rows, const double* kss, double* var) {
   const int s = h->cfg.variance_slices;
   const int64_t N = h->N, ldq = h->wq_ldq;
@@ -901,7 +814,7 @@ int run_sliced_variance(nngp_handle* h, const double* B, int64_t ldb, int64_t ro
     rc = slice_matrix(h, B + r0 * ldb, ldb, nr, N, 0, s, ra, ldq, h->Aq.as<int8_t>(), h->ascale.as<double>());
     if (rc == NNGP_OK)
       rc = launch_sliced(h, h->Aq.as<int8_t>(), ra, h->ascale.as<double>(), h->Wq.as<int8_t>(), h->wq_rb,
-                         h->wscale.as<double>(), ldq, s, 1, nr, N, N, h->partial.as<double>(), nullptr, 0, sliced_skip_weak());
+                         h->wscale.as<double>(), ldq, s, 1, nr, N, N, h->partial.as<double>(), nullptr, 0, 1);
     if (rc == NNGP_OK) {
       var_from_partial_kernel<<<(unsigned)((nr + 255) / 256), 256, 0, h->stream>>>(kss + r0, h->partial.as<double>(), 2 * col_tiles, (int)nr, var + r0);
       h->st.kernel_launches++;
@@ -918,37 +831,35 @@ int run_sliced_variance(nngp_handle* h, const double* B, int64_t ldb, int64_t ro
 // (`Winv`: the inverses of L's 64 x 64 diagonal blocks, as the factorisation / run_trtri_diag leave them in h->Linv)
 int run_trsv_bwd(nngp_handle* h, const double* L, int64_t ld, int64_t N, double* z, double* out, const double* Winv) {
   const int64_t nblk = (N + NB - 1) / NB;
-  static const bool steps = [] { const char* e = getenv("NNGP_TRSV"); return e && !strcmp(e, "steps"); }();
-  if (!steps) {  // one persistent launch: column slices of SW, one CTA each, all co-resident (grid <= #SMs)
-    int64_t sw = 4 * NB;
-    while ((N + sw - 1) / sw > h->sm_count) sw += NB;
-    const int grid = (int)((N + sw - 1) / sw);
-    const size_t smem = (size_t)(NB * (NB + 1) + 2 * NB + sw) * sizeof(double);
-    if (smem <= 200 * 1024) {
-      CKR(ensure(h, h->sync_ints, (size_t)(nblk + 1) * sizeof(int)));
-      CK(cudaMemsetAsync(h->sync_ints.p, 0, (size_t)nblk * sizeof(int), h->stream));
-      CK(cudaFuncSetAttribute(trsv_bwd_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      // The kernel's CTAs wait on each other's flags, so they must all be resident: a cooperative launch makes the
-      // driver guarantee that (it waits for room when another handle or process holds SMs) instead of relying on
-      // the dispatch order; if the grid cannot be co-resident at all the stepwise kernels below take over.
-      int Ni = (int)N, swi = (int)sw;
-      const double* zc = z;
-      int* fl = h->sync_ints.as<int>();
-      void* args[] = {(void*)&L, (void*)&ld, (void*)&Ni, (void*)&swi, (void*)&zc, (void*)&out, (void*)&fl, (void*)&Winv};
-      cudaError_t le = cudaLaunchCooperativeKernel((const void*)trsv_bwd_persistent_kernel, dim3((unsigned)grid),
-                                                   dim3(TRSVP_THREADS), args, smem, h->stream);
-      if (le == cudaSuccess) {
-        h->st.kernel_launches++;
-        return NNGP_OK;
-      }
-      cudaGetLastError();   // not co-schedulable here: fall through to one launch per block
+  // one persistent launch: column slices of SW, one CTA each, all co-resident (grid <= #SMs)
+  int64_t sw = 4 * NB;
+  while ((N + sw - 1) / sw > h->sm_count) sw += NB;
+  const int grid = (int)((N + sw - 1) / sw);
+  const size_t smem = (size_t)(NB * (NB + 1) + 2 * NB + sw) * sizeof(double);
+  if (smem <= 200 * 1024) {
+    CKR(ensure(h, h->sync_ints, (size_t)(nblk + 1) * sizeof(int)));
+    CK(cudaMemsetAsync(h->sync_ints.p, 0, (size_t)nblk * sizeof(int), h->stream));
+    CK(cudaFuncSetAttribute(trsv_bwd_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    // The kernel's CTAs wait on each other's flags, so they must all be resident: a cooperative launch makes the
+    // driver guarantee that (it waits for room when another handle or process holds SMs) instead of relying on
+    // the dispatch order; if the grid cannot be co-resident at all the stepwise kernels below take over.
+    int Ni = (int)N, swi = (int)sw;
+    const double* zc = z;
+    int* fl = h->sync_ints.as<int>();
+    void* args[] = {(void*)&L, (void*)&ld, (void*)&Ni, (void*)&swi, (void*)&zc, (void*)&out, (void*)&fl, (void*)&Winv};
+    cudaError_t le = cudaLaunchCooperativeKernel((const void*)trsv_bwd_persistent_kernel, dim3((unsigned)grid),
+                                                 dim3(TRSVP_THREADS), args, smem, h->stream);
+    if (le == cudaSuccess) {
+      h->st.kernel_launches++;
+      return NNGP_OK;
     }
+    cudaGetLastError();   // not co-schedulable here: fall through to one launch per block
   }
   for (int64_t jb = nblk - 1; jb >= 0; --jb) {
     const int64_t j0 = jb * NB;
     const int64_t nb = std::min<int64_t>(NB, N - j0);
-    int grid = (int)std::min<int64_t>(std::max<int64_t>(1, (j0 + TRSV_THREADS - 1) / TRSV_THREADS), 4 * h->sm_count);
-    trsv_bwd_step_kernel<<<grid, TRSV_THREADS, 0, h->stream>>>(L, ld, (int)j0, (int)nb, z, out);
+    const int sgrid = (int)std::min<int64_t>(std::max<int64_t>(1, (j0 + TRSV_THREADS - 1) / TRSV_THREADS), 4 * h->sm_count);
+    trsv_bwd_step_kernel<<<sgrid, TRSV_THREADS, 0, h->stream>>>(L, ld, (int)j0, (int)nb, z, out);
     h->st.kernel_launches++;
   }
   CK(cudaGetLastError());
@@ -1228,11 +1139,10 @@ static int create_single(const nngp_config* cfg, nngp_handle** out) {
   cudaError_t e1 = cudaFuncSetAttribute(gemm_nt_kernel<EPI_GRAM>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES);
   cudaError_t e2 = cudaFuncSetAttribute(gemm_nt_kernel<EPI_SUB>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES);
   if (e2 == cudaSuccess) e2 = cudaFuncSetAttribute(gemm_nt_kernel<EPI_ROWDOT>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES);
-  cudaError_t e3 = cudaFuncSetAttribute(trsm_rows_64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TRSM_SMEM_BYTES);
-  if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(trsm_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TF_SMEM_BYTES);
+  cudaError_t e3 = cudaFuncSetAttribute(trsm_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TF_SMEM_BYTES);
   if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(trsm_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TF_SMEM_BYTES);
   if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(gemm_nt_kernel<EPI_DIAG>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES);
-  if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(potrf_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PANEL_SMEM_MAX);
+  if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(potrf_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TF_SMEM_BYTES);
   if (e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess) {
     fail(h, NNGP_ECUDA, "cudaFuncSetAttribute(max dynamic smem) failed: %s",
          cudaGetErrorString(e1 != cudaSuccess ? e1 : (e2 != cudaSuccess ? e2 : e3)));
@@ -2237,19 +2147,13 @@ int nngp_diag_potrf(nngp_handle* h, double* a, int64_t N) {
   if (!h || !a || N <= 0) return NNGP_EINVAL;
   CKR(bind_device(h));
   const int64_t ld = round_up(N, 16);
-  const int64_t extra = getenv("NNGP_DIAG_EXTRA") ? 1 : 0;  // debug: carry a row of ones like nngp_fit carries y^T
   DevBuf A;
-  CKR(ensure(h, A, (size_t)(N + extra) * ld * 8));
+  CKR(ensure(h, A, (size_t)N * ld * 8));
   int rc = NNGP_OK;
   cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream);
   rc = upload_matrix(h, a, N, N, A.as<double>(), ld);
-  if (rc == NNGP_OK && extra) {
-    std::vector<double> ones(N, 1.0);
-    cudaMemcpyAsync(A.as<double>() + N * ld, ones.data(), N * sizeof(double), cudaMemcpyHostToDevice, h->stream);
-    cudaStreamSynchronize(h->stream);
-  }
   if (rc == NNGP_OK) rc = ensure(h, h->panel_inv, (size_t)round_up(N, NB) * NB * sizeof(double));
-  if (rc == NNGP_OK) rc = run_potrf(h, A.as<double>(), ld, N, extra, h->panel_inv.as<double>());
+  if (rc == NNGP_OK) rc = run_potrf(h, A.as<double>(), ld, N, 0, h->panel_inv.as<double>());
   if (rc == NNGP_OK) rc = download(h, A.as<double>(), N, N, ld, a);
   int flags[2] = {0, 0};
   cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream);

@@ -1,8 +1,7 @@
 // dense_kernels.cuh -- the small kernels around the DMMA GEMM core:
 //   row_sqnorm / q_final          layer-0 kernel diagonal and K(x,x)            (K2, K9)
 //   diag_reg                      lambda = diag_reg * trace(K)/N ; K += lambda I (K4)
-//   potf2_64                      64x64 diagonal-block Cholesky, 4 x 4 register blocks            (K5 panel)
-//   trsm_rows_64                  X L_JJ^T = B, one thread per row                               (K5 panel)
+//   potf2_64_block                64x64 diagonal-block Cholesky, 4 x 4 register blocks            (K5 panel)
 //   trtri_diag                    inv(L_JJ) of every diagonal block: operand of the solves' diagonal step (K10)
 //   trsv_bwd_persistent / _step   backward substitution L^T alpha = z (the forward one rides through
 //                                 the Cholesky as an extra row of the factor buffer)              (K6)
@@ -177,8 +176,8 @@ __device__ __forceinline__ void store_inverse_64(const double (*Ls)[NB + 1], dou
   }
 }
 
-// Shared memory of one 64 x 64 block factorisation (45.9 KB): static in potf2_64_kernel, aliased onto the drained
-// operand ring in the fused panel kernel (potrf_panel.cuh).
+// Shared memory of one 64 x 64 block factorisation (45.9 KB), aliased onto the drained operand ring in the fused
+// panel kernel (potrf_panel.cuh).
 struct Potf2Smem {
   double Ld[2][4][4];     // factored diagonal 4 x 4 block (lower), double-buffered by micro-panel parity
   double Rinv[2][4];      // reciprocal pivots of its 4 columns
@@ -335,83 +334,8 @@ __device__ __forceinline__ int potf2_64_block(double* __restrict__ A, long long 
   return 0;
 }
 
-__global__ void __launch_bounds__(POTF2_THREADS, 1) potf2_64_kernel(double* __restrict__ A, long long ld, int n, int pivot0,
-                                                                    int* __restrict__ info, double* __restrict__ Winv) {
-  __shared__ Potf2Smem sm;
-  potf2_64_block(A, ld, n, pivot0, info, Winv, sm);
-}
-
-// X * Ljj^T = B in place, for `rows` rows of B (row-major, ldb) and the n x n (n <= 64) lower block
-// Ljj (row-major, ldl).  128 rows per CTA, one thread per row.  The row lives in 64 registers and is
-// solved right-looking (x_j = b_j / l_jj ; b_k -= x_j l_kj for k > j): 63-j independent FMAs per step, so
-// the substitution is issue-bound instead of latency-bound.  Global traffic is staged through smem so
-// that it stays coalesced; loads are batched 8 deep per thread.
-constexpr int TRSM_ROWS = 128;
-constexpr int TRSM_SMEM_BYTES = (TRSM_ROWS * (NB + 1) + NB * (NB + 2) + NB) * 8;
-
-// solve one row held in x[0..63] against Lt (Lt[j][k] = L[k][j], row pitch NB+2 doubles) and rdiag
-__device__ __forceinline__ void solve_row_regs(double (&x)[NB], const double* __restrict__ Lt,
-                                               const double* __restrict__ rdiag) {
-#pragma unroll
-  for (int j = 0; j < NB; ++j) {
-    x[j] *= rdiag[j];
-    const double xj = x[j];
-    const double* lt = Lt + j * (NB + 2);
-#pragma unroll
-    for (int k = j + 1; k < NB; ++k) x[k] = fma(-xj, lt[k], x[k]);
-  }
-}
-
-__global__ void __launch_bounds__(TRSM_ROWS) trsm_rows_64_kernel(double* __restrict__ B, long long ldb, int rows,
-                                                                const double* __restrict__ Ljj, long long ldl,
-                                                                int n) {
-  extern __shared__ double sm[];
-  double(*Bs)[NB + 1] = reinterpret_cast<double(*)[NB + 1]>(sm);
-  double* Lt = sm + TRSM_ROWS * (NB + 1);            // [NB][NB+2], transposed diagonal block
-  double* rdiag = Lt + NB * (NB + 2);
-  const int tid = threadIdx.x;
-  const int row0 = blockIdx.x * TRSM_ROWS;
-  const int c = tid & 63, rsub = tid >> 6;  // thread covers column c of rows rsub, rsub+2, ...
-  for (int r0 = 0; r0 < NB; r0 += 16) {
-    double t[8];
-#pragma unroll
-    for (int u = 0; u < 8; ++u) {
-      const int r = r0 + 2 * u + rsub;
-      t[u] = (r < n && c <= r) ? __ldcg(Ljj + (long long)r * ldl + c) : ((r == c) ? 1.0 : 0.0);
-    }
-#pragma unroll
-    for (int u = 0; u < 8; ++u) Lt[c * (NB + 2) + r0 + 2 * u + rsub] = t[u];   // Lt[c][r] = L[r][c]
-  }
-  for (int r0 = 0; r0 < TRSM_ROWS; r0 += 16) {
-    double t[8];
-#pragma unroll
-    for (int u = 0; u < 8; ++u) {
-      const int r = r0 + 2 * u + rsub;
-      t[u] = (row0 + r < rows && c < n) ? __ldcg(B + (long long)(row0 + r) * ldb + c) : 0.0;
-    }
-#pragma unroll
-    for (int u = 0; u < 8; ++u) Bs[r0 + 2 * u + rsub][c] = t[u];
-  }
-  __syncthreads();
-  if (tid < NB) rdiag[tid] = 1.0 / Lt[tid * (NB + 2) + tid];
-  __syncthreads();
-  {
-    double x[NB];
-#pragma unroll
-    for (int j = 0; j < NB; ++j) x[j] = Bs[tid][j];
-    solve_row_regs(x, Lt, rdiag);
-#pragma unroll
-    for (int j = 0; j < NB; ++j) Bs[tid][j] = x[j];
-  }
-  __syncthreads();
-  for (int r0 = 0; r0 < TRSM_ROWS; r0 += 2) {
-    const int r = r0 + rsub;
-    if (row0 + r < rows && c < n) B[(long long)(row0 + r) * ldb + c] = Bs[r][c];
-  }
-}
-
 // W_J = inv(L_JJ) for every 64 x 64 diagonal block of the factor (identity padded when the last block is short):
-// one CTA per block, the SAME routine (invert_lower_64_inplace) the factorisation's potf2_64_kernel runs on the block it has
+// one CTA per block, the SAME routine (invert_lower_64_inplace) the factorisation's potf2_64_block runs on the block it has
 // just factored -- so a state that was imported (nngp_set_state / nngp_state_import_end) predicts with bitwise the
 // inverses of the handle that fitted it.  Output: row-major 64 x 64 blocks stacked along the rows (block J at rows
 // [64 J, 64 J + 64)), the B operand of the diagonal step of the row-wise triangular solves.

@@ -12,8 +12,8 @@
 //                                                                         gates every TMA issue on progress[r] (A
 //                                                                         operand) and progress[J / 2] (the rows of
 //                                                                         diagonal block J live in row tile J / 2)
-//     owner (r == J / 2):  R -> global;  potf2_64_block on the diagonal block (factor + inverse, the code of
-//                          potf2_64_kernel, its shared memory aliased onto the drained ring);  publish inv_ready[J]
+//     owner (r == J / 2):  R -> global;  potf2_64_block on the diagonal block (factor + inverse, its shared memory
+//                          aliased onto the drained ring);  publish inv_ready[J]
 //     everyone:            V[r, J] = R W_J^T  on the tensor pipe (the diagonal step of trsm_fused.cuh), rows strictly
 //                          below the diagonal block only;  publish progress[r] = J + 1
 // Items above the diagonal are skipped.  Items are claimed in J-major order from a counter, so whatever an item waits

@@ -27,7 +27,6 @@
 // inside, the 4 column tiles of one pair adjacent -- CTAs 4k..4k+3 stream the same K_* planes (the second to fourth
 // read hit L2, sparing HBM) and all CTAs of a wave stream the same W planes.  That only holds while the CTAs stay in
 // step, so the producers re-align at a grid-wide counter at every tile (wave_barrier): DRAM reads -55 %, +6.6 %.
-// Clusters of two CTAs with TMA multicast of the W stages (template CL = 2) are bit-identical but slower; kept for A/B.
 #pragma once
 #include "ptx.cuh"
 
@@ -47,8 +46,6 @@ constexpr int SL_SUPER = 4;                // column tiles per supercolumn
 constexpr int SL_MAX_SLICES = 9;
 constexpr int SL_SMEM_BYTES = SL_STAGES * (SL_A_BYTES + SL_B_BYTES) + 1024 /*alignment*/ + 256 /*barriers*/;
 constexpr int SL_SLICE_THREADS = 256;
-constexpr int SL_CLUSTER_DEFAULT = 1;      // CTAs per cluster (NNGP_SLICED_CLUSTER=1|2): 2 = W stages by TMA multicast
-constexpr int SL_SYNC_DEFAULT = 1;         // wave re-alignment at every tile (NNGP_SLICED_SYNC=0|1|2): see wave_barrier
 
 struct SlicedParams {
   int s;                   // digit planes per operand
@@ -57,7 +54,6 @@ struct SlicedParams {
   int K;                   // inner dimension (= N for the triangular W)
   int row_tiles, col_tiles;
   int tri;                 // W lower triangular: column tile j needs K < 256 (j + 1) only
-  int rt;                  // row tiles per CTA tile: 2 (both accumulators); 1 = A/B variant (more, lighter tiles; slower)
   long long ra, rb;        // rows per plane in the stacked plane arrays of K_* / W
   const double* rscale;    // [rows]  2^(e-6) of the K_* rows
   const double* cscale;    // [N]     2^(e-6) of the W rows
@@ -68,9 +64,8 @@ struct SlicedParams {
   int skip_weak;           // 1 (variance path): drop the pair (A plane s-1, W plane 0).  A row of W = L^-1 is dominated by
                            // its diagonal entry, so plane 0 of W holds digits 0 / +-1 almost everywhere and this pair
                            // weighs like the first DROPPED group (tools/ozaki_pairskip_study.py): 1 / 28 of the MACs
-  int cl;                  // CTAs per cluster sharing every W stage by TMA multicast: 1 or 2 (== the kernel's template argument)
-  int* wave_sync;          // sync_mode > 0: one arrival counter per tile round (x s for per-group syncs), zeroed before launch
-  int sync_mode;           // 0: free-running CTAs; 1: the producers re-align at every tile; 2: at every digit group
+  int* wave_sync;          // one arrival counter per tile round, zeroed before a cooperative launch: the producers
+                           // re-align at every tile (wave_barrier); null: free-running CTAs
 };
 
 // ---- digit planes ---------------------------------------------------------------------------------------------
@@ -135,28 +130,6 @@ __device__ __forceinline__ void tc_mma_i8(uint32_t tmem_d, uint64_t desc_a, uint
       ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-__device__ __forceinline__ void tc_commit_mc(uint64_t* bar, uint16_t cta_mask) {   // same, on `bar` of every CTA in the mask
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)), "h"(cta_mask)
-               : "memory");
-}
-// TMA load delivered to the same shared-memory offset (and signalled on the same mbarrier offset) of every CTA in the mask
-__device__ __forceinline__ void tma_load_2d_mc(void* smem_dst, const CUtensorMap* tmap, int c0, int c1, uint64_t* bar,
-                                               uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%2, %3}], [%4], %5;" ::"r"(smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1), "r"(smem_u32(bar)), "h"(cta_mask)
-      : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_rank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
 // shared-memory matrix descriptor: K-major, 128-byte swizzle, rows 128 B apart, 8-row groups 1024 B apart
 __device__ __forceinline__ uint64_t tc_smem_desc(uint32_t smem_addr) {
   return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) | (1ull << 16) /*LBO (unused)*/ | (64ull << 32) /*SBO = 1024 B*/ |
@@ -183,9 +156,7 @@ __device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&r)[32]) {   /
 // ---- tile order -------------------------------------------------------------------------------------------------
 struct SlicedTile { int ip, jt, nkb; };   // row-tile pair, column tile, K blocks
 __device__ __forceinline__ bool sliced_tile(const SlicedParams& p, long long idx, SlicedTile& t) {
-  // cl = 2: consecutive tile indices (= the two CTAs of a cluster) are two row pairs of the SAME column tile, so that
-  // they can share its W stages; the pair count is rounded up to even (a phantom pair computes on padding, writes nothing)
-  const int row_pairs = ((p.row_tiles + p.rt - 1) / p.rt + p.cl - 1) / p.cl * p.cl;
+  const int row_pairs = (p.row_tiles + SL_RT - 1) / SL_RT;
   const long long total = (long long)row_pairs * p.col_tiles;
   if (idx >= total) return false;
   const int nsup = (p.col_tiles + SL_SUPER - 1) / SL_SUPER;
@@ -194,14 +165,12 @@ __device__ __forceinline__ bool sliced_tile(const SlicedParams& p, long long idx
   int sup, c;
   if (idx < first) {
     sup = nsup - 1;
-    const long long q = idx / p.cl;
-    t.ip = (int)(q / wlast) * p.cl + (int)(idx % p.cl); c = (int)(q % wlast);
+    t.ip = (int)(idx / wlast); c = (int)(idx % wlast);
   } else {
     const long long r = idx - first, per = (long long)row_pairs * SL_SUPER;
     sup = nsup - 2 - (int)(r / per);
     const long long in = r % per;
-    const long long q = in / p.cl;
-    t.ip = (int)(q / SL_SUPER) * p.cl + (int)(in % p.cl); c = (int)(q % SL_SUPER);
+    t.ip = (int)(in / SL_SUPER); c = (int)(in % SL_SUPER);
   }
   t.jt = sup * SL_SUPER + c;
   // the whole supercolumn runs the K extent of its last column tile, so that its CTAs stay in lockstep
@@ -226,10 +195,6 @@ __device__ __forceinline__ void wave_barrier(int* counter, int participants) {
 }
 
 // ---- the kernel -------------------------------------------------------------------------------------------------
-// CL = 2: launched as clusters of two CTAs (same column tile, neighbouring row pairs).  Each CTA fetches HALF of the
-// W stage (128 rows, tensor map tmB with a 128-row box) and TMA-multicasts it into both CTAs, so every W byte crosses
-// the L2 -> SM fabric once per cluster; a stage is free when BOTH CTAs' MMAs have read it (multicast tcgen05.commit).
-template <int CL>
 __global__ void __launch_bounds__(SL_THREADS, 1)
 sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                    const SlicedParams p) {
@@ -248,7 +213,7 @@ sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   const int lane = threadIdx.x & 31;
 
   if (threadIdx.x == 0) {
-    for (int i = 0; i < SL_STAGES; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], CL); }
+    for (int i = 0; i < SL_STAGES; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
     mbar_init(acc_full, 1);
     mbar_init(acc_empty, 32 * SL_EPI_WARPS);
     fence_mbar_init();
@@ -264,38 +229,27 @@ sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_slot);
-  uint32_t crank = 0;
-  if constexpr (CL > 1) {   // the peer's barriers must exist before a multicast load or commit can reach them
-    cluster_sync_all();
-    crank = cluster_rank();
-  }
-  constexpr uint16_t cl_mask = (uint16_t)((1u << CL) - 1u);
 
   if (warp == 0) {
     if (lane == 0) {   // ===== TMA producer =====
       uint32_t n = 0;
       SlicedTile t;
-      const long long total = (long long)(((p.row_tiles + p.rt - 1) / p.rt + p.cl - 1) / p.cl * p.cl) * p.col_tiles;
+      const long long total = (long long)((p.row_tiles + SL_RT - 1) / SL_RT) * p.col_tiles;
       int round = 0;
       for (long long idx = blockIdx.x; sliced_tile(p, idx, t); idx += gridDim.x, ++round) {
-        const int participants = (int)min((long long)gridDim.x, total - (long long)round * gridDim.x);
+        if (p.wave_sync != nullptr)
+          wave_barrier(p.wave_sync + round, (int)min((long long)gridDim.x, total - (long long)round * gridDim.x));
         for (int g = p.s - 1; g >= 0; --g) {
-          if (p.sync_mode == 2 || (p.sync_mode == 1 && g == p.s - 1))
-            wave_barrier(p.wave_sync + (p.sync_mode == 2 ? round * p.s + g : round), participants);
           const int pa_last = (p.skip_weak && g == p.s - 1 && g > 0) ? g - 1 : g;
           for (int pa = 0; pa <= pa_last; ++pa) {
-            const int a_row = (int)(pa * p.ra) + t.ip * (p.rt * SL_BM);   // (rt = 1: the second half of the box is not used)
+            const int a_row = (int)(pa * p.ra) + t.ip * (SL_RT * SL_BM);
             const int b_row = (int)((g - pa) * p.rb) + t.jt * SL_BN;
             for (int kb = 0; kb < t.nkb; ++kb, ++n) {
               const uint32_t st = n % SL_STAGES, ph = (n / SL_STAGES) & 1u;
               mbar_wait(&empty_bar[st], ph ^ 1u);
               mbar_arrive_expect_tx(&full_bar[st], SL_A_BYTES + SL_B_BYTES);
               tma_load_2d(ringA + st * SL_A_BYTES, &tmA, kb * SL_BK, a_row, &full_bar[st]);   // both row tiles: 256 rows
-              if constexpr (CL == 1)
-                tma_load_2d(ringB + st * SL_B_BYTES, &tmB, kb * SL_BK, b_row, &full_bar[st]);
-              else        // my half of the W stage, into both CTAs (the peer sends the other half)
-                tma_load_2d_mc(ringB + st * SL_B_BYTES + crank * (SL_B_BYTES / CL), &tmB, kb * SL_BK,
-                               b_row + (int)crank * (SL_BN / CL), &full_bar[st], cl_mask);
+              tma_load_2d(ringB + st * SL_B_BYTES, &tmB, kb * SL_BK, b_row, &full_bar[st]);
             }
           }
         }
@@ -306,7 +260,7 @@ sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       uint32_t n = 0, a = 0;
       SlicedTile t;
       for (long long idx = blockIdx.x; sliced_tile(p, idx, t); idx += gridDim.x) {
-        const bool two = p.rt == 2 && t.ip * 2 + 1 < p.row_tiles;     // the second row tile exists
+        const bool two = t.ip * 2 + 1 < p.row_tiles;     // the second row tile exists
         for (int g = p.s - 1; g >= 0; --g, ++a) {
           mbar_wait(acc_empty, (a & 1u) ^ 1u);              // the epilogue has drained both accumulators
           tc_fence_after();
@@ -326,8 +280,7 @@ sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                 if (two) tc_mma_i8(tmem_base + SL_BN, da1 + 2u * k, db + 2u * k, SL_IDESC, acc);
                 acc = 1;
               }
-              if constexpr (CL == 1) tc_commit(&empty_bar[st]);          // stage free once these MMAs have read it
-              else tc_commit_mc(&empty_bar[st], cl_mask);               // ... in every CTA that multicasts into it
+              tc_commit(&empty_bar[st]);                     // stage free once these MMAs have read it
             }
           tc_commit(acc_full);                           // group complete: hand the accumulators to the epilogue
         }
@@ -341,7 +294,7 @@ sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
     uint32_t a = 0;
     SlicedTile t;
     for (long long idx = blockIdx.x; sliced_tile(p, idx, t); idx += gridDim.x) {
-      const int ntile = (p.rt == 2 && t.ip * 2 + 1 < p.row_tiles) ? 2 : 1;
+      const int ntile = (t.ip * 2 + 1 < p.row_tiles) ? 2 : 1;
       double sum[SL_RT] = {0.0, 0.0};
       for (int g = p.s - 1; g >= 0; --g, ++a) {
         mbar_wait(acc_full, a & 1u);
@@ -349,7 +302,7 @@ sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         tc_fence_after();
         const bool first = (g == p.s - 1);
         for (int h = 0; h < ntile; ++h) {
-          const int grow = (t.ip * p.rt + h) * SL_BM + row;
+          const int grow = (t.ip * SL_RT + h) * SL_BM + row;
           const double rs = (grow < p.rows) ? p.rscale[grow] : 0.0;
           const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + h * SL_BN + half * (SL_BN / 2);
           double* sch = sc + (h * SL_BN + half * (SL_BN / 2)) * SL_BM;
@@ -381,7 +334,7 @@ sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       }
       if (p.vpart)
         for (int h = 0; h < ntile; ++h) {
-          const int grow = (t.ip * p.rt + h) * SL_BM + row;
+          const int grow = (t.ip * SL_RT + h) * SL_BM + row;
           if (grow < p.rows) p.vpart[((long long)t.jt * 2 + half) * p.rows + grow] = sum[h];   // two partials per column tile
         }
     }
@@ -389,7 +342,6 @@ sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 
   tc_fence_before();
   __syncthreads();
-  if constexpr (CL > 1) cluster_sync_all();   // no CTA leaves while its peer may still write into it / arrive on its barriers
   if (warp == 1) {
     __syncwarp();
     tc_fence_after();

@@ -31,4 +31,4 @@ for r in range(reps):
     if not same:
         bad += 1
         print(f"rep {r}: MISMATCH alpha rel {da:.3e} mean abs {dm:.3e} var rel {dv:.3e}", flush=True)
-print(f"N={n} reps={reps} lookahead={os.environ.get('NNGP_CHOL_LOOKAHEAD', '1')} la_mode={os.environ.get('NNGP_LA_MODE', '1')} W={os.environ.get('NNGP_CHOL_W')} mismatches={bad}")
+print(f"N={n} reps={reps} lookahead={os.environ.get('NNGP_CHOL_LOOKAHEAD', '1')} mismatches={bad}")

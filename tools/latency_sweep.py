@@ -1,5 +1,5 @@
 """nngp_predict latency at small and medium batch sizes, default handle vs latency mode (explicit L^-1), plus fit
-times with the pieces of the Cholesky panel chain (A/B of the panel solve).  Host numpy buffers in, mean + variance
+times with the pieces of the Cholesky (Gram, factorisation, solve).  Host numpy buffers in, mean + variance
 out, wall clock around the C-ABI call, averages after warm-up.  Prints one JSON object.
     python tools/latency_sweep.py [N] [D]"""
 import json
@@ -62,7 +62,7 @@ out["flop_floor_ms_1024_rows"] = 1024 * (float(N) * N + 2.0 * N * D) / 37.0e12 *
 hl.close()
 hl2.close()
 
-# fit times: N sweep, default panel solve (DMMA) -- the 'fma' A/B needs a fresh process (the switch is read once)
+# fit times: N sweep (the key names the panel solve, a DMMA product, as in the earlier sweeps under profiles/)
 fits = {}
 for n in (2048, 4096, 8192, 16384):
     if n > N and n > 16384:
@@ -78,5 +78,5 @@ for n in (2048, 4096, 8192, 16384):
     fits[str(n)] = {"fit_total_ms": s["fit_total_ms"] / 3, "chol_ms": s["fit_chol_ms"] / 3, "gram_ms": s["fit_gram_ms"] / 3,
                     "solve_ms": s["fit_solve_ms"] / 3, "chol_tflops": n**3 / 3 / (s["fit_chol_ms"] / 3) / 1e9}
     hf.close()
-out["fit_ms_panel_" + os.environ.get("NNGP_PANEL_SOLVE", "dmma")] = fits
+out["fit_ms_panel_dmma"] = fits
 print(json.dumps(out, indent=1))
