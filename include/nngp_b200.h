@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define NNGP_B200_ABI_VERSION 6
+#define NNGP_B200_ABI_VERSION 7
 #define NNGP_MAX_GPUS 8
 #define NNGP_MAX_LAYERS 16
 
@@ -118,6 +118,7 @@ typedef struct nngp_stats_t {
   double inverse_ms;       /* latency_mode: device time of building L^-1 in the last fit */
   double sliced_ms;        /* variance_slices: device time of digit-plane splitting + the int8 plane products   */
   double sliced_macs;      /* int8 multiply-accumulates issued to the tensor cores in them                       */
+  int64_t device_allocs;   /* device buffer allocations (cudaMalloc); 0 between rounds after nngp_reserve        */
 } nngp_stats_t;
 
 typedef struct nngp_handle nngp_handle;
@@ -146,7 +147,8 @@ NNGP_API void* nngp_get_stream(nngp_handle* h);
  *
  * Accepted input range (nngp_kernel, nngp_fit, nngp_append_fit, nngp_predict): every element finite, and every
  * row's layer-0 diagonal q = sigma_w^2 |x|^2 / D + sigma_b^2 below 2^512, so that q q' is a finite double;
- * anything else is NNGP_EINVAL.  There is no lower bound: rows down to the subnormal range (and zero rows) are
+ * anything else is NNGP_EINVAL.  nngp_set_state and nngp_state_import_end hold the imported X to the same range
+ * (NNGP_EINVAL, the handle is left without a fitted model).  There is no lower bound: rows down to the subnormal range (and zero rows) are
  * accepted, but an entry whose q, q q' or k^2 is subnormal carries fewer significant bits.
  */
 NNGP_API int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2_or_null, int64_t N2,

@@ -76,7 +76,7 @@ struct nngp_handle {
   int64_t N = 0, D = 0, ldx = 0, ldl = 0;
   double lambda = 0.0;
   double lml_terms[2] = {0.0, 0.0};  // {sum log diag(L), y^T (K+lambda I)^-1 y}; valid after nngp_fit
-  bool have_lml = false;
+  bool have_labels = false;   // fitted from labels on this handle (nngp_fit / nngp_append_fit): y, z and lml_terms are valid
   bool have_M = false;   // NTK mode: M = L^-1 K_dd L^-T is present (nngp_fit or nngp_set_state_ntk_m)
   DevBuf X, q, L, alpha;
   DevBuf Linv;    // inv(L_JJ) of every 64 x 64 diagonal block of L (trtri_diag_kernel), operand of the solves' diagonal step
@@ -93,7 +93,6 @@ struct nngp_handle {
   bool have_wq = false;
   int64_t wq_ldq = 0, wq_rb = 0;
   DevBuf L2;      // second factor buffer: target of the incremental (fixed-lambda) append, then swapped with L
-  bool have_y = false;
   bool importing = false;   // between nngp_state_import_begin and _end
   DevBuf flags;   // int[2]: {potrf info, non-finite input}
   DevBuf lam_d;   // double[4]: {lambda, sum log diag L, z^T z, spare}
@@ -104,6 +103,7 @@ struct nngp_handle {
   DevBuf Mmat, Kdd, blk2, cross, partial, mean_partial;
   // nngp_kernel workspace
   DevBuf ka, kb, kqa, kqb, kout;
+  DevBuf stage;   // nngp_state_pack / _unpack with host memory on the other side: one range at a time
   // nngp_active_select workspace
   DevBuf sel_mean, sel_var, sel_score, sel_key, sel_state, sel_okey, sel_oidx, sel_max;
 
@@ -156,7 +156,7 @@ int ensure(nngp_handle* h, DevBuf& b, size_t bytes) {
   // multi-GB cudaFree / cudaMalloc pairs do not recur every round; exact size if that does not fit.
   if (regrow && bytes >= (64u << 20)) {
     const size_t roomy = bytes + bytes / 4;
-    if (cudaMalloc(&b.p, roomy) == cudaSuccess) { b.cap = roomy; return NNGP_OK; }
+    if (cudaMalloc(&b.p, roomy) == cudaSuccess) { b.cap = roomy; h->st.device_allocs++; return NNGP_OK; }
     b.p = nullptr;
     cudaGetLastError();
   }
@@ -167,6 +167,7 @@ int ensure(nngp_handle* h, DevBuf& b, size_t bytes) {
     return fail(h, NNGP_ENOMEM, "cudaMalloc(%zu bytes) failed: %s", bytes, cudaGetErrorString(e));
   }
   b.cap = bytes;
+  h->st.device_allocs++;
   return NNGP_OK;
 }
 
@@ -355,6 +356,147 @@ int chol_outer_width(int64_t N) {
   return N >= 24576 ? 1024 : (N >= 4096 ? 512 : 256);
 }
 
+// ---- device buffer sizes ----------------------------------------------------------------------------
+// Every size passed to ensure() for a buffer of the handle comes from one function here, which both the code using the
+// buffer and nngp_reserve call: a reserved handle never reallocates.
+
+bool builds_inverse(const nngp_handle* h) { return h->cfg.latency_mode && h->cfg.kernel_type == 0; }   // L^-1
+bool can_append_incrementally(const nngp_handle* h) { return h->cfg.diag_reg_absolute && h->cfg.kernel_type == 0; }
+
+// fused panel kernel of an N-column factorisation of R rows: {item counter, progress[row tiles], inv_ready[col blocks]}
+int ensure_panel_sync(nngp_handle* h, int64_t N, int64_t R) {
+  return ensure(h, h->panel_sync, (size_t)(2 + (R + GEMM_BM - 1) / GEMM_BM + (chol_outer_width(N) + NB - 1) / NB) * sizeof(int));
+}
+
+// solves over `rows` rows: sums of squares per row, counters of trsm_fused (per 128-row tile) / trsv_bwd (per 64-block)
+int ensure_solve_workspace(nngp_handle* h, int64_t rows) {
+  CKR(ensure(h, h->ssq, (size_t)rows * sizeof(double)));
+  return ensure(h, h->sync_ints, (size_t)((rows + NB - 1) / NB + 1) * sizeof(int));
+}
+
+// Rows per sub-block of run_sliced_variance: its planes fit 16 GiB, in whole waves of 37 row tiles x 4 column tiles (so
+// that the static tile order stays balanced).
+int64_t sliced_rows(const nngp_handle* h, int64_t N, int64_t rows) {
+  const int64_t wave_rows = (int64_t)(h->sm_count / SL_SUPER) * SL_RT * SL_BM;
+  const int64_t sb = ((16LL << 30) / ((int64_t)h->cfg.variance_slices * round_up(N, SL_BK))) / wave_rows * wave_rows;
+  return std::min<int64_t>(std::max<int64_t>(sb, SL_RT * SL_BM), round_up(rows, SL_RT * SL_BM));
+}
+
+// launch_sliced over rows x N: CTAs 4k..4k+3 share K_* row tiles; per-CTA running-sum tiles, one counter per round
+int sliced_grid(nngp_handle* h, int64_t rows, int64_t N, int* grid, int64_t* rounds) {
+  const int64_t tiles = ((rows + SL_BM - 1) / SL_BM + SL_RT - 1) / SL_RT * ((N + SL_BN - 1) / SL_BN);
+  *grid = (int)std::min<int64_t>((h->sm_count / SL_SUPER) * SL_SUPER, tiles);
+  *rounds = (tiles + *grid - 1) / *grid;
+  CKR(ensure(h, h->slscratch, (size_t)*grid * SL_RT * SL_BM * SL_BN * sizeof(double)));
+  return *rounds >= 2 ? ensure(h, h->slsync, (size_t)*rounds * sizeof(int)) : NNGP_OK;
+}
+
+// h->partial of a variance over `rows` rows, whichever path runs: the 'ntk' row-dot and the widest split of
+// run_inverse_variance (tri_gemv; <= 8 K chunks, only while rows x N spans < 4 tiles per SM; one per column tile), and
+// run_sliced_variance.  Non-decreasing in N and rows, so the largest problem's size covers the smaller ones.
+size_t partial_bytes(const nngp_handle* h, int64_t N, int64_t rows) {
+  int64_t n = rows * ((N + GEMM_BN - 1) / GEMM_BN);
+  if (builds_inverse(h)) {
+    const int64_t chunks = std::min<int64_t>(8, ((N + GEMM_BK - 1) / GEMM_BK + 63) / 64);
+    n = std::max({n, std::min<int64_t>(rows, TGV_MAXR) * N, chunks * std::min<int64_t>(rows * N, 4LL * h->sm_count * GEMM_BM * GEMM_BN)});
+    if (h->cfg.variance_slices > 0) n = std::max(n, 2 * ((N + SL_BN - 1) / SL_BN) * sliced_rows(h, N, rows));
+  }
+  return (size_t)n * sizeof(double);
+}
+
+// run_sliced_variance over `rows` rows: K_* digit planes and row scales of a sub-block, partials, launch workspace
+int ensure_sliced_block(nngp_handle* h, int64_t N, int64_t rows) {
+  const int64_t sb = sliced_rows(h, N, rows);
+  int grid;
+  int64_t rounds;
+  CKR(ensure(h, h->Aq, (size_t)h->cfg.variance_slices * sb * round_up(N, SL_BK)));
+  CKR(ensure(h, h->ascale, (size_t)sb * sizeof(double)));
+  CKR(ensure(h, h->partial, partial_bytes(h, N, rows)));
+  return sliced_grid(h, sb, N, &grid, &rounds);
+}
+
+// the training rows X and their layer-0 diagonals q
+int ensure_inputs(nngp_handle* h, int64_t N, int64_t D) {
+  CKR(ensure(h, h->X, (size_t)N * round_up(D, 2) * sizeof(double)));
+  return ensure(h, h->q, (size_t)N * sizeof(double));
+}
+
+// A fitted state of N x D, on every handle that holds one (replicas too): X, q, L (+1 row: y^T rides through the
+// factorisation), alpha, inv(L_JJ); M ('ntk'); in latency mode L^-1 and, with variance_slices, its digit planes.
+int ensure_model(nngp_handle* h, int64_t N, int64_t D) {
+  const int64_t ldl = round_up(N, 16), ldq = round_up(N, SL_BK);
+  const int s = h->cfg.variance_slices;
+  CKR(ensure_inputs(h, N, D));
+  CKR(ensure(h, h->L, (size_t)(N + 1) * ldl * sizeof(double)));
+  CKR(ensure(h, h->alpha, (size_t)ldl * sizeof(double)));
+  CKR(ensure(h, h->Linv, (size_t)round_up(N, NB) * NB * sizeof(double)));
+  if (h->cfg.kernel_type == 1) CKR(ensure(h, h->Mmat, (size_t)N * ldl * sizeof(double)));
+  if (builds_inverse(h)) CKR(ensure(h, h->Linvfull, (size_t)N * ldl * sizeof(double)));
+  if (s <= 0) return NNGP_OK;
+  if ((int64_t)s * 4096 * ldq >= (1LL << 31))
+    return fail(h, NNGP_EINVAL, "variance_slices = %d: int32 plane sums need N <= %lld (N = %lld)", s,
+                (long long)((1LL << 19) / s), (long long)N);
+  CKR(ensure(h, h->Wq, (size_t)s * round_up(N, SL_BN) * ldq));
+  return ensure(h, h->wscale, (size_t)N * sizeof(double));
+}
+
+// Only the handle that fits N rows: y, z = L^-1 y, the panel counters of the (N + 1)-row factorisation, K_dd ('ntk')
+// or the scratch of L^-T (latency mode), and the solves over N rows ('ntk' M, build_inverse, the alpha solve).
+int ensure_fit_workspace(nngp_handle* h, int64_t N) {
+  CKR(ensure(h, h->y, (size_t)N * sizeof(double)));
+  CKR(ensure(h, h->zkeep, (size_t)N * sizeof(double)));
+  CKR(ensure_panel_sync(h, N, N + 1));
+  if (h->cfg.kernel_type == 1 || builds_inverse(h)) CKR(ensure(h, h->Kdd, (size_t)N * round_up(N, 16) * sizeof(double)));
+  return ensure_solve_workspace(h, N);
+}
+
+// nngp_append_fit up to N x D: the staging [X; X_new], [y; y_new]; for the incremental append the second factor and
+// the inverses of the Schur block (at most N rows)
+int ensure_append_workspace(nngp_handle* h, int64_t N, int64_t D) {
+  CKR(ensure(h, h->app_x, (size_t)N * D * sizeof(double)));
+  CKR(ensure(h, h->app_y, (size_t)N * sizeof(double)));
+  if (!can_append_incrementally(h)) return NNGP_OK;
+  CKR(ensure(h, h->L2, (size_t)(N + 1) * round_up(N, 16) * sizeof(double)));
+  return ensure(h, h->panel_inv, (size_t)round_up(N, NB) * NB * sizeof(double));
+}
+
+// Rows per block of nngp_predict: what fits cfg.max_block_bytes (the 'ntk' variance holds two blocks), in equal blocks
+// of whole 128-row tiles -- the persistent solve keeps every SM busy with any tile count, what hurts is a last block
+// with too few row tiles to fill the GPU.
+int64_t predict_block_rows(const nngp_handle* h, int64_t N, int64_t T, bool want_var) {
+  int64_t cap_rows = h->cfg.max_block_bytes / (round_up(N, 16) * 8) / (h->cfg.kernel_type == 1 && want_var ? 2 : 1);
+  cap_rows = std::min<int64_t>(std::max<int64_t>(cap_rows, GEMM_BM), 65535LL * GEMM_BM);
+  const int64_t nblocks = (T + cap_rows - 1) / cap_rows;
+  return std::min<int64_t>(round_up(T, 2), round_up((T + nblocks - 1) / nblocks, GEMM_BM));
+}
+
+// nngp_predict of T rows against N x D training rows
+int ensure_predict_workspace(nngp_handle* h, int64_t N, int64_t D, int64_t T, bool want_var) {
+  const int64_t TB = predict_block_rows(h, N, T, want_var), ldl = round_up(N, 16);
+  const bool ntk = h->cfg.kernel_type == 1;
+  for (DevBuf* b : {&h->qt, &h->kss}) CKR(ensure(h, *b, (size_t)TB * sizeof(double)));
+  CKR(ensure(h, h->xt, (size_t)TB * round_up(D, 2) * sizeof(double)));
+  CKR(ensure(h, h->blk, (size_t)TB * ldl * sizeof(double)));
+  CKR(ensure(h, h->mean_partial, (size_t)TB * 2 * ((N + GEMM_BN - 1) / GEMM_BN) * sizeof(double)));  // per 32 columns
+  CKR(ensure(h, h->mean_d, (size_t)T * sizeof(double)));
+  if (!want_var) return NNGP_OK;
+  CKR(ensure(h, h->var_d, (size_t)T * sizeof(double)));
+  CKR(ensure_solve_workspace(h, TB));
+  if (ntk) CKR(ensure(h, h->blk2, (size_t)TB * ldl * sizeof(double)));
+  if (ntk) CKR(ensure(h, h->cross, (size_t)TB * sizeof(double)));
+  if (ntk || builds_inverse(h)) CKR(ensure(h, h->partial, partial_bytes(h, N, TB)));
+  return h->cfg.variance_slices > 0 ? ensure_sliced_block(h, N, TB) : NNGP_OK;
+}
+
+// nngp_active_select of k out of T pool rows
+int ensure_select_workspace(nngp_handle* h, int64_t T, int64_t k) {
+  for (DevBuf* b : {&h->sel_mean, &h->sel_var, &h->sel_score, &h->sel_key}) CKR(ensure(h, *b, (size_t)T * 8));
+  CKR(ensure(h, h->sel_okey, (size_t)k * 8));
+  CKR(ensure(h, h->sel_oidx, (size_t)k * 4));
+  CKR(ensure(h, h->sel_state, sizeof(SelectState)));
+  return ensure(h, h->sel_max, 8);
+}
+
 // One outer panel, columns [j0, j0 + w) of the rows from j0 down to `R` = N + extra rows riding along below the
 // matrix (see run_potrf), as one persistent kernel (potrf_panel.cuh).  Per 64-wide sub-panel: the left-looking
 // update from the panel's earlier columns, potf2_64_block (Cholesky of the diagonal block AND its inverse
@@ -434,8 +576,7 @@ int run_potrf(nngp_handle* h, double* A, int64_t ld, int64_t N, int64_t extra, d
   const int W = chol_outer_width(N);
   const int64_t R = N + extra;
   MatView Av{A, R, N, ld};
-  // counters / flags of the fused panel kernel, sized once so that nothing is (re)allocated between the panels
-  CKR(ensure(h, h->panel_sync, (size_t)(2 + (R + GEMM_BM - 1) / GEMM_BM + (W + NB - 1) / NB) * sizeof(int)));
+  CKR(ensure_panel_sync(h, N, R));
   const bool lookahead = h->panel_stream != nullptr && N > 2 * W;
   cudaEvent_t ev_cols = get_event(h), ev_panel = get_event(h);
   auto edge = [&](cudaEvent_t e, cudaStream_t from, cudaStream_t to) -> cudaError_t {
@@ -507,8 +648,7 @@ int run_trsm_fused(nngp_handle* h, double* B, int64_t ldb, int64_t rows, const d
   p.B = B; p.ldb = ldb; p.rows = (int)rows; p.L = L; p.ldl = ldl; p.N = (int)N;
   p.row_tiles = (int)((rows + GEMM_BM - 1) / GEMM_BM);
   p.col_blocks = (int)((N + NB - 1) / NB);
-  CKR(ensure(h, h->sync_ints, (size_t)(p.row_tiles + 1) * sizeof(int)));
-  CKR(ensure(h, h->ssq, (size_t)rows * sizeof(double)));
+  CKR(ensure_solve_workspace(h, rows));
   CK(cudaMemsetAsync(h->sync_ints.p, 0, (size_t)(p.row_tiles + 1) * sizeof(int), h->stream));
   p.counter = h->sync_ints.as<int>();
   p.progress = h->sync_ints.as<int>() + 1;
@@ -553,7 +693,7 @@ int run_trsm_right(nngp_handle* h, double* B, int64_t ldb, int64_t rows, const d
   const int col_blocks = (int)((N + NB - 1) / NB);
   // one or two row tiles are launch-latency bound: keep the plain 64-wide sweep (2 launches per column block)
   const int64_t OW = rows <= 2 * GEMM_BM ? NB : 4 * NB;
-  if (var) CKR(ensure(h, h->ssq, (size_t)rows * sizeof(double)));
+  CKR(ensure_solve_workspace(h, rows));
   for (int64_t o0 = 0; o0 < N; o0 += OW) {
     const int64_t o1 = std::min<int64_t>(o0 + OW, N);
     for (int64_t j0 = o0; j0 < o1; j0 += NB) {
@@ -604,8 +744,7 @@ int run_predict_solve(nngp_handle* h, double* B, int64_t ldb, int64_t rows, cons
 int build_w_planes(nngp_handle* h);
 int build_inverse(nngp_handle* h) {
   const int64_t N = h->N, ldl = h->ldl;
-  CKR(ensure(h, h->Linvfull, (size_t)N * ldl * sizeof(double)));
-  CKR(ensure(h, h->Kdd, (size_t)N * ldl * sizeof(double)));     // scratch for L^-T (otherwise the 'ntk' K_dd buffer)
+  CKR(ensure_fit_workspace(h, N));                             // Kdd: scratch for L^-T; the solve workspace
   double* X = h->Kdd.as<double>();
   cudaEvent_t a = get_event(h), b = get_event(h);
   cudaEventRecord(a, h->stream);
@@ -645,9 +784,9 @@ int run_inverse_variance(nngp_handle* h, const double* B, int64_t ldb, int64_t r
   p.ldc = ldb; p.W = nullptr; p.tri_k = 1;
   MatView a{B, rows, N, ldb}, b{h->Linvfull.as<double>(), N, N, h->ldl};
   const int64_t row_tiles = (rows + GEMM_BM - 1) / GEMM_BM;
+  CKR(ensure(h, h->partial, partial_bytes(h, N, rows)));
   if (rows <= TGV_MAXR) {
     // A handful of queries: one streaming pass over L^-1 (tri_gemv_kernel), then the fixed-order row reduction.
-    CKR(ensure(h, h->partial, (size_t)rows * N * 8));
     const int ngroups = (int)((N + 7) / 8);
     const dim3 tg((unsigned)((ngroups + 1) / 2));
     const double* Wf = h->Linvfull.as<double>();
@@ -665,13 +804,11 @@ int run_inverse_variance(nngp_handle* h, const double* B, int64_t ldb, int64_t r
     int kchunk = 64;
     while ((p.ktiles + kchunk - 1) / kchunk > 8) kchunk *= 2;
     const int nz = (p.ktiles + kchunk - 1) / kchunk;
-    CKR(ensure(h, h->partial, (size_t)nz * rows * N * 8));
     p.kchunk = kchunk; p.vpart = h->partial.as<double>();
     CKR(launch_gemm<EPI_ROWDOT>(h, a, 0, 0, b, 0, 0, p, nz));
     h->st.gemm_flops -= (double)rows * (double)N * (double)p.ktiles * GEMM_BK;
     var_from_split_kernel<<<(unsigned)rows, 256, 0, h->stream>>>(kss, h->partial.as<double>(), (int)rows, (int)N, p.ktiles, kchunk, var);
   } else {
-    CKR(ensure(h, h->partial, (size_t)rows * col_tiles * 8));
     p.partial = h->partial.as<double>();
     CKR(launch_gemm<EPI_ROWDOT>(h, a, 0, 0, b, 0, 0, p));
     // launch_gemm counted 2*M*N*K for the full square; the triangular product is half of it: N^2 flop per row
@@ -735,9 +872,9 @@ int launch_sliced(nngp_handle* h, const int8_t* qa, int64_t ra, const double* sa
   // Two row tiles per CTA tile (SL_RT): 32 KiB of operands per MMA set instead of 48.  (Single row tiles -- twice as
   // many, lighter tiles -- were measured for small batches and lose: 1024 rows at N = 8192 take 1.82 ms instead of
   // 1.55 ms, the kernel is bound by bytes per MAC even there.)
-  const int64_t tiles = (int64_t)((p.row_tiles + SL_RT - 1) / SL_RT) * p.col_tiles;
-  const int grid = (int)std::min<int64_t>((h->sm_count / SL_SUPER) * SL_SUPER, tiles);   // CTAs 4k..4k+3 share K_* row tiles
-  CKR(ensure(h, h->slscratch, (size_t)grid * SL_RT * SL_BM * SL_BN * sizeof(double)));
+  int grid;
+  int64_t rounds;
+  CKR(sliced_grid(h, rows, N, &grid, &rounds));
   p.scratch = h->slscratch.as<double>();
   CUtensorMap tmA, tmB;
   CKR(get_tmap_u8(h, qa, (uint64_t)s * ra, (uint64_t)ldq, SL_RT * SL_BM, &tmA));
@@ -752,10 +889,8 @@ int launch_sliced(nngp_handle* h, const int8_t* qa, int64_t ra, const double* sa
   // The wave re-alignment (wave_barrier, one counter per round of tiles) needs every CTA resident: a cooperative
   // launch.  With a single round there is nothing to re-align, and when the grid cannot be co-scheduled (another
   // context holds SMs) the launch is refused: then the CTAs run free.
-  const int64_t rounds = (tiles + grid - 1) / grid;
   bool launched = false;
   if (rounds >= 2) {
-    CKR(ensure(h, h->slsync, (size_t)rounds * sizeof(int)));
     CK(cudaMemsetAsync(h->slsync.p, 0, (size_t)rounds * sizeof(int), h->stream));
     p.wave_sync = h->slsync.as<int>();
     lc.attrs = &coop; lc.numAttrs = 1;
@@ -780,32 +915,21 @@ int launch_sliced(nngp_handle* h, const int8_t* qa, int64_t ra, const double* sa
 int build_w_planes(nngp_handle* h) {
   const int s = h->cfg.variance_slices;
   const int64_t N = h->N;
-  const int64_t ldq = round_up(N, SL_BK), rb = round_up(N, SL_BN);
-  if ((int64_t)s * 4096 * ldq >= (1LL << 31))
-    return fail(h, NNGP_EINVAL, "variance_slices = %d: int32 plane sums need N <= %lld (N = %lld)", s,
-                (long long)((1LL << 19) / s), (long long)N);
-  CKR(ensure(h, h->Wq, (size_t)s * rb * ldq));
-  CKR(ensure(h, h->wscale, (size_t)N * sizeof(double)));
+  const int64_t ldq = round_up(N, SL_BK), rb = round_up(N, SL_BN);   // (Wq, wscale: sized by ensure_model)
   CKR(slice_matrix(h, h->Linvfull.as<double>(), h->ldl, N, N, 1, s, rb, ldq, h->Wq.as<int8_t>(), h->wscale.as<double>()));
   CK(cudaStreamSynchronize(h->stream));
   h->wq_ldq = ldq; h->wq_rb = rb; h->have_wq = true;
   return NNGP_OK;
 }
 
-// var[r] = kss[r] - |K_*[r,:] W^T|^2 with the product on the int8 tensor cores, in row sub-blocks whose planes fit
-// 16 GiB (whole waves of 37 row tiles x 4 column tiles, so that the static tile order stays balanced).  The plane
-// pair (s-1, 0) is dropped (SlicedParams::skip_weak).
+// var[r] = kss[r] - |K_*[r,:] W^T|^2 with the product on the int8 tensor cores, in row sub-blocks of sliced_rows().
+// The plane pair (s-1, 0) is dropped (SlicedParams::skip_weak).
 int run_sliced_variance(nngp_handle* h, const double* B, int64_t ldb, int64_t rows, const double* kss, double* var) {
   const int s = h->cfg.variance_slices;
   const int64_t N = h->N, ldq = h->wq_ldq;
   const int col_tiles = (int)((N + SL_BN - 1) / SL_BN);
-  const int64_t wave_rows = (int64_t)(h->sm_count / SL_SUPER) * SL_RT * SL_BM;
-  int64_t sb = ((16LL << 30) / ((int64_t)s * ldq)) / wave_rows * wave_rows;
-  sb = std::max<int64_t>(sb, SL_RT * SL_BM);
-  sb = std::min<int64_t>(sb, round_up(rows, SL_RT * SL_BM));
-  CKR(ensure(h, h->Aq, (size_t)s * sb * ldq));
-  CKR(ensure(h, h->ascale, (size_t)sb * sizeof(double)));
-  CKR(ensure(h, h->partial, (size_t)2 * col_tiles * sb * sizeof(double)));
+  const int64_t sb = sliced_rows(h, N, rows);
+  CKR(ensure_sliced_block(h, N, rows));
   cudaEvent_t a = get_event(h), b = get_event(h);
   cudaEventRecord(a, h->stream);
   int rc = NNGP_OK;
@@ -837,7 +961,7 @@ int run_trsv_bwd(nngp_handle* h, const double* L, int64_t ld, int64_t N, double*
   const int grid = (int)((N + sw - 1) / sw);
   const size_t smem = (size_t)(NB * (NB + 1) + 2 * NB + sw) * sizeof(double);
   if (smem <= 200 * 1024) {
-    CKR(ensure(h, h->sync_ints, (size_t)(nblk + 1) * sizeof(int)));
+    CKR(ensure_solve_workspace(h, N));
     CK(cudaMemsetAsync(h->sync_ints.p, 0, (size_t)nblk * sizeof(int), h->stream));
     CK(cudaFuncSetAttribute(trsv_bwd_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // The kernel's CTAs wait on each other's flags, so they must all be resident: a cooperative launch makes the
@@ -902,23 +1026,33 @@ int input_error(nngp_handle* h, int flag, const char* who, const char* what) {
               "(the kernel needs q q' < 2^1024)", who, what);
 }
 
+// Rows [new0, rows) of X are new input: check them finite, and derive q of all `rows` rows with the range flag.
+// Both report in flags[1], which the caller reads back and turns into input_error.
+int derive_q(nngp_handle* h, int64_t rows, int64_t new0) {
+  const double* X = h->X.as<double>();
+  CKR(check_finite_async(h, X + new0 * h->ldx, h->ldx, rows - new0, h->D));
+  row_sqnorm_kernel<<<(unsigned)((rows * 32 + 255) / 256), 256, 0, h->stream>>>(X, h->ldx, (int)rows, (int)h->D, h->lsw2[0], h->lsb2[0], h->q.as<double>(), h->flags.as<int>() + 1);
+  h->st.kernel_launches++;
+  return NNGP_OK;
+}
+
 int bind_device(nngp_handle* h) {
   CK(cudaSetDevice(h->device));
   return NNGP_OK;
 }
 
-void drop_fit(nngp_handle* h) { h->importing = false; h->have_inv = false; h->have_wq = false; h->fitted = false; h->have_lml = false; h->have_y = false; h->have_M = false; }
+void drop_fit(nngp_handle* h) { h->importing = false; h->have_inv = false; h->have_wq = false; h->fitted = false; h->have_labels = false; h->have_M = false; }
 
-int alloc_state(nngp_handle* h, int64_t N, int64_t D) {
+// Start installing a fitted state of N x D on h: bind its device, drop the fitted state of h and its replicas, size
+// the model buffers.
+int begin_state(nngp_handle* h, int64_t N, int64_t D) {
+  CKR(bind_device(h));
+  drop_fit(h);
+  for (auto* p : h->peers) drop_fit(p);
   h->N = N; h->D = D;
   h->ldx = round_up(D, 2);
   h->ldl = round_up(N, 16);
-  CKR(ensure(h, h->X, (size_t)N * h->ldx * sizeof(double)));
-  CKR(ensure(h, h->q, (size_t)N * sizeof(double)));
-  CKR(ensure(h, h->L, (size_t)(N + 1) * h->ldl * sizeof(double)));  // +1 row: y^T rides through the factorisation
-  CKR(ensure(h, h->alpha, (size_t)h->ldl * sizeof(double)));
-  CKR(ensure(h, h->Linv, (size_t)round_up(N, NB) * NB * sizeof(double)));
-  return NNGP_OK;
+  return ensure_model(h, N, D);
 }
 
 // inv(L_JJ) for all diagonal blocks of the factor in h->L (after a factorisation or an imported state)
@@ -942,7 +1076,6 @@ int run_trtri_diag(nngp_handle* h) {
 int replicate_state(nngp_handle* h) {
   if (h->peers.empty() || !h->fitted) return NNGP_OK;
   const int64_t N = h->N, D = h->D, ldx = h->ldx, ldl = h->ldl;
-  const bool ntk = h->cfg.kernel_type == 1;
   const auto t_begin = std::chrono::steady_clock::now();
   std::vector<nngp_handle*> chain;
   chain.push_back(h);
@@ -950,17 +1083,13 @@ int replicate_state(nngp_handle* h) {
   const int G = (int)chain.size();
   for (int g = 1; g < G; ++g) {
     nngp_handle* p = chain[g];
-    CK(cudaSetDevice(p->device));
-    drop_fit(p);
-    int rc = alloc_state(p, N, D);
-    if (rc == NNGP_OK && ntk && h->have_M) rc = ensure(p, p->Mmat, (size_t)N * ldl * sizeof(double));
-    if (rc == NNGP_OK && h->have_inv) rc = ensure(p, p->Linvfull, (size_t)N * ldl * sizeof(double));
+    const int rc = begin_state(p, N, D);
     if (rc != NNGP_OK) { h->err = "replica on device " + std::to_string(p->device) + ": " + p->err; cudaSetDevice(h->device); return rc; }
   }
   const int64_t RP = 512;                       // rows per panel
   const int npanel = (int)((N + RP - 1) / RP);
   // items in chain order: 0 = small vectors (X, q, alpha, Linv), 1..npanel = factor panels, then M panels
-  const int nM = (ntk && h->have_M) ? npanel : 0;
+  const int nM = h->have_M ? npanel : 0;
   const int nI = h->have_inv ? npanel : 0;          // latency mode: the explicit inverse (lower trapezoids, like L)
   const int nitems = 1 + npanel + nM + nI;
   std::vector<std::vector<cudaEvent_t>> ev((size_t)G);   // ev[g][i]: item i has arrived on chain[g]
@@ -1013,8 +1142,7 @@ int replicate_state(nngp_handle* h) {
   if (ce != cudaSuccess) return fail(h, NNGP_ECUDA, "replicating the fitted state to the other GPUs failed: %s", cudaGetErrorString(ce));
   for (int g = 1; g < G; ++g) {
     nngp_handle* p = chain[g];
-    p->lambda = h->lambda; p->fitted = true; p->have_M = ntk && h->have_M;
-    p->have_lml = false; p->have_y = false; p->have_inv = h->have_inv;
+    p->lambda = h->lambda; p->fitted = true; p->have_M = h->have_M; p->have_inv = h->have_inv;
     if (h->have_wq) {          // each replica splits its own copy of L^-1 (a few ms) instead of receiving s more planes
       cudaSetDevice(p->device);
       const int rc = build_w_planes(p);
@@ -1034,6 +1162,17 @@ int replicate_state(nngp_handle* h) {
   if (nI) bytes += bytes_tri;
   h->st.replicate_bytes = bytes;
   return NNGP_OK;
+}
+
+// The common tail of every call that installs a fitted state (the factor, alpha, inv(L_JJ) and, as `have_M` says, M
+// are on the device and the flags have been read back): mark it fitted, build the explicit inverse in latency mode and
+// copy the state to the replicas.  `labels`: the state was fitted from labels on this handle.
+int publish_state(nngp_handle* h, bool labels, bool have_M) {
+  h->fitted = true;
+  h->have_labels = labels;
+  h->have_M = have_M;
+  if (builds_inverse(h)) CKR(build_inverse(h));
+  return replicate_state(h);
 }
 
 }  // namespace
@@ -1281,7 +1420,7 @@ void nngp_destroy(nngp_handle* h) {
   cudaSetDevice(h->device);
   if (h->stream) cudaStreamSynchronize(h->stream);
   for (DevBuf* b : {&h->X, &h->q, &h->L, &h->alpha, &h->flags, &h->lam_d, &h->xt, &h->qt, &h->kss,
-                    &h->blk, &h->mean_d, &h->var_d, &h->ssq, &h->sync_ints, &h->Mmat, &h->Kdd, &h->blk2, &h->cross, &h->partial, &h->mean_partial, &h->ka, &h->kb, &h->kqa, &h->kqb, &h->kout, &h->Linv, &h->Linvfull, &h->panel_inv, &h->panel_sync, &h->zkeep, &h->L2, &h->y, &h->app_x, &h->app_y, &h->sel_mean, &h->sel_var, &h->sel_score, &h->sel_key,
+                    &h->blk, &h->mean_d, &h->var_d, &h->ssq, &h->sync_ints, &h->Mmat, &h->Kdd, &h->blk2, &h->cross, &h->partial, &h->mean_partial, &h->ka, &h->kb, &h->kqa, &h->kqb, &h->kout, &h->stage, &h->Linv, &h->Linvfull, &h->panel_inv, &h->panel_sync, &h->zkeep, &h->L2, &h->y, &h->app_x, &h->app_y, &h->sel_mean, &h->sel_var, &h->sel_score, &h->sel_key,
                     &h->sel_state, &h->sel_okey, &h->sel_oidx, &h->sel_max, &h->Wq, &h->wscale, &h->Aq, &h->ascale, &h->slscratch, &h->slsync})
     release(*b);
   for (auto& r : h->pending) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -1305,6 +1444,7 @@ int nngp_stats(nngp_handle* h, nngp_stats_t* out) {
     out->d2h_bytes += p->st.d2h_bytes;
     out->gemm_launches += p->st.gemm_launches;
     out->gram_launches += p->st.gram_launches;
+    out->device_allocs += p->st.device_allocs;
   }
   return NNGP_OK;
 }
@@ -1368,19 +1508,16 @@ int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2, i
 static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train, int64_t N, int64_t D);
 int nngp_fit(nngp_handle* h, const double* x_train, const double* y_train, int64_t N, int64_t D) {
   if (!h) return NNGP_EINVAL;
-  for (auto* p : h->peers) drop_fit(p);
   CKR(fit_impl(h, x_train, y_train, N, D));
-  return replicate_state(h);
+  return publish_state(h, true, h->cfg.kernel_type == 1);
 }
 
 static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train, int64_t N, int64_t D) {
   if (!x_train || !y_train || N <= 0 || D <= 0)
     return fail(h, NNGP_EINVAL, "nngp_fit: bad argument (N=%lld D=%lld)", (long long)N, (long long)D);
   if (N > 65535LL * GEMM_BM || D > 0x7fffffffLL) return fail(h, NNGP_EINVAL, "nngp_fit: N=%lld too large", (long long)N);
-  CKR(bind_device(h));
-  drop_fit(h);
-  CKR(alloc_state(h, N, D));
-  const double sw2 = h->lsw2[0], sb2 = h->lsb2[0];   // first Dense layer
+  CKR(begin_state(h, N, D));
+  CKR(ensure_fit_workspace(h, N));
   double* X = h->X.as<double>();
   double* L = h->L.as<double>();
   double* alpha = h->alpha.as<double>();
@@ -1390,21 +1527,16 @@ static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train
   CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
   CKR(upload_matrix(h, x_train, N, D, X, h->ldx));
   CKR(upload_matrix(h, y_train, N, 1, alpha, 1));
-  CKR(ensure(h, h->y, (size_t)N * sizeof(double)));
   CK(cudaMemcpyAsync(h->y.p, alpha, (size_t)N * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
   t_h2d.stop();
-  CKR(check_finite_async(h, X, h->ldx, N, D));
   CKR(check_finite_async(h, alpha, 1, N, 1));
 
   StageTimer t_gram(h, &h->st.fit_gram_ms);
-  row_sqnorm_kernel<<<(unsigned)((N * 32 + 255) / 256), 256, 0, h->stream>>>(X, h->ldx, (int)N, (int)D, sw2, sb2, q, h->flags.as<int>() + 1);
-  h->st.kernel_launches++;
+  CKR(derive_q(h, N, 0));
   const bool ntk = h->cfg.kernel_type == 1;
   if (!ntk) {
     CKR(run_gram(h, X, h->ldx, N, q, X, h->ldx, N, q, D, L, h->ldl, 1));
   } else {  // NTK: Theta_dd (to be factored) -> L, the full symmetric K_dd -> Kdd (for M = L^-1 K_dd L^-T)
-    CKR(ensure(h, h->Kdd, (size_t)N * h->ldl * sizeof(double)));
-    CKR(ensure(h, h->Mmat, (size_t)N * h->ldl * sizeof(double)));
     CKR(run_gram(h, X, h->ldx, N, q, X, h->ldx, N, q, D, L, h->ldl, 0, h->Kdd.as<double>()));
   }
   diag_reg_kernel<<<1, 1024, 0, h->stream>>>(L, h->ldl, (int)N, h->cfg.diag_reg, h->cfg.diag_reg_absolute, h->lam_d.as<double>());
@@ -1420,7 +1552,6 @@ static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train
   StageTimer t_solve(h, &h->st.fit_solve_ms);
   lml_terms_kernel<<<1, 1024, 0, h->stream>>>(L, h->ldl, (int)N, L + N * h->ldl, h->lam_d.as<double>() + 1);
   h->st.kernel_launches++;
-  CKR(ensure(h, h->zkeep, (size_t)N * sizeof(double)));
   CK(cudaMemcpyAsync(h->zkeep.p, L + N * h->ldl, (size_t)N * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
   CKR(run_trsv_bwd(h, L, h->ldl, N, L + N * h->ldl, alpha, h->Linv.as<double>()));  // alpha = L^-T z
   if (ntk) {  // M = L^-1 K_dd L^-T : two row-wise solves around a transpose (M is symmetric)
@@ -1446,11 +1577,6 @@ static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train
   if (flags[0])
     return fail(h, NNGP_ENOTPD, "nngp_fit: K + lambda*I is not positive definite (pivot %d of %lld, lambda=%.6g)",
                 flags[0] - 1, (long long)N, h->lambda);
-  h->fitted = true;
-  h->have_lml = true;
-  h->have_y = true;
-  h->have_M = ntk;
-  if (h->cfg.latency_mode && !ntk) CKR(build_inverse(h));
   return NNGP_OK;
 }
 
@@ -1465,14 +1591,7 @@ int nngp_active_select(nngp_handle* h, const double* x_pool, int64_t T, int64_t 
   if (T > 0xffffffffLL) return fail(h, NNGP_EINVAL, "nngp_active_select: T=%lld exceeds 2^32-1 rows", (long long)T);
   CKR(bind_device(h));
   const int64_t k = budget < T ? budget : T;   // num_select = budget if num_test > budget else num_test
-  CKR(ensure(h, h->sel_mean, (size_t)T * 8));
-  CKR(ensure(h, h->sel_var, (size_t)T * 8));
-  CKR(ensure(h, h->sel_score, (size_t)T * 8));
-  CKR(ensure(h, h->sel_key, (size_t)T * 8));
-  CKR(ensure(h, h->sel_okey, (size_t)k * 8));
-  CKR(ensure(h, h->sel_oidx, (size_t)k * 4));
-  CKR(ensure(h, h->sel_state, sizeof(SelectState)));
-  CKR(ensure(h, h->sel_max, 8));
+  CKR(ensure_select_workspace(h, T, k));
   // posterior mean / variance of the pool, left on the device (outputs are device pointers)
   CKR(nngp_predict(h, x_pool, T, h->sel_mean.as<double>(), h->sel_var.as<double>()));
 
@@ -1522,94 +1641,29 @@ int nngp_active_select(nngp_handle* h, const double* x_pool, int64_t T, int64_t 
   return NNGP_OK;
 }
 
-// latency mode / variance_slices: the explicit inverse, its build scratch, the digit planes of W and of a K_* sub-block
-// at (N, T) -- so that a growing training set (the active-learning loop) does not reallocate them round after round
-static int reserve_inverse_buffers(nngp_handle* h, int64_t N, int64_t T) {
-  if (!h->cfg.latency_mode || h->cfg.kernel_type != 0) return NNGP_OK;
-  const int64_t ldl = round_up(N, 16);
-  CKR(ensure(h, h->Linvfull, (size_t)N * ldl * 8));
-  if (!h->owner) CKR(ensure(h, h->Kdd, (size_t)N * ldl * 8));       // (replicas receive L^-1, they do not build it)
-  const int s = h->cfg.variance_slices;
-  if (s <= 0) return NNGP_OK;
-  const int64_t ldq = round_up(N, SL_BK), rb = round_up(N, SL_BN);
-  CKR(ensure(h, h->Wq, (size_t)s * rb * ldq));
-  CKR(ensure(h, h->wscale, (size_t)N * sizeof(double)));
-  if (T > 0) {                                                       // as run_sliced_variance sizes its sub-blocks
-    const int64_t wave_rows = (int64_t)(h->sm_count / SL_SUPER) * SL_RT * SL_BM;
-    int64_t sb = ((16LL << 30) / ((int64_t)s * ldq)) / wave_rows * wave_rows;
-    sb = std::min<int64_t>(std::max<int64_t>(sb, SL_RT * SL_BM), round_up(T, SL_RT * SL_BM));
-    CKR(ensure(h, h->Aq, (size_t)s * sb * ldq));
-    CKR(ensure(h, h->ascale, (size_t)sb * sizeof(double)));
-    CKR(ensure(h, h->partial, (size_t)2 * (rb / SL_BN) * sb * sizeof(double)));
-  }
-  return NNGP_OK;
-}
-
 int nngp_reserve(nngp_handle* h, int64_t n_train_max, int64_t dim, int64_t n_test_max) {
   if (!h) return NNGP_EINVAL;
   if (n_train_max <= 0 || dim <= 0 || n_test_max < 0 || n_train_max > 65535LL * GEMM_BM)
     return fail(h, NNGP_EINVAL, "nngp_reserve: bad argument (n_train_max=%lld dim=%lld n_test_max=%lld)",
                 (long long)n_train_max, (long long)dim, (long long)n_test_max);
   CKR(bind_device(h));
+  const int64_t N = n_train_max, D = dim, T = n_test_max;
   drop_fit(h);   // growing a buffer does not keep its contents
-  const int64_t N = n_train_max, T = n_test_max;
-  const int64_t ldx = round_up(dim, 2), ldl = round_up(N, 16);
-  CKR(ensure(h, h->X, (size_t)N * ldx * 8));
-  CKR(ensure(h, h->q, (size_t)N * 8));
-  CKR(ensure(h, h->y, (size_t)N * 8));
-  CKR(ensure(h, h->app_x, (size_t)N * dim * 8));
-  CKR(ensure(h, h->app_y, (size_t)N * 8));
-  CKR(ensure(h, h->L, (size_t)(N + 1) * ldl * 8));
-  CKR(ensure(h, h->alpha, (size_t)ldl * 8));
-  CKR(ensure(h, h->Linv, (size_t)round_up(N, NB) * NB * 8));
-  CKR(ensure(h, h->zkeep, (size_t)N * 8));
-  if (h->cfg.diag_reg_absolute && h->cfg.kernel_type == 0)   // the incremental append ping-pongs between two factors
-    CKR(ensure(h, h->L2, (size_t)(N + 1) * ldl * 8));
-  if (T > 0) {   // the row-block workspace of nngp_predict / nngp_active_select at (N, T)
-    int64_t cap_rows = h->cfg.max_block_bytes / (ldl * 8);
-    cap_rows = std::min<int64_t>(std::max<int64_t>(cap_rows, GEMM_BM), 65535LL * GEMM_BM);
-    const int64_t nblocks = (T + cap_rows - 1) / cap_rows;   // as nngp_predict sizes its row blocks
-    const int64_t TB = std::min<int64_t>(round_up(T, 2), round_up((T + nblocks - 1) / nblocks, GEMM_BM));
-    const int64_t col_tiles = (N + GEMM_BN - 1) / GEMM_BN;
-    CKR(ensure(h, h->xt, (size_t)TB * ldx * 8));
-    CKR(ensure(h, h->qt, (size_t)TB * 8));
-    CKR(ensure(h, h->kss, (size_t)TB * 8));
-    CKR(ensure(h, h->blk, (size_t)TB * ldl * 8));
-    CKR(ensure(h, h->mean_partial, (size_t)TB * 2 * col_tiles * 8));
-    CKR(ensure(h, h->mean_d, (size_t)T * 8));
-    CKR(ensure(h, h->var_d, (size_t)T * 8));
-    for (DevBuf* b : {&h->sel_mean, &h->sel_var, &h->sel_score, &h->sel_key}) CKR(ensure(h, *b, (size_t)T * 8));
-  }
-  CKR(reserve_inverse_buffers(h, N, T));
-  // replicas (cfg.n_gpus > 1): the state buffers at full size and the workspace for this GPU's share of the rows, so
-  // that a growing training set does not make every replica free and reallocate multi-GB buffers round after round
+  CKR(ensure_fit_workspace(h, N));
+  CKR(ensure_append_workspace(h, N, D));
+  if (T > 0) CKR(ensure_select_workspace(h, T, T));
+  // the model and the predict workspace on every GPU; a replica predicts its share of the rows (nngp_predict)
   const int G = 1 + (int)h->peers.size();
-  for (auto* p : h->peers) {
+  for (int g = 0; g < G; ++g) {
+    nngp_handle* p = g == 0 ? h : h->peers[(size_t)g - 1];
+    const int64_t Tg = g == 0 || T == 0 ? T : (T + G - 1) / G + 1;
     CK(cudaSetDevice(p->device));
     drop_fit(p);
-    int rc = ensure(p, p->X, (size_t)N * ldx * 8);
-    if (rc == NNGP_OK) rc = ensure(p, p->q, (size_t)N * 8);
-    if (rc == NNGP_OK) rc = ensure(p, p->L, (size_t)(N + 1) * ldl * 8);
-    if (rc == NNGP_OK) rc = ensure(p, p->alpha, (size_t)ldl * 8);
-    if (rc == NNGP_OK) rc = ensure(p, p->Linv, (size_t)round_up(N, NB) * NB * 8);
-    if (rc == NNGP_OK) rc = reserve_inverse_buffers(p, N, T > 0 ? (T + G - 1) / G + 1 : 0);
-    if (rc == NNGP_OK && T > 0) {
-      const int64_t Tg = (T + G - 1) / G + 1;
-      int64_t cap_rows = p->cfg.max_block_bytes / (ldl * 8);
-      cap_rows = std::min<int64_t>(std::max<int64_t>(cap_rows, GEMM_BM), 65535LL * GEMM_BM);
-      const int64_t nblocks = (Tg + cap_rows - 1) / cap_rows;
-      const int64_t TB = std::min<int64_t>(round_up(Tg, 2), round_up((Tg + nblocks - 1) / nblocks, GEMM_BM));
-      const int64_t col_tiles = (N + GEMM_BN - 1) / GEMM_BN;
-      rc = ensure(p, p->xt, (size_t)TB * ldx * 8);
-      if (rc == NNGP_OK) rc = ensure(p, p->qt, (size_t)TB * 8);
-      if (rc == NNGP_OK) rc = ensure(p, p->kss, (size_t)TB * 8);
-      if (rc == NNGP_OK) rc = ensure(p, p->blk, (size_t)TB * ldl * 8);
-      if (rc == NNGP_OK) rc = ensure(p, p->mean_partial, (size_t)TB * 2 * col_tiles * 8);
-      if (rc == NNGP_OK) rc = ensure(p, p->mean_d, (size_t)Tg * 8);
-      if (rc == NNGP_OK) rc = ensure(p, p->var_d, (size_t)Tg * 8);
-    }
+    int rc = ensure_model(p, N, D);
+    for (bool want_var : {false, true})
+      if (rc == NNGP_OK && Tg > 0) rc = ensure_predict_workspace(p, N, D, Tg, want_var);
     if (rc != NNGP_OK) {
-      h->err = "replica on device " + std::to_string(p->device) + ": " + p->err;
+      if (p != h) h->err = "replica on device " + std::to_string(p->device) + ": " + p->err;
       cudaSetDevice(h->device);
       return rc;
     }
@@ -1624,14 +1678,13 @@ int nngp_reserve(nngp_handle* h, int64_t n_train_max, int64_t dim, int64_t n_tes
 // L21 z)] (the y row rides through that small Cholesky as in the full fit), alpha' = L'^-T z'.  N^2 M + M^3/3 flop
 // instead of (N+M)^3/3.  Exact in exact arithmetic; in FP64 it agrees with a fresh fit to rounding (tested), not
 // bitwise.  Not applicable to the reference's relative diag_reg: there lambda = 1e-3 tr(K)/N moves with every row.
-// On entry X/y staging holds [X; X_new], [y; y_new]; h->L, h->Linv, h->zkeep describe the old N-row model.
+// On entry X/y staging holds [X; X_new], [y; y_new]; h->L, h->Linv, h->zkeep describe the old N-row model, and L2 and
+// panel_inv are sized for Nn rows (ensure_append_workspace).
 static int append_incremental(nngp_handle* h, int64_t M) {
   const int64_t N = h->N, D = h->D, Nn = N + M;
   const int64_t ldo = h->ldl, ldn = round_up(Nn, 16);
-  h->have_inv = false; h->have_wq = false;    // (latency mode: rebuilt by nngp_append_fit once the factor is extended)
-  const double sw2 = h->lsw2[0], sb2 = h->lsb2[0];   // first Dense layer
+  drop_fit(h);   // a half-extended model is not a model (nngp_append_fit publishes the extended one)
   StageTimer t_total(h, &h->st.fit_total_ms);
-  CKR(ensure(h, h->L2, (size_t)(Nn + 1) * ldn * sizeof(double)));
   double* Ln = h->L2.as<double>();
   CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
   // old factor (lower part incl. diagonal blocks) and old z into the new pitch
@@ -1640,20 +1693,16 @@ static int append_incremental(nngp_handle* h, int64_t M) {
   CK(cudaMemsetAsync(Ln + Nn * ldn, 0, (size_t)ldn * sizeof(double), h->stream));
   CK(cudaMemcpyAsync(Ln + Nn * ldn, h->zkeep.p, (size_t)N * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
   CK(cudaMemcpyAsync(Ln + Nn * ldn + N, h->app_y.as<double>() + N, (size_t)M * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
-  // X, y, q for all Nn rows (the staging buffers are contiguous)
-  CKR(ensure(h, h->X, (size_t)Nn * h->ldx * sizeof(double)));
-  CKR(ensure(h, h->q, (size_t)Nn * sizeof(double)));
-  CKR(ensure(h, h->y, (size_t)Nn * sizeof(double)));
-  CKR(ensure(h, h->alpha, (size_t)ldn * sizeof(double)));
-  CKR(ensure(h, h->zkeep, (size_t)Nn * sizeof(double)));
+  // X, y, q for all Nn rows (the staging buffers are contiguous).  The old X, y and z are in the staging and in Ln now,
+  // so their buffers may grow; the rest of the model grows only after the L21 solve has read the old inv(L_JJ).
+  CKR(ensure_fit_workspace(h, Nn));
+  CKR(ensure_inputs(h, Nn, D));
   double* X = h->X.as<double>();
   double* q = h->q.as<double>();
   CKR(upload_matrix(h, h->app_x.as<double>(), Nn, D, X, h->ldx));
   CK(cudaMemcpyAsync(h->y.p, h->app_y.p, (size_t)Nn * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
-  CKR(check_finite_async(h, X + N * h->ldx, h->ldx, M, D));
+  CKR(derive_q(h, Nn, N));
   CKR(check_finite_async(h, h->y.as<double>() + N, 1, M, 1));
-  row_sqnorm_kernel<<<(unsigned)((Nn * 32 + 255) / 256), 256, 0, h->stream>>>(X, h->ldx, (int)Nn, (int)D, sw2, sb2, q, h->flags.as<int>() + 1);
-  h->st.kernel_launches++;
 
   StageTimer t_gram(h, &h->st.fit_gram_ms);
   double* L21 = Ln + N * ldn;        // rows N..Nn-1, columns 0..N-1
@@ -1670,12 +1719,12 @@ static int append_incremental(nngp_handle* h, int64_t M) {
     MatView Av{Ln, Nn + 1, N, ldn};
     CKR(run_gemm_sub(h, Av, N, 0, Av, N, 0, M + 1, M, round_up(N, GEMM_BK), S, ldn, 1));
   }
-  CKR(ensure(h, h->panel_inv, (size_t)round_up(M, NB) * NB * sizeof(double)));   // inverses on the Schur block's own 64-grid
+  // (panel_inv: inverses on the Schur block's own 64-grid)
   CKR(run_potrf(h, S, ldn, M, 1, h->panel_inv.as<double>()));                                              // L22, z_new
   // from here on the handle describes the extended model
   std::swap(h->L, h->L2);
   h->N = Nn; h->ldl = ldn;
-  CKR(ensure(h, h->Linv, (size_t)round_up(Nn, NB) * NB * sizeof(double)));   // (old inverses are no longer needed)
+  CKR(ensure_model(h, Nn, D));   // (the old inverses are no longer needed)
   CKR(run_trtri_diag(h));
   t_chol.stop();
 
@@ -1694,18 +1743,16 @@ static int append_incremental(nngp_handle* h, int64_t M) {
   CK(cudaStreamSynchronize(h->stream));
   t_total.collect(); t_gram.collect(); t_chol.collect(); t_solve.collect();
   flush_class_events(h);
-  if (flags[1]) { drop_fit(h); return input_error(h, flags[1], "nngp_append_fit", "x_new / y_new"); }
-  if (flags[0]) {
-    drop_fit(h);
+  if (flags[1]) return input_error(h, flags[1], "nngp_append_fit", "x_new / y_new");
+  if (flags[0])
     return fail(h, NNGP_ENOTPD, "nngp_append_fit: the extended K + lambda*I is not positive definite (pivot %lld of %lld)",
                 (long long)(N + flags[0] - 1), (long long)Nn);
-  }
   return NNGP_OK;
 }
 
 int nngp_append_fit(nngp_handle* h, const double* x_new, const double* y_new, int64_t M) {
   if (!h) return NNGP_EINVAL;
-  if (!h->fitted || !h->have_y)
+  if (!h->fitted || !h->have_labels)
     return fail(h, NNGP_ESTATE, "nngp_append_fit: needs a model fitted by nngp_fit on this handle (the labels are kept there)");
   if (!x_new || !y_new || M <= 0) return fail(h, NNGP_EINVAL, "nngp_append_fit: bad argument (M=%lld)", (long long)M);
   CKR(bind_device(h));
@@ -1713,8 +1760,7 @@ int nngp_append_fit(nngp_handle* h, const double* x_new, const double* y_new, in
   // [X_old; x_new], [y_old; y_new] contiguous on the device, then an ordinary fit from device pointers
   DevBuf& xc = h->app_x;
   DevBuf& yc = h->app_y;
-  int rc = ensure(h, xc, (size_t)(N + M) * D * sizeof(double));
-  if (rc == NNGP_OK) rc = ensure(h, yc, (size_t)(N + M) * sizeof(double));
+  int rc = ensure_append_workspace(h, N + M, D);
   auto body = [&]() -> int {
     CK(cudaMemcpy2DAsync(xc.p, D * sizeof(double), h->X.p, h->ldx * sizeof(double), D * sizeof(double), N,
                          cudaMemcpyDeviceToDevice, h->stream));
@@ -1725,17 +1771,12 @@ int nngp_append_fit(nngp_handle* h, const double* x_new, const double* y_new, in
     // fixed lambda: extend the factor (NNGP_APPEND_INCREMENTAL=0 forces the full refit, e.g. for A/B runs)
     const char* inc = getenv("NNGP_APPEND_INCREMENTAL");
     // (an odd N would put the Schur block at an 8-byte-aligned column: TMA bases and the double2 epilogues need 16)
-    if (h->cfg.diag_reg_absolute && h->cfg.kernel_type == 0 && N % 2 == 0 && !(inc && !strcmp(inc, "0"))) {
-      const int r = append_incremental(h, M);
-      if (r != NNGP_OK) drop_fit(h);   // a half-extended model is not a model
-      return r;
-    }
+    if (can_append_incrementally(h) && N % 2 == 0 && !(inc && !strcmp(inc, "0"))) return append_incremental(h, M);
     return fit_impl(h, xc.as<double>(), yc.as<double>(), N + M, D);
   };
   for (auto* p : h->peers) drop_fit(p);
   if (rc == NNGP_OK) rc = body();
-  if (rc == NNGP_OK && h->cfg.latency_mode && h->cfg.kernel_type == 0 && !h->have_inv) rc = build_inverse(h);
-  if (rc == NNGP_OK) rc = replicate_state(h);
+  if (rc == NNGP_OK) rc = publish_state(h, true, h->cfg.kernel_type == 1);
   return rc;
 }
 
@@ -1787,29 +1828,10 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
   const int64_t N = h->N, D = h->D, ldx = h->ldx, ldl = h->ldl;
   const double sw2 = h->lsw2[0], sb2 = h->lsb2[0];   // first Dense layer
 
-  // Row-block size: what fits the buffer cap, in equal blocks of whole 128-row tiles.
   const bool ntk = h->cfg.kernel_type == 1;
-  int64_t cap_rows = h->cfg.max_block_bytes / (ldl * 8) / (ntk && var_out ? 2 : 1);  // NTK variance needs two row blocks
-  cap_rows = std::max<int64_t>(cap_rows, GEMM_BM);
-  cap_rows = std::min<int64_t>(cap_rows, 65535LL * GEMM_BM);
-  // equal blocks (whole 128-row tiles) instead of full blocks plus a short tail: the persistent solve keeps every SM
-  // busy with any tile count, what hurts is a last block with too few row tiles to fill the GPU
-  const int64_t nblocks = (T + cap_rows - 1) / cap_rows;
-  const int64_t TB = std::min<int64_t>(round_up(T, 2), round_up((T + nblocks - 1) / nblocks, GEMM_BM));
-
-  CKR(ensure(h, h->xt, (size_t)TB * ldx * 8));
-  CKR(ensure(h, h->qt, (size_t)TB * 8));
-  CKR(ensure(h, h->kss, (size_t)TB * 8));
-  CKR(ensure(h, h->blk, (size_t)TB * ldl * 8));
+  const int64_t TB = predict_block_rows(h, N, T, var_out != nullptr);
   const int col_tiles = (int)((N + GEMM_BN - 1) / GEMM_BN);
-  CKR(ensure(h, h->mean_partial, (size_t)TB * 2 * col_tiles * 8));  // one partial per 32-column warp slab
-  if (ntk && var_out) {
-    CKR(ensure(h, h->blk2, (size_t)TB * ldl * 8));
-    CKR(ensure(h, h->cross, (size_t)TB * 8));
-    CKR(ensure(h, h->partial, (size_t)TB * col_tiles * 8));
-  }
-  CKR(ensure(h, h->mean_d, (size_t)T * 8));
-  if (var_out) CKR(ensure(h, h->var_d, (size_t)T * 8));
+  CKR(ensure_predict_workspace(h, N, D, T, var_out != nullptr));
   CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
 
   double* xt = h->xt.as<double>();
@@ -1926,7 +1948,7 @@ int nngp_get_dims(nngp_handle* h, int64_t* N, int64_t* D, double* lambda_out) {
 
 int nngp_log_marginal_likelihood(nngp_handle* h, double* lml_out) {
   if (!h || !lml_out) return NNGP_EINVAL;
-  if (!h->fitted || !h->have_lml)
+  if (!h->fitted || !h->have_labels)
     return fail(h, NNGP_ESTATE, "nngp_log_marginal_likelihood: needs a model fitted by nngp_fit on this handle");
   const double two_pi = 6.283185307179586476925;
   *lml_out = -0.5 * h->lml_terms[1] - h->lml_terms[0] - 0.5 * (double)h->N * log(two_pi);
@@ -1949,26 +1971,30 @@ int nngp_get_state(nngp_handle* h, double* x_out, double* l_out, double* alpha_o
   return NNGP_OK;
 }
 
+// The tail of nngp_set_state / nngp_state_import_end: X, L and alpha are on the device.  X gets the checks of a fit
+// (the handle stays unfitted if it fails them); q and inv(L_JJ) are derived, then the state is published.
+static int finish_import(nngp_handle* h, double lambda, bool have_M, const char* who) {
+  CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
+  CKR(derive_q(h, h->N, 0));
+  CKR(run_trtri_diag(h));
+  int flags[2];
+  CK(cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  CK(cudaGetLastError());
+  if (flags[1]) return input_error(h, flags[1], who, "x");
+  h->lambda = lambda;
+  return publish_state(h, false, have_M);
+}
+
 int nngp_set_state(nngp_handle* h, const double* x, const double* l, const double* alpha, int64_t N, int64_t D,
                    double lambda) {
   if (!h) return NNGP_EINVAL;
   if (!x || !l || !alpha || N <= 0 || D <= 0) return fail(h, NNGP_EINVAL, "nngp_set_state: bad argument");
-  CKR(bind_device(h));
-  drop_fit(h);
-  CKR(alloc_state(h, N, D));
-  const double sw2 = h->lsw2[0], sb2 = h->lsb2[0];   // first Dense layer
+  CKR(begin_state(h, N, D));
   CKR(upload_matrix(h, x, N, D, h->X.as<double>(), h->ldx));
   CKR(upload_matrix(h, l, N, N, h->L.as<double>(), h->ldl));
   CKR(upload_matrix(h, alpha, N, 1, h->alpha.as<double>(), 1));
-  row_sqnorm_kernel<<<(unsigned)((N * 32 + 255) / 256), 256, 0, h->stream>>>(h->X.as<double>(), h->ldx, (int)N, (int)D, sw2, sb2, h->q.as<double>());
-  h->st.kernel_launches++;
-  CKR(run_trtri_diag(h));
-  CK(cudaStreamSynchronize(h->stream));
-  CK(cudaGetLastError());
-  h->lambda = lambda;
-  h->fitted = true;
-  if (h->cfg.latency_mode && h->cfg.kernel_type == 0) CKR(build_inverse(h));
-  return replicate_state(h);
+  return finish_import(h, lambda, false, "nngp_set_state");
 }
 
 // NTK mode: the fitted state also holds M = L^-1 K_dd L^-T (N x N, symmetric, dense), needed by the posterior variance.
@@ -1987,11 +2013,9 @@ int nngp_set_state_ntk_m(nngp_handle* h, const double* m) {
   if (!h->fitted || h->cfg.kernel_type != 1)
     return fail(h, NNGP_ESTATE, "nngp_set_state_ntk_m: call nngp_set_state on an 'ntk' handle first");
   CKR(bind_device(h));
-  CKR(ensure(h, h->Mmat, (size_t)h->N * h->ldl * sizeof(double)));
-  CKR(upload_matrix(h, m, h->N, h->N, h->Mmat.as<double>(), h->ldl));
+  CKR(upload_matrix(h, m, h->N, h->N, h->Mmat.as<double>(), h->ldl));   // (Mmat: sized by ensure_model)
   CK(cudaStreamSynchronize(h->stream));
-  h->have_M = true;
-  return replicate_state(h);
+  return publish_state(h, h->have_labels, true);
 }
 
 // -------------------------------------------------------------------------------------------------
@@ -2014,8 +2038,8 @@ static int pack_range(nngp_handle* h, int64_t offset, int64_t count, double* ext
   double* dptr = ext;
   const bool dev = is_device_ptr(ext);
   if (!dev) {   // host memory on the other side: stage the range through a device buffer
-    CKR(ensure(h, h->kout, (size_t)count * 8));
-    dptr = h->kout.as<double>();
+    CKR(ensure(h, h->stage, (size_t)count * 8));
+    dptr = h->stage.as<double>();
     if (unpack) { CK(cudaMemcpyAsync(dptr, ext, (size_t)count * 8, cudaMemcpyHostToDevice, h->stream)); h->st.h2d_bytes += count * 8; }
   }
   const int grid = (int)std::min<int64_t>((count + 255) / 256, 16LL * h->sm_count);
@@ -2045,12 +2069,8 @@ int nngp_state_pack(nngp_handle* h, int64_t offset, int64_t count, double* dst) 
 int nngp_state_import_begin(nngp_handle* h, int64_t N, int64_t D) {
   if (!h) return NNGP_EINVAL;
   if (N <= 0 || D <= 0 || N > 65535LL * GEMM_BM) return fail(h, NNGP_EINVAL, "nngp_state_import_begin: bad shape (N=%lld D=%lld)", (long long)N, (long long)D);
-  CKR(bind_device(h));
-  drop_fit(h);
-  for (auto* p : h->peers) drop_fit(p);
-  CKR(alloc_state(h, N, D));
+  CKR(begin_state(h, N, D));
   if (h->ldx != D) CK(cudaMemsetAsync(h->X.p, 0, (size_t)N * h->ldx * 8, h->stream));   // the pad column stays zero
-  if (h->cfg.kernel_type == 1) CKR(ensure(h, h->Mmat, (size_t)N * h->ldl * 8));
   CK(cudaStreamSynchronize(h->stream));
   h->importing = true;
   return NNGP_OK;
@@ -2067,17 +2087,7 @@ int nngp_state_import_end(nngp_handle* h, double lambda) {
   if (!h->importing) return fail(h, NNGP_ESTATE, "nngp_state_import_end: no import in progress");
   CKR(bind_device(h));
   h->importing = false;
-  const double sw2 = h->lsw2[0], sb2 = h->lsb2[0];   // first Dense layer
-  row_sqnorm_kernel<<<(unsigned)((h->N * 32 + 255) / 256), 256, 0, h->stream>>>(h->X.as<double>(), h->ldx, (int)h->N, (int)h->D, sw2, sb2, h->q.as<double>());
-  h->st.kernel_launches++;
-  CKR(run_trtri_diag(h));
-  CK(cudaStreamSynchronize(h->stream));
-  CK(cudaGetLastError());
-  h->lambda = lambda;
-  h->fitted = true;
-  h->have_M = h->cfg.kernel_type == 1;
-  if (h->cfg.latency_mode && h->cfg.kernel_type == 0) CKR(build_inverse(h));
-  return replicate_state(h);
+  return finish_import(h, lambda, h->cfg.kernel_type == 1, "nngp_state_import_end");
 }
 
 // -------------------------------------------------------------------------------------------------
@@ -2147,20 +2157,20 @@ int nngp_diag_potrf(nngp_handle* h, double* a, int64_t N) {
   if (!h || !a || N <= 0) return NNGP_EINVAL;
   CKR(bind_device(h));
   const int64_t ld = round_up(N, 16);
-  DevBuf A;
+  DevBuf A, W;   // the matrix and the inverses of its diagonal blocks
   CKR(ensure(h, A, (size_t)N * ld * 8));
   int rc = NNGP_OK;
   cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream);
   rc = upload_matrix(h, a, N, N, A.as<double>(), ld);
-  if (rc == NNGP_OK) rc = ensure(h, h->panel_inv, (size_t)round_up(N, NB) * NB * sizeof(double));
-  if (rc == NNGP_OK) rc = run_potrf(h, A.as<double>(), ld, N, 0, h->panel_inv.as<double>());
+  if (rc == NNGP_OK) rc = ensure(h, W, (size_t)round_up(N, NB) * NB * sizeof(double));
+  if (rc == NNGP_OK) rc = run_potrf(h, A.as<double>(), ld, N, 0, W.as<double>());
   if (rc == NNGP_OK) rc = download(h, A.as<double>(), N, N, ld, a);
   int flags[2] = {0, 0};
   cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream);
   cudaError_t e = cudaStreamSynchronize(h->stream);
   flush_class_events(h);
   h->tmaps.clear();
-  release(A);
+  release(A); release(W);
   if (rc != NNGP_OK) return rc;
   if (e != cudaSuccess) return fail(h, NNGP_ECUDA, "potrf failed: %s", cudaGetErrorString(e));
   if (flags[0]) return fail(h, NNGP_ENOTPD, "nngp_diag_potrf: not positive definite (pivot %d)", flags[0] - 1);

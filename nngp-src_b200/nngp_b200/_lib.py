@@ -52,7 +52,7 @@ class NngpStats(C.Structure):
         + [(n, C.c_double) for n in ("gram_ms", "gram_flops", "gram_evals")]
         + [(n, C.c_int64) for n in ("gram_launches", "kernel_launches", "h2d_bytes", "d2h_bytes", "queries")]
         + [("replicate_ms", C.c_double), ("replicate_bytes", C.c_int64), ("inverse_ms", C.c_double),
-           ("sliced_ms", C.c_double), ("sliced_macs", C.c_double)]
+           ("sliced_ms", C.c_double), ("sliced_macs", C.c_double), ("device_allocs", C.c_int64)]
     )
 
     def as_dict(self) -> dict:

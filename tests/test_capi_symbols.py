@@ -33,7 +33,7 @@ def test_library_exports_every_declared_symbol(lib):
     cdll = ctypes.CDLL(str(lib.LIB_PATH))
     for name in declared_functions():
         assert hasattr(cdll, name), f"{name} declared in include/nngp_b200.h but not exported"
-    assert cdll.nngp_abi_version() == 6
+    assert cdll.nngp_abi_version() == 7
     cdll.nngp_build_id.restype = ctypes.c_char_p
     from nngp_b200 import _build
     assert cdll.nngp_build_id().decode() == _build.source_hash() == lib.built_id()
@@ -56,7 +56,8 @@ def test_struct_layouts_match_header(lib):
     assert lib.NngpConfig.n_gpus.offset == 56 and lib.NngpConfig.device_ids.offset == 60
     assert lib.NngpConfig.latency_mode.offset == 92 and lib.NngpConfig.per_layer.offset == 96
     assert lib.NngpConfig.sigma_w_layers.offset == 104 and lib.NngpConfig.sigma_b_layers.offset == 232
-    assert ctypes.sizeof(lib.NngpStats) == 8 * 27
+    assert ctypes.sizeof(lib.NngpStats) == 8 * 28
+    assert lib.NngpStats.device_allocs.offset == 8 * 27            # ABI 7 appended it; earlier fields keep their offsets
 
 
 def test_no_cpu_fallback_without_gpu(lib):
