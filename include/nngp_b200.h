@@ -174,6 +174,21 @@ NNGP_API int nngp_fit(nngp_handle* h, const double* x_train, const double* y_tra
  */
 NNGP_API int nngp_predict(nngp_handle* h, const double* x_test, int64_t T, double* mean_out, double* var_out);
 
+/*
+ * predict_fn(x_test=X, get=..., compute_cov=True) without the diag(): the full posterior covariance of a test batch
+ *   'nngp': cov = K(X*,X*) - V V^T,                          V = K_* L^-T
+ *   'ntk' : cov = K(X*,X*) + V M V^T - (V U^T + U V^T),       V = Theta_* L^-T, U = K_* L^-T, M as in SURVEY A.5
+ * mean_out[T] as nngp_predict; cov_out[T*T] row-major, host or device memory.  cov_out is bitwise symmetric, its
+ * diagonal is bitwise the var_out of nngp_predict for the same batch on the same handle (whichever variance path
+ * that takes: substitution, latency mode or variance_slices; the off-diagonal products are always FP64), and the
+ * mean is bitwise nngp_predict's.  The test x test Gram and every product run on the lower triangle on the DMMA
+ * GEMM core, then the triangle is mirrored.  The batch is ONE prediction block: V (for 'ntk' also U and V M) of
+ * all T rows must fit cfg.max_block_bytes (T * round_up(N, 16) * 8 bytes each) -- a larger T is NNGP_EINVAL and the
+ * message names the largest T allowed.  With cfg.n_gpus > 1 the covariance is computed on the fit GPU.
+ * Errors otherwise as nngp_predict; an imported 'ntk' state without M is NNGP_ESTATE.
+ */
+NNGP_API int nngp_predict_cov(nngp_handle* h, const double* x_test, int64_t T, double* mean_out, double* cov_out);
+
 /* Fitted-state export/import: used to broadcast a fit to the other ranks of a
  * row-sharded prediction job (one process per GPU) and to save/load a model.
  * nngp_get_dims reports N, D and the lambda actually used.

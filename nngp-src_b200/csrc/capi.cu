@@ -101,6 +101,8 @@ struct nngp_handle {
   DevBuf xt, qt, kss, blk, mean_d, var_d, ssq, sync_ints;
   // NTK mode: M = L^-1 K_dd L^-T (N x N), scratch for building it, second row block, cross / partial terms
   DevBuf Mmat, Kdd, blk2, cross, partial, mean_partial;
+  // nngp_predict_cov: the T x T posterior covariance, and P = -V M ('ntk')
+  DevBuf cov, covP;
   // nngp_kernel workspace
   DevBuf ka, kb, kqa, kqb, kout;
   DevBuf stage;   // nngp_state_pack / _unpack with host memory on the other side: one range at a time
@@ -298,13 +300,14 @@ int launch_gemm(nngp_handle* h, const MatView& A, int a_row0, int a_col0, const 
 }
 
 // K(A rows, B rows) -> out (M x N, ld ldo).  A: M x D (lda), B: N x D (ldb); qa/qb layer-0 diagonals.
-// In NTK mode (cfg.kernel_type == 1) `out` receives Theta and `out2` (optional) the NNGP kernel K.
+// In NTK mode (cfg.kernel_type == 1) `out` receives Theta and `out2` (optional) the NNGP kernel K -- unless
+// `nngp_only`: then `out` receives K in either mode.
 int run_gram(nngp_handle* h, const double* A, int64_t lda, int64_t M, const double* qa, const double* B, int64_t ldb,
              int64_t N, const double* qb, int64_t D, double* out, int64_t ldo, int lower, double* out2 = nullptr,
-             const double* alpha = nullptr, double* mean_partial = nullptr) {
+             const double* alpha = nullptr, double* mean_partial = nullptr, bool nngp_only = false) {
   GemmParams p{};
   p.alpha = alpha; p.mean_partial = mean_partial;
-  p.ntk = h->cfg.kernel_type == 1 ? 1 : 0;
+  p.ntk = h->cfg.kernel_type == 1 && !nngp_only ? 1 : 0;
   p.C2 = out2;
   p.M = (int)M; p.N = (int)N;
   p.ktiles = (int)((D + GEMM_BK - 1) / GEMM_BK);
@@ -486,6 +489,20 @@ int ensure_predict_workspace(nngp_handle* h, int64_t N, int64_t D, int64_t T, bo
   if (ntk) CKR(ensure(h, h->cross, (size_t)TB * sizeof(double)));
   if (ntk || builds_inverse(h)) CKR(ensure(h, h->partial, partial_bytes(h, N, TB)));
   return h->cfg.variance_slices > 0 ? ensure_sliced_block(h, N, TB) : NNGP_OK;
+}
+
+// nngp_predict_cov: the largest batch whose V ('ntk': V, U and P = -V M) fits cfg.max_block_bytes -- the whole batch is
+// one prediction block (T <= this keeps predict_block_rows at one block of T rows, so V and U are blk and blk2)
+int64_t cov_max_rows(const nngp_handle* h, int64_t N) {
+  const int64_t per_row = round_up(N, 16) * 8 * (h->cfg.kernel_type == 1 ? 3 : 1);
+  return std::min<int64_t>(h->cfg.max_block_bytes / per_row, 65535LL * GEMM_BM);
+}
+
+// nngp_predict_cov of T rows (on top of ensure_predict_workspace): the T x T result, leading dimension round_up(T, 2)
+// (the GEMM epilogues store pairs of columns), and P = -V M ('ntk', T x round_up(N, 16))
+int ensure_cov_workspace(nngp_handle* h, int64_t N, int64_t T) {
+  CKR(ensure(h, h->cov, (size_t)T * round_up(T, 2) * sizeof(double)));
+  return h->cfg.kernel_type == 1 ? ensure(h, h->covP, (size_t)T * round_up(N, 16) * sizeof(double)) : NNGP_OK;
 }
 
 // nngp_active_select of k out of T pool rows
@@ -1175,6 +1192,88 @@ int publish_state(nngp_handle* h, bool labels, bool have_M) {
   return replicate_state(h);
 }
 
+// ---- posterior variance and covariance of a prediction block ---------------------------------------------------
+// The posterior variance of one block of `rows` rows of a T-row batch (blk: K_*, 'ntk': Theta_*; blk2: K_* ('ntk');
+// kss: K(x,x)), by the path chosen for that T.  nngp_predict and nngp_predict_cov both take it, so the covariance's
+// diagonal is bitwise the variance.  *solved: blk now holds V = blk L^-T ('ntk': also blk2 holds U = K_* L^-T) --
+// the latency-mode and digit-plane paths never write V.
+int block_variance(nngp_handle* h, int64_t T, int64_t rows, double* var, std::vector<StageTimer>& timers, bool* solved) {
+  const int64_t N = h->N, ldl = h->ldl;
+  double* blk = h->blk.as<double>();
+  const double* L = h->L.as<double>();
+  const double* kss = h->kss.as<double>();
+  *solved = true;
+  if (h->cfg.kernel_type == 1) {
+    // var_i = K_ii + v_i^T M v_i - 2 v_i . u_i,  v_i = L^-1 theta_i, u_i = L^-1 k_i, M = L^-1 K_dd L^-T
+    double* blk2 = h->blk2.as<double>();
+    timers.emplace_back(h, &h->st.pred_trsm_ms);
+    CKR(run_predict_solve(h, blk, ldl, rows, L, ldl, N, nullptr, nullptr));    // V
+    CKR(run_predict_solve(h, blk2, ldl, rows, L, ldl, N, nullptr, nullptr));   // U
+    timers.back().stop();
+    timers.emplace_back(h, &h->st.pred_var_ms);
+    rowdot_kernel<<<(unsigned)((rows * 32 + 255) / 256), 256, 0, h->stream>>>(blk, blk2, ldl, (int)rows, (int)N, h->cross.as<double>());
+    CKR(run_gemm_rowdot(h, blk, ldl, rows, h->Mmat.as<double>(), N, h->partial.as<double>()));
+    ntk_var_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, h->stream>>>(kss, h->partial.as<double>(), (int)((N + GEMM_BN - 1) / GEMM_BN), (int)rows, h->cross.as<double>(), var);
+    h->st.kernel_launches += 2;
+    timers.back().stop();
+    return NNGP_OK;
+  }
+  timers.emplace_back(h, &h->st.pred_trsm_ms);
+  if (T <= latency_rows(h)) {                      // latency mode, small batch: dependency-free product with L^-1
+    *solved = false;
+    CKR(run_inverse_variance(h, blk, ldl, rows, kss, var));
+  } else if (h->have_wq) {                         // variance_slices: the same product on the int8 tensor cores
+    *solved = false;
+    CKR(run_sliced_variance(h, blk, ldl, rows, kss, var));
+  } else {                                         // solve + variance in one persistent kernel
+    CKR(run_predict_solve(h, blk, ldl, rows, L, ldl, N, kss, var));
+  }
+  timers.back().stop();
+  return NNGP_OK;
+}
+
+// The T x T posterior covariance of a batch that is one prediction block, after block_variance (var: its variance):
+// xt / qt hold the batch, blk (blk2) V (U) unless !solved.  Lower tiles only (the full square below 4 row tiles, as
+// nngp_kernel), then one kernel mirrors them and installs `var` on the diagonal.  Every product is an EPI_SUB launch
+// of the DMMA core with K = round_up(N, 16); the columns past N are the tensor maps' zero fill (MatView cols = N).
+//   'nngp': C = K(X*,X*) - V V^T
+//   'ntk' : P = -V M (M symmetric: P -= V M^T on P = 0), C = K(X*,X*) - P V^T - U V^T - V U^T
+int block_covariance(nngp_handle* h, int64_t T, bool solved, const double* var, double* C, int64_t ldc,
+                     std::vector<StageTimer>& timers) {
+  const int64_t N = h->N, D = h->D, ldl = h->ldl, K = round_up(N, GEMM_BK);
+  double* blk = h->blk.as<double>();
+  double* xt = h->xt.as<double>();
+  const double* qt = h->qt.as<double>();
+  if (!solved) {
+    timers.emplace_back(h, &h->st.pred_trsm_ms);
+    CKR(run_predict_solve(h, blk, ldl, T, h->L.as<double>(), ldl, N, nullptr, nullptr));
+    timers.back().stop();
+  }
+  const int lower = T >= 4 * GEMM_BM ? 1 : 0;
+  timers.emplace_back(h, &h->st.pred_gram_ms);
+  CKR(run_gram(h, xt, h->ldx, T, qt, xt, h->ldx, T, qt, D, C, ldc, lower, nullptr, nullptr, nullptr, true));
+  timers.back().stop();
+  timers.emplace_back(h, &h->st.pred_var_ms);
+  const MatView Vv{blk, T, N, ldl};
+  if (h->cfg.kernel_type == 1) {
+    double* P = h->covP.as<double>();
+    const MatView Uv{h->blk2.as<double>(), T, N, ldl}, Pv{P, T, N, ldl}, Mv{h->Mmat.as<double>(), N, N, ldl};
+    CK(cudaMemsetAsync(P, 0, (size_t)T * ldl * sizeof(double), h->stream));
+    CKR(run_gemm_sub(h, Vv, 0, 0, Mv, 0, 0, T, N, K, P, ldl, 0));
+    CKR(run_gemm_sub(h, Pv, 0, 0, Vv, 0, 0, T, T, K, C, ldc, 1));
+    CKR(run_gemm_sub(h, Uv, 0, 0, Vv, 0, 0, T, T, K, C, ldc, 1));
+    CKR(run_gemm_sub(h, Vv, 0, 0, Uv, 0, 0, T, T, K, C, ldc, 1));
+  } else {
+    CKR(run_gemm_sub(h, Vv, 0, 0, Vv, 0, 0, T, T, K, C, ldc, 1));
+  }
+  const dim3 mg((unsigned)((T + 31) / 32), (unsigned)((T + 31) / 32));
+  mirror_lower_kernel<<<mg, dim3(32, 8), 0, h->stream>>>(C, ldc, (int)T, var);
+  h->st.kernel_launches++;
+  timers.back().stop();
+  CK(cudaGetLastError());
+  return NNGP_OK;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -1420,7 +1519,7 @@ void nngp_destroy(nngp_handle* h) {
   cudaSetDevice(h->device);
   if (h->stream) cudaStreamSynchronize(h->stream);
   for (DevBuf* b : {&h->X, &h->q, &h->L, &h->alpha, &h->flags, &h->lam_d, &h->xt, &h->qt, &h->kss,
-                    &h->blk, &h->mean_d, &h->var_d, &h->ssq, &h->sync_ints, &h->Mmat, &h->Kdd, &h->blk2, &h->cross, &h->partial, &h->mean_partial, &h->ka, &h->kb, &h->kqa, &h->kqb, &h->kout, &h->stage, &h->Linv, &h->Linvfull, &h->panel_inv, &h->panel_sync, &h->zkeep, &h->L2, &h->y, &h->app_x, &h->app_y, &h->sel_mean, &h->sel_var, &h->sel_score, &h->sel_key,
+                    &h->blk, &h->mean_d, &h->var_d, &h->ssq, &h->sync_ints, &h->Mmat, &h->Kdd, &h->blk2, &h->cov, &h->covP, &h->cross, &h->partial, &h->mean_partial, &h->ka, &h->kb, &h->kqa, &h->kqb, &h->kout, &h->stage, &h->Linv, &h->Linvfull, &h->panel_inv, &h->panel_sync, &h->zkeep, &h->L2, &h->y, &h->app_x, &h->app_y, &h->sel_mean, &h->sel_var, &h->sel_score, &h->sel_key,
                     &h->sel_state, &h->sel_okey, &h->sel_oidx, &h->sel_max, &h->Wq, &h->wscale, &h->Aq, &h->ascale, &h->slscratch, &h->slsync})
     release(*b);
   for (auto& r : h->pending) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -1492,7 +1591,7 @@ int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2, i
   CKR(run_gram(h, h->ka.as<double>(), ldx, M, h->kqa.as<double>(), bptr, ldx, Nn, qb, D, h->kout.as<double>(), ldo, sym ? 1 : 0));
   if (sym) {
     dim3 mg((unsigned)((M + 31) / 32), (unsigned)((M + 31) / 32));
-    mirror_lower_kernel<<<mg, dim3(32, 8), 0, h->stream>>>(h->kout.as<double>(), ldo, (int)M);
+    mirror_lower_kernel<<<mg, dim3(32, 8), 0, h->stream>>>(h->kout.as<double>(), ldo, (int)M, nullptr);
     h->st.kernel_launches++;
   }
   CKR(download(h, h->kout.as<double>(), M, Nn, ldo, k_out));
@@ -1781,7 +1880,8 @@ int nngp_append_fit(nngp_handle* h, const double* x_new, const double* y_new, in
 }
 
 // -------------------------------------------------------------------------------------------------
-static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double* mean_out, double* var_out);
+static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double* mean_out, double* var_out,
+                        double* cov_out = nullptr);
 
 // cfg.n_gpus > 1: rows [g*T/G, (g+1)*T/G) go to GPU g (SURVEY 8e); the replicas run on one host thread each while the
 // calling thread drives the first GPU.  Rows are independent and every reduction has a fixed order, so the result
@@ -1819,19 +1919,23 @@ int nngp_predict(nngp_handle* h, const double* x_test, int64_t T, double* mean_o
   return NNGP_OK;
 }
 
-static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double* mean_out, double* var_out) {
+// cov_out (nngp_predict_cov, which has checked that T rows are one block): also the T x T posterior covariance.
+static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double* mean_out, double* var_out,
+                        double* cov_out) {
   if (!h->fitted) return fail(h, NNGP_ESTATE, "nngp_predict: no fitted model (call nngp_fit or nngp_set_state)");
   if (!x_test || !mean_out || T <= 0) return fail(h, NNGP_EINVAL, "nngp_predict: bad argument (T=%lld)", (long long)T);
-  if (h->cfg.kernel_type == 1 && var_out && !h->have_M)
+  const bool want_var = var_out != nullptr || cov_out != nullptr;
+  if (h->cfg.kernel_type == 1 && want_var && !h->have_M)
     return fail(h, NNGP_ESTATE, "nngp_predict: this imported 'ntk' state has no M yet (nngp_set_state_ntk_m) -- the variance needs it");
   CKR(bind_device(h));
   const int64_t N = h->N, D = h->D, ldx = h->ldx, ldl = h->ldl;
   const double sw2 = h->lsw2[0], sb2 = h->lsb2[0];   // first Dense layer
 
   const bool ntk = h->cfg.kernel_type == 1;
-  const int64_t TB = predict_block_rows(h, N, T, var_out != nullptr);
+  const int64_t TB = predict_block_rows(h, N, T, want_var);
   const int col_tiles = (int)((N + GEMM_BN - 1) / GEMM_BN);
-  CKR(ensure_predict_workspace(h, N, D, T, var_out != nullptr));
+  CKR(ensure_predict_workspace(h, N, D, T, want_var));
+  if (cov_out) CKR(ensure_cov_workspace(h, N, T));
   CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
 
   double* xt = h->xt.as<double>();
@@ -1866,7 +1970,7 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
       row_sqnorm_kernel<<<(unsigned)((cr * 32 + 255) / 256), 256, 0, h->stream>>>(xt + c0 * ldx, ldx, (int)cr, (int)D, sw2, sb2, qt_c, h->flags.as<int>() + 1);
       h->st.kernel_launches++;
       CKR(run_gram(h, xt + c0 * ldx, ldx, cr, qt_c, h->X.as<double>(), ldx, N, h->q.as<double>(), D, blk + c0 * ldl, ldl, 0,
-                   (ntk && var_out) ? h->blk2.as<double>() + c0 * ldl : nullptr, h->alpha.as<double>(), mp_c));
+                   (ntk && want_var) ? h->blk2.as<double>() + c0 * ldl : nullptr, h->alpha.as<double>(), mp_c));
       mean_reduce_kernel<<<(unsigned)((cr + 255) / 256), 256, 0, h->stream>>>(mp_c, 2 * col_tiles, (int)cr, h->mean_d.as<double>() + t0 + c0);
       h->st.kernel_launches++;
     }
@@ -1877,39 +1981,20 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
     CK(cudaEventRecord(ev_xt_free, h->stream));   // the next block's upload may overlap this block's solve
     for (auto e : ev_chunk) h->ev_pool.push_back(e);
 
-    if (var_out) {
+    if (want_var) {
       LayerSig sig;
       for (int i = 0; i < 16; ++i) { sig.sw2[i] = h->lsw2[std::min(i + 1, NNGP_MAX_LAYERS - 1)]; sig.sb2[i] = h->lsb2[std::min(i + 1, NNGP_MAX_LAYERS - 1)]; }
       q_final_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, h->stream>>>(h->qt.as<double>(), (int)rows, h->cfg.depth - 1, sig, h->kss.as<double>());
       h->st.kernel_launches++;
-      if (ntk) {
-        // var_i = K_ii + v_i^T M v_i - 2 v_i . u_i,  v_i = L^-1 theta_i, u_i = L^-1 k_i, M = L^-1 K_dd L^-T
-        double* blk2 = h->blk2.as<double>();
-        timers.emplace_back(h, &h->st.pred_trsm_ms);
-        CKR(run_predict_solve(h, blk, ldl, rows, h->L.as<double>(), ldl, N, nullptr, nullptr));    // V
-        CKR(run_predict_solve(h, blk2, ldl, rows, h->L.as<double>(), ldl, N, nullptr, nullptr));   // U
-        timers.back().stop();
-        timers.emplace_back(h, &h->st.pred_var_ms);
-        rowdot_kernel<<<(unsigned)((rows * 32 + 255) / 256), 256, 0, h->stream>>>(blk, blk2, ldl, (int)rows, (int)N, h->cross.as<double>());
-        CKR(run_gemm_rowdot(h, blk, ldl, rows, h->Mmat.as<double>(), N, h->partial.as<double>()));
-        ntk_var_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, h->stream>>>(h->kss.as<double>(), h->partial.as<double>(), col_tiles, (int)rows, h->cross.as<double>(), h->var_d.as<double>() + t0);
-        h->st.kernel_launches += 2;
-        timers.back().stop();
-      } else {
-        timers.emplace_back(h, &h->st.pred_trsm_ms);
-        if (T <= latency_rows(h))                      // latency mode, small batch: dependency-free product with L^-1
-          CKR(run_inverse_variance(h, blk, ldl, rows, h->kss.as<double>(), h->var_d.as<double>() + t0));
-        else if (h->have_wq)                           // variance_slices: the same product on the int8 tensor cores
-          CKR(run_sliced_variance(h, blk, ldl, rows, h->kss.as<double>(), h->var_d.as<double>() + t0));
-        else                                           // solve + variance in one persistent kernel
-          CKR(run_predict_solve(h, blk, ldl, rows, h->L.as<double>(), ldl, N, h->kss.as<double>(), h->var_d.as<double>() + t0));
-        timers.back().stop();
-      }
+      bool solved = false;
+      CKR(block_variance(h, T, rows, h->var_d.as<double>() + t0, timers, &solved));
+      if (cov_out) CKR(block_covariance(h, T, solved, h->var_d.as<double>(), h->cov.as<double>(), round_up(T, 2), timers));
     }
   }
   timers.emplace_back(h, &h->st.d2h_ms);
   CKR(download(h, h->mean_d.as<double>(), T, 1, 1, mean_out));
   if (var_out) CKR(download(h, h->var_d.as<double>(), T, 1, 1, var_out));
+  if (cov_out) CKR(download(h, h->cov.as<double>(), T, T, round_up(T, 2), cov_out));
   timers.back().stop();
   t_total.stop();
   int flags[2];
@@ -1931,9 +2016,27 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
     h->ev_pool.push_back(sp.first); h->ev_pool.push_back(sp.second);
   }
   flush_class_events(h);
-  if (flags[1]) return input_error(h, flags[1], "nngp_predict", "x_test");
+  if (flags[1]) return input_error(h, flags[1], cov_out ? "nngp_predict_cov" : "nngp_predict", "x_test");
   h->st.queries += T;
   return NNGP_OK;
+}
+
+// The covariance couples every pair of rows, so it is not sharded: on a handle with replicas it runs on the fit GPU,
+// which makes it bitwise the single-GPU result.
+int nngp_predict_cov(nngp_handle* h, const double* x_test, int64_t T, double* mean_out, double* cov_out) {
+  if (!h) return NNGP_EINVAL;
+  if (!h->fitted) return fail(h, NNGP_ESTATE, "nngp_predict_cov: no fitted model (call nngp_fit or nngp_set_state)");
+  if (!x_test || !mean_out || !cov_out || T <= 0)
+    return fail(h, NNGP_EINVAL, "nngp_predict_cov: bad argument (T=%lld)", (long long)T);
+  if (h->cfg.kernel_type == 1 && !h->have_M)
+    return fail(h, NNGP_ESTATE, "nngp_predict_cov: this imported 'ntk' state has no M yet (nngp_set_state_ntk_m) -- the covariance needs it");
+  const int64_t cap = cov_max_rows(h, h->N);
+  if (T > cap)
+    return fail(h, NNGP_EINVAL, "nngp_predict_cov: T=%lld rows do not fit one prediction block: %s of the batch must fit "
+                "max_block_bytes=%lld at N=%lld, which allows T <= %lld", (long long)T,
+                h->cfg.kernel_type == 1 ? "V, U and V M" : "V", (long long)h->cfg.max_block_bytes, (long long)h->N,
+                (long long)cap);
+  return predict_impl(h, x_test, T, mean_out, nullptr, cov_out);
 }
 
 // -------------------------------------------------------------------------------------------------

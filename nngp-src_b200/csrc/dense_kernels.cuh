@@ -734,7 +734,9 @@ __global__ void transpose_kernel(const double* __restrict__ in, double* __restri
 // A[j][i] <- A[i][j] for i > j: fills the strict upper triangle of a symmetric matrix whose lower tiles were computed
 // (kernel_fn(x, None): the Gram kernel then skips the tiles above the diagonal).  32 x 32 tiles through shared memory,
 // one CTA per lower tile (bx <= by); grid (n/32, n/32), block (32, 8).
-__global__ void mirror_lower_kernel(double* __restrict__ A, long long ld, int n) {
+// `diag` (optional): A[i][i] <- diag[i] as well -- the posterior covariance (nngp_predict_cov) gets nngp_predict's
+// variance on its diagonal.  The diagonal tiles read their block before the barrier and write it after.
+__global__ void mirror_lower_kernel(double* __restrict__ A, long long ld, int n, const double* __restrict__ diag) {
   __shared__ double tile[32][33];
   if (blockIdx.x > blockIdx.y) return;
   const int c0 = blockIdx.x * 32, r0 = blockIdx.y * 32;     // source tile: rows r0.., columns c0.. (c0 <= r0)
@@ -746,6 +748,10 @@ __global__ void mirror_lower_kernel(double* __restrict__ A, long long ld, int n)
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
     const int r = c0 + i, c = r0 + threadIdx.x;             // destination: rows c0.., columns r0..
     if (r < n && c < n && c > r) A[(long long)r * ld + c] = tile[threadIdx.x][i];
+  }
+  if (diag != nullptr && blockIdx.x == blockIdx.y && threadIdx.y == 0) {
+    const int r = r0 + threadIdx.x;
+    if (r < n) A[(long long)r * ld + r] = diag[r];
   }
 }
 

@@ -81,6 +81,7 @@ EXPORTS = {
     "nngp_kernel": (C.c_int, [_P, _P, _I64, _P, _I64, _I64, _P]),
     "nngp_fit": (C.c_int, [_P, _P, _P, _I64, _I64]),
     "nngp_predict": (C.c_int, [_P, _P, _I64, _P, _P]),
+    "nngp_predict_cov": (C.c_int, [_P, _P, _I64, _P, _P]),
     "nngp_get_dims": (C.c_int, [_P, C.POINTER(_I64), C.POINTER(_I64), _DP]),
     "nngp_get_state": (C.c_int, [_P, _P, _P, _P]),
     "nngp_set_state": (C.c_int, [_P, _P, _P, _P, _I64, _I64, C.c_double]),
@@ -318,6 +319,21 @@ class Handle:
         vp = _out_ptr(var_out, (T,), "var_out") if want_var else None
         self._ck(self._lib.nngp_predict(self._h, xp, T, mp, vp))
         return mean_out, (var_out if want_var else None)
+
+    def predict_cov(self, x, mean_out=None, cov_out=None):
+        """Posterior mean [T] and full covariance [T, T] of the rows of ``x`` (``nngp_predict_cov``): the covariance's
+        diagonal is bitwise ``predict``'s variance.  Outputs may be preallocated numpy arrays or device tensors."""
+        xp, kx = _ptr(x)
+        self._check_width(kx, "x_test")
+        T = kx.shape[0]
+        if mean_out is None:
+            mean_out = np.empty(T, dtype=np.float64)
+        if cov_out is None:
+            cov_out = np.empty((T, T), dtype=np.float64)
+        mp = _out_ptr(mean_out, (T,), "mean_out")
+        cp = _out_ptr(cov_out, (T, T), "cov_out")
+        self._ck(self._lib.nngp_predict_cov(self._h, xp, T, mp, cp))
+        return mean_out, cov_out
 
     def dims(self):
         n, d, lam = _I64(), _I64(), C.c_double()

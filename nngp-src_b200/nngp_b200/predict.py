@@ -8,7 +8,10 @@ active/ActiveLearner.py:27-28 + 35-36,44-45.  Semantics kept ([nt 0.6.1] predict
   * ``predict_fn(x_test=X, get='nngp', compute_cov=True)`` returns ``Gaussian(mean[T,1], covariance)``;
   * every caller only takes ``sqrt(diag(covariance))`` (train.py:180, estimator.py:55, ActiveLearner.py:46),
     so ``covariance`` is a lazy (T,T)-shaped object exposing the posterior-variance diagonal -- the T x T
-    matrix the reference materialises (and throws away) is never built.
+    matrix the reference materialises (and throws away) is never built;
+  * code that needs the joint posterior (correlations between queries, the variance of a sum, joint samples)
+    asks for it explicitly: ``predict_fn.full_covariance(x_test, get)`` returns ``Gaussian(mean, cov[T,T])``
+    from the same cached fit.
 All arithmetic: libnngp_b200.so (sm_100a CUDA).  Unsupported options raise NotImplementedError.
 """
 from __future__ import annotations
@@ -50,7 +53,8 @@ class LazyCovariance:
     def __array__(self, *a, **k):
         raise NotImplementedError(
             "nngp_b200 computes the posterior-variance DIAGONAL only (the reference's callers use nothing else: "
-            "train.py:180, estimator.py:55, ActiveLearner.py:46); use np.diag(cov) / cov.diagonal()")
+            "train.py:180, estimator.py:55, ActiveLearner.py:46); use np.diag(cov) / cov.diagonal(), or "
+            "predict_fn.full_covariance(x_test, get) for the T x T matrix")
 
     def __repr__(self):
         return f"LazyCovariance(shape={self.shape}, diagonal-only)"
@@ -103,6 +107,16 @@ def gradient_descent_mse_ensemble(kernel_fn, x_train, y_train, learning_rate=1.0
             return mean
         return Gaussian(mean, LazyCovariance(var))
 
+    def _full_covariance(x_test=None, get="nngp"):
+        """``predict_fn(x_test, get=get, compute_cov=True)`` with the covariance as the dense (T, T) posterior
+        covariance neural-tangents returns (mean (T, 1) or (T,) like predict_fn).  x_test=None: the training inputs."""
+        if get not in ("nngp", "ntk"):
+            raise NotImplementedError(f"full_covariance(get={get!r}): 'nngp' and 'ntk' are implemented (one at a time)")
+        h = _fitted(get)
+        xt = x_train if x_test is None else runtime.as_matrix(x_test, "x_test")
+        mean, cov = h.predict_cov(xt)
+        return Gaussian(mean.reshape(-1, 1) if len(y_shape) == 2 else mean, cov)
+
     def _release(get="nngp"):
         """Hand the fitted engine of ``get`` over to the caller and forget it here: this closure then refits from its
         own (x_train, y_train) the next time it is used -- in the reference every ``gradient_descent_mse_ensemble``
@@ -112,5 +126,6 @@ def gradient_descent_mse_ensemble(kernel_fn, x_train, y_train, learning_rate=1.0
 
     predict_fn.engine = _fitted            # bench / tests: access to the underlying C-ABI handle
     predict_fn.release = _release
+    predict_fn.full_covariance = _full_covariance
     predict_fn.spec = kernel_fn.spec
     return predict_fn
