@@ -74,7 +74,11 @@ typedef struct nngp_config {
   int32_t diag_reg_absolute;  /* 0: lambda = diag_reg * trace(K)/N  (nt default)      */
   int32_t device;             /* CUDA ordinal; -1 = current device                    */
   int64_t max_block_bytes;    /* cap of the test-row block buffer; 0 = default 16 GiB */
-  int32_t stats_level;        /* 0 none, 1 per-stage events, 2 per-kernel-class events*/
+  int32_t stats_level;        /* device times nngp_stats_t fills (its counters and replicate_ms, a host clock, are kept
+                                 at every level):
+                                 0: sliced_ms and inverse_ms only;
+                                 1: also fit_*_ms, pred_*_ms, h2d_ms and d2h_ms (one event pair per stage);
+                                 2: also gemm_ms and gram_ms (one event pair per DMMA launch)                        */
   int32_t kernel_type;        /* 0 = 'nngp' (reference default), 1 = 'ntk' (train.py:254)  */
   int32_t n_gpus;             /* 0 / 1: one GPU (`device`); G > 1: prediction rows are split over G GPUs   */
   int32_t device_ids[NNGP_MAX_GPUS]; /* CUDA ordinals when n_gpus > 1 ([0] = fit GPU); all -1: 0..G-1   */
@@ -96,12 +100,14 @@ typedef struct nngp_config {
   int32_t reserved0;
 } nngp_config;
 
-/* Per-stage device timings (CUDA events on the handle's stream) and work counters,
+/* Per-stage device timings (CUDA events; cfg.stats_level says which are filled) and work counters,
  * accumulated since the last nngp_stats_reset().  Replaces the wall-clock prints at
  * train.py:170-176,191-195 and estimator.py:44,52-54. */
 typedef struct nngp_stats_t {
   double fit_gram_ms, fit_chol_ms, fit_solve_ms, fit_total_ms;
-  double pred_gram_ms, pred_mean_ms, pred_trsm_ms, pred_var_ms, pred_total_ms;
+  double pred_gram_ms;
+  double pred_mean_ms;     /* always 0: the mean is reduced inside the Gram stage (pred_gram_ms)                  */
+  double pred_trsm_ms, pred_var_ms, pred_total_ms;
   double h2d_ms, d2h_ms;
   double gemm_ms;          /* stats_level 2: time inside the DMMA GEMM-update kernels  */
   double gemm_flops;       /* algorithmic flops of those launches (2*M*N*K)            */

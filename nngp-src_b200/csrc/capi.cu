@@ -45,10 +45,12 @@ struct DevBuf {
   T* as() const { return static_cast<T*>(p); }
 };
 
-enum EvClass { EV_GEMM = 0, EV_GRAM = 1 };
-struct EvRec {
+// Device time between two events recorded on `s`, added to *dst when the call settles (end_call).  A span without an
+// end or a destination is an event that only orders streams inside the call.
+struct Span {
   cudaEvent_t a, b;
-  int cls;
+  cudaStream_t s;
+  double* dst;
 };
 
 inline int64_t round_up(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
@@ -112,9 +114,8 @@ struct nngp_handle {
   std::map<std::tuple<const void*, uint64_t, uint64_t, uint64_t, uint32_t>, CUtensorMap> tmaps;
 
   nngp_stats_t st;
-  std::vector<EvRec> pending;
+  std::vector<Span> spans;   // of the current call: settled by end_call, or discarded by the next begin_call
   std::vector<cudaEvent_t> ev_pool;
-  std::vector<std::pair<cudaEvent_t, cudaEvent_t>> sliced_spans;   // run_sliced_variance, collected by nngp_predict
   std::vector<cudaEvent_t> rep_events;   // no-timing events of replicate_state (recorded on this handle's copy stream)
 };
 
@@ -186,55 +187,51 @@ bool is_device_ptr(const void* p) {
   return at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged;
 }
 
-// ---- events ----------------------------------------------------------------------------------
+// ---- events and stage timing ------------------------------------------------------------------
 cudaEvent_t get_event(nngp_handle* h) {
   if (!h->ev_pool.empty()) { cudaEvent_t e = h->ev_pool.back(); h->ev_pool.pop_back(); return e; }
   cudaEvent_t e;
   cudaEventCreate(&e);
   return e;
 }
-struct StageTimer {  // level >= 1: accumulates into *dst at flush time
-  nngp_handle* h;
-  cudaEvent_t a = nullptr, b = nullptr;
-  double* dst;
-  StageTimer(nngp_handle* h_, double* dst_) : h(h_), dst(dst_) {
-    if (h->cfg.stats_level >= 1) { a = get_event(h); cudaEventRecord(a, h->stream); }
-  }
-  void stop() {
-    if (a && !b) { b = get_event(h); cudaEventRecord(b, h->stream); }
-  }
-  // call after the stream has been synchronised
-  void collect() {
-    if (a && b) {
-      float ms = 0.f;
-      if (cudaEventElapsedTime(&ms, a, b) == cudaSuccess) *dst += ms;
-      h->ev_pool.push_back(a); h->ev_pool.push_back(b);
-      a = b = nullptr;
-    }
-  }
-};
-void class_begin(nngp_handle* h, int cls, cudaEvent_t* a) {
-  *a = nullptr;
-  if (h->cfg.stats_level >= 2) { *a = get_event(h); cudaEventRecord(*a, h->cur); }
-  (void)cls;
+
+// Opens a span on stream s that adds into *dst, if cfg.stats_level >= level.  Returns its index, or -1 (no span).
+int span_open(nngp_handle* h, int level, cudaStream_t s, double* dst) {
+  if (h->cfg.stats_level < level) return -1;
+  const cudaEvent_t a = get_event(h);
+  cudaEventRecord(a, s);
+  h->spans.push_back({a, nullptr, s, dst});
+  return (int)h->spans.size() - 1;
 }
-void class_end(nngp_handle* h, int cls, cudaEvent_t a) {
-  if (a) {
-    cudaEvent_t b = get_event(h);
-    cudaEventRecord(b, h->cur);
-    h->pending.push_back({a, b, cls});
-  }
+
+void span_close(nngp_handle* h, int i) {
+  if (i < 0) return;
+  Span& sp = h->spans[(size_t)i];
+  sp.b = get_event(h);
+  cudaEventRecord(sp.b, sp.s);
 }
-void flush_class_events(nngp_handle* h) {  // after a stream sync
-  for (auto& r : h->pending) {
+
+// An event that orders two streams inside the current call; it goes back to the pool with the call's spans.
+cudaEvent_t call_event(nngp_handle* h) {
+  const cudaEvent_t e = get_event(h);
+  h->spans.push_back({e, nullptr, nullptr, nullptr});
+  return e;
+}
+
+// After the call's synchronisation: add every closed span's time to its destination (`add`) and return all events
+// to the pool.  A span whose end event has not completed adds nothing; only the predict upload's can be pending, on
+// copy_stream, which the main stream waits for chunk by chunk but not to the span's end.
+void settle_spans(nngp_handle* h, bool add = true) {
+  for (const Span& sp : h->spans) {
     float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, r.a, r.b) == cudaSuccess) {
-      if (r.cls == EV_GEMM) h->st.gemm_ms += ms; else h->st.gram_ms += ms;
-    }
-    h->ev_pool.push_back(r.a); h->ev_pool.push_back(r.b);
+    if (add && sp.b && cudaEventElapsedTime(&ms, sp.a, sp.b) == cudaSuccess) *sp.dst += ms;
+    h->ev_pool.push_back(sp.a);
+    if (sp.b) h->ev_pool.push_back(sp.b);
   }
-  h->pending.clear();
+  h->spans.clear();
 }
+
+void discard_spans(nngp_handle* h) { settle_spans(h, false); }
 
 // ---- tensor maps ------------------------------------------------------------------------------
 // Row-major FP64 matrix [rows, cols] with leading dimension ld (elements); box = 16 x box_rows,
@@ -279,15 +276,17 @@ int launch_gemm(nngp_handle* h, const MatView& A, int a_row0, int a_col0, const 
   p.a_row0 = a_row0; p.a_col0 = a_col0; p.b_row0 = b_row0; p.b_col0 = b_col0;
   dim3 grid((p.N + GEMM_BN - 1) / GEMM_BN, (p.M + GEMM_BM - 1) / GEMM_BM, grid_z);
   if (grid.y > 65535) return fail(h, NNGP_EINVAL, "internal: GEMM row range too large (%d rows)", p.M);
-  cudaEvent_t ev;
-  const int cls = (EPI == EPI_GRAM) ? EV_GRAM : EV_GEMM;  // ROWDOT counts as a GEMM-class launch
-  class_begin(h, cls, &ev);
+  // (ROWDOT counts as a GEMM-class launch)
+  const int span = span_open(h, 2, h->cur, EPI == EPI_GRAM ? &h->st.gram_ms : &h->st.gemm_ms);
   gemm_nt_kernel<EPI><<<grid, GEMM_THREADS, GEMM_SMEM_BYTES, h->cur>>>(tmA, tmB, p);
-  class_end(h, cls, ev);
+  span_close(h, span);
   CK(cudaGetLastError());
   h->st.kernel_launches++;
-  const double frac = p.lower ? 0.5 : 1.0;  // algorithmic work of a lower-triangular range
-  const double flops = 2.0 * (double)p.M * (double)p.N * (double)p.ktiles * GEMM_BK * frac;
+  // algorithmic work: half the product for a lower-triangular range or a triangular B; the Gram's inner extent is the
+  // true D (A's width), the other products count their K extent
+  const double frac = p.lower || p.tri_k ? 0.5 : 1.0;
+  const double k = EPI == EPI_GRAM ? (double)A.cols : (double)p.ktiles * GEMM_BK;
+  const double flops = 2.0 * (double)p.M * (double)p.N * k * frac;
   if (EPI == EPI_GRAM) {
     h->st.gram_launches++;
     h->st.gram_flops += flops;
@@ -319,11 +318,7 @@ int run_gram(nngp_handle* h, const double* A, int64_t lda, int64_t M, const doub
     p.lsb2[i] = h->lsb2[std::min(i + 1, NNGP_MAX_LAYERS - 1)];
   }
   MatView a{A, M, D, lda}, b{B, N, D, ldb};
-  // the flop counter must use the true D, not the padded k extent
-  const double before = h->st.gram_flops;
-  CKR(launch_gemm<EPI_GRAM>(h, a, 0, 0, b, 0, 0, p));
-  h->st.gram_flops = before + 2.0 * (double)M * (double)N * (double)D * (lower ? 0.5 : 1.0);
-  return NNGP_OK;
+  return launch_gemm<EPI_GRAM>(h, a, 0, 0, b, 0, 0, p);
 }
 
 // C(M x N at `C`, ldc) -= Aop[a_row0:+M, a_col0:+K] * Bop[b_row0:+N, b_col0:+K]^T ; K % 16 == 0.
@@ -679,8 +674,7 @@ int run_trsm_fused(nngp_handle* h, double* B, int64_t ldb, int64_t rows, const d
   // column blocks of V as their producers publish them (software pipeline along J, see the gate in the kernel).
   const int grid = (int)std::min<long long>(total, 2LL * h->sm_count);
   p.static_sched = (p.row_tiles % grid == 0) ? 1 : 0;
-  cudaEvent_t ev;
-  class_begin(h, EV_GEMM, &ev);
+  const int span = span_open(h, 2, h->cur, &h->st.gemm_ms);
   // Plenty of row tiles (or exactly one static round of them): dependencies are practically always met when an item
   // starts, and the ungated kernel is 0.5 % faster (34.8 vs 34.6 TFLOP/s at C2).  Measured at N = 8192: 296 tiles
   // 81 ms ungated / 83 gated; 313 tiles 92 ms ungated / 86 gated.
@@ -688,7 +682,7 @@ int run_trsm_fused(nngp_handle* h, double* B, int64_t ldb, int64_t rows, const d
     trsm_fused_kernel<false><<<grid, GEMM_THREADS, TF_SMEM_BYTES, h->stream>>>(tmB, tmL, tmW, p);
   else                       // several CTAs per row tile: pipeline along J
     trsm_fused_kernel<true><<<grid, GEMM_THREADS, TF_SMEM_BYTES, h->stream>>>(tmB, tmL, tmW, p);
-  class_end(h, EV_GEMM, ev);
+  span_close(h, span);
   CK(cudaGetLastError());
   h->st.kernel_launches++;
   h->st.gemm_launches++;
@@ -763,21 +757,18 @@ int build_inverse(nngp_handle* h) {
   const int64_t N = h->N, ldl = h->ldl;
   CKR(ensure_fit_workspace(h, N));                             // Kdd: scratch for L^-T; the solve workspace
   double* X = h->Kdd.as<double>();
-  cudaEvent_t a = get_event(h), b = get_event(h);
-  cudaEventRecord(a, h->stream);
+  h->st.inverse_ms = 0.0;   // the last fit's, not a sum
+  const int span = span_open(h, 0, h->stream, &h->st.inverse_ms);
   set_identity_kernel<<<4 * h->sm_count, 256, 0, h->stream>>>(X, ldl, (int)N);
   h->st.kernel_launches++;
   CKR(run_trsm_fused(h, X, ldl, N, h->L.as<double>(), ldl, N, h->Linv.as<double>(), nullptr, nullptr, 1));
   dim3 tg((unsigned)((N + 31) / 32), (unsigned)((N + 31) / 32));
   transpose_kernel<<<tg, dim3(32, 8), 0, h->stream>>>(X, h->Linvfull.as<double>(), ldl, (int)N);
   h->st.kernel_launches++;
-  cudaEventRecord(b, h->stream);
+  span_close(h, span);
   CK(cudaStreamSynchronize(h->stream));
   CK(cudaGetLastError());
-  float ms = 0.f;
-  if (cudaEventElapsedTime(&ms, a, b) == cudaSuccess) h->st.inverse_ms = ms;
-  h->ev_pool.push_back(a); h->ev_pool.push_back(b);
-  flush_class_events(h);
+  settle_spans(h);
   h->have_inv = true;
   if (h->cfg.variance_slices > 0) CKR(build_w_planes(h));
   return NNGP_OK;
@@ -823,13 +814,10 @@ int run_inverse_variance(nngp_handle* h, const double* B, int64_t ldb, int64_t r
     const int nz = (p.ktiles + kchunk - 1) / kchunk;
     p.kchunk = kchunk; p.vpart = h->partial.as<double>();
     CKR(launch_gemm<EPI_ROWDOT>(h, a, 0, 0, b, 0, 0, p, nz));
-    h->st.gemm_flops -= (double)rows * (double)N * (double)p.ktiles * GEMM_BK;
     var_from_split_kernel<<<(unsigned)rows, 256, 0, h->stream>>>(kss, h->partial.as<double>(), (int)rows, (int)N, p.ktiles, kchunk, var);
   } else {
     p.partial = h->partial.as<double>();
     CKR(launch_gemm<EPI_ROWDOT>(h, a, 0, 0, b, 0, 0, p));
-    // launch_gemm counted 2*M*N*K for the full square; the triangular product is half of it: N^2 flop per row
-    h->st.gemm_flops -= (double)rows * (double)N * (double)p.ktiles * GEMM_BK;
     var_from_partial_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, h->stream>>>(kss, h->partial.as<double>(), col_tiles, (int)rows, var);
   }
   h->st.kernel_launches++;
@@ -947,23 +935,16 @@ int run_sliced_variance(nngp_handle* h, const double* B, int64_t ldb, int64_t ro
   const int col_tiles = (int)((N + SL_BN - 1) / SL_BN);
   const int64_t sb = sliced_rows(h, N, rows);
   CKR(ensure_sliced_block(h, N, rows));
-  cudaEvent_t a = get_event(h), b = get_event(h);
-  cudaEventRecord(a, h->stream);
-  int rc = NNGP_OK;
-  for (int64_t r0 = 0; r0 < rows && rc == NNGP_OK; r0 += sb) {
+  const int span = span_open(h, 0, h->stream, &h->st.sliced_ms);
+  for (int64_t r0 = 0; r0 < rows; r0 += sb) {
     const int64_t nr = std::min<int64_t>(sb, rows - r0), ra = round_up(nr, SL_RT * SL_BM);
-    rc = slice_matrix(h, B + r0 * ldb, ldb, nr, N, 0, s, ra, ldq, h->Aq.as<int8_t>(), h->ascale.as<double>());
-    if (rc == NNGP_OK)
-      rc = launch_sliced(h, h->Aq.as<int8_t>(), ra, h->ascale.as<double>(), h->Wq.as<int8_t>(), h->wq_rb,
-                         h->wscale.as<double>(), ldq, s, 1, nr, N, N, h->partial.as<double>(), nullptr, 0, 1);
-    if (rc == NNGP_OK) {
-      var_from_partial_kernel<<<(unsigned)((nr + 255) / 256), 256, 0, h->stream>>>(kss + r0, h->partial.as<double>(), 2 * col_tiles, (int)nr, var + r0);
-      h->st.kernel_launches++;
-    }
+    CKR(slice_matrix(h, B + r0 * ldb, ldb, nr, N, 0, s, ra, ldq, h->Aq.as<int8_t>(), h->ascale.as<double>()));
+    CKR(launch_sliced(h, h->Aq.as<int8_t>(), ra, h->ascale.as<double>(), h->Wq.as<int8_t>(), h->wq_rb,
+                      h->wscale.as<double>(), ldq, s, 1, nr, N, N, h->partial.as<double>(), nullptr, 0, 1));
+    var_from_partial_kernel<<<(unsigned)((nr + 255) / 256), 256, 0, h->stream>>>(kss + r0, h->partial.as<double>(), 2 * col_tiles, (int)nr, var + r0);
+    h->st.kernel_launches++;
   }
-  cudaEventRecord(b, h->stream);          // (also on the error path: the span is collected or recycled either way)
-  h->sliced_spans.push_back({a, b});
-  CKR(rc);
+  span_close(h, span);
   CK(cudaGetLastError());
   return NNGP_OK;
 }
@@ -1041,6 +1022,27 @@ int input_error(nngp_handle* h, int flag, const char* who, const char* what) {
   return fail(h, NNGP_EINVAL,
               "%s: %s out of range: a row's layer-0 kernel diagonal sigma_w^2 |x|^2 / D + sigma_b^2 reaches 2^512 "
               "(the kernel needs q q' < 2^1024)", who, what);
+}
+
+// Every call that reads `flags` back runs between begin_call and end_call.  begin_call clears the flags and discards
+// whatever spans a failed earlier call left behind, so their time is charged to no later call.  No call may run
+// another begin_call inside while it has spans open.
+int begin_call(nngp_handle* h) {
+  discard_spans(h);
+  CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
+  return NNGP_OK;
+}
+
+// Enqueues the flags read-back (after the caller's own), waits for the main stream and settles the spans.  flags[1]
+// becomes input_error(who, what); flags[0], the potrf pivot + 1 (0: none), goes to *pivot.
+int end_call(nngp_handle* h, const char* who, const char* what, int* pivot = nullptr) {
+  int flags[2];
+  CK(cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  CK(cudaGetLastError());
+  settle_spans(h);
+  if (pivot) *pivot = flags[0];
+  return flags[1] ? input_error(h, flags[1], who, what) : NNGP_OK;
 }
 
 // Rows [new0, rows) of X are new input: check them finite, and derive q of all `rows` rows with the range flag.
@@ -1197,28 +1199,27 @@ int publish_state(nngp_handle* h, bool labels, bool have_M) {
 // kss: K(x,x)), by the path chosen for that T.  nngp_predict and nngp_predict_cov both take it, so the covariance's
 // diagonal is bitwise the variance.  *solved: blk now holds V = blk L^-T ('ntk': also blk2 holds U = K_* L^-T) --
 // the latency-mode and digit-plane paths never write V.
-int block_variance(nngp_handle* h, int64_t T, int64_t rows, double* var, std::vector<StageTimer>& timers, bool* solved) {
+int block_variance(nngp_handle* h, int64_t T, int64_t rows, double* var, bool* solved) {
   const int64_t N = h->N, ldl = h->ldl;
   double* blk = h->blk.as<double>();
   const double* L = h->L.as<double>();
   const double* kss = h->kss.as<double>();
   *solved = true;
+  const int trsm = span_open(h, 1, h->stream, &h->st.pred_trsm_ms);
   if (h->cfg.kernel_type == 1) {
     // var_i = K_ii + v_i^T M v_i - 2 v_i . u_i,  v_i = L^-1 theta_i, u_i = L^-1 k_i, M = L^-1 K_dd L^-T
     double* blk2 = h->blk2.as<double>();
-    timers.emplace_back(h, &h->st.pred_trsm_ms);
     CKR(run_predict_solve(h, blk, ldl, rows, L, ldl, N, nullptr, nullptr));    // V
     CKR(run_predict_solve(h, blk2, ldl, rows, L, ldl, N, nullptr, nullptr));   // U
-    timers.back().stop();
-    timers.emplace_back(h, &h->st.pred_var_ms);
+    span_close(h, trsm);
+    const int vs = span_open(h, 1, h->stream, &h->st.pred_var_ms);
     rowdot_kernel<<<(unsigned)((rows * 32 + 255) / 256), 256, 0, h->stream>>>(blk, blk2, ldl, (int)rows, (int)N, h->cross.as<double>());
     CKR(run_gemm_rowdot(h, blk, ldl, rows, h->Mmat.as<double>(), N, h->partial.as<double>()));
     ntk_var_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, h->stream>>>(kss, h->partial.as<double>(), (int)((N + GEMM_BN - 1) / GEMM_BN), (int)rows, h->cross.as<double>(), var);
     h->st.kernel_launches += 2;
-    timers.back().stop();
+    span_close(h, vs);
     return NNGP_OK;
   }
-  timers.emplace_back(h, &h->st.pred_trsm_ms);
   if (T <= latency_rows(h)) {                      // latency mode, small batch: dependency-free product with L^-1
     *solved = false;
     CKR(run_inverse_variance(h, blk, ldl, rows, kss, var));
@@ -1228,7 +1229,7 @@ int block_variance(nngp_handle* h, int64_t T, int64_t rows, double* var, std::ve
   } else {                                         // solve + variance in one persistent kernel
     CKR(run_predict_solve(h, blk, ldl, rows, L, ldl, N, kss, var));
   }
-  timers.back().stop();
+  span_close(h, trsm);
   return NNGP_OK;
 }
 
@@ -1238,22 +1239,21 @@ int block_variance(nngp_handle* h, int64_t T, int64_t rows, double* var, std::ve
 // of the DMMA core with K = round_up(N, 16); the columns past N are the tensor maps' zero fill (MatView cols = N).
 //   'nngp': C = K(X*,X*) - V V^T
 //   'ntk' : P = -V M (M symmetric: P -= V M^T on P = 0), C = K(X*,X*) - P V^T - U V^T - V U^T
-int block_covariance(nngp_handle* h, int64_t T, bool solved, const double* var, double* C, int64_t ldc,
-                     std::vector<StageTimer>& timers) {
+int block_covariance(nngp_handle* h, int64_t T, bool solved, const double* var, double* C, int64_t ldc) {
   const int64_t N = h->N, D = h->D, ldl = h->ldl, K = round_up(N, GEMM_BK);
   double* blk = h->blk.as<double>();
   double* xt = h->xt.as<double>();
   const double* qt = h->qt.as<double>();
   if (!solved) {
-    timers.emplace_back(h, &h->st.pred_trsm_ms);
+    const int trsm = span_open(h, 1, h->stream, &h->st.pred_trsm_ms);
     CKR(run_predict_solve(h, blk, ldl, T, h->L.as<double>(), ldl, N, nullptr, nullptr));
-    timers.back().stop();
+    span_close(h, trsm);
   }
   const int lower = T >= 4 * GEMM_BM ? 1 : 0;
-  timers.emplace_back(h, &h->st.pred_gram_ms);
+  const int gram = span_open(h, 1, h->stream, &h->st.pred_gram_ms);
   CKR(run_gram(h, xt, h->ldx, T, qt, xt, h->ldx, T, qt, D, C, ldc, lower, nullptr, nullptr, nullptr, true));
-  timers.back().stop();
-  timers.emplace_back(h, &h->st.pred_var_ms);
+  span_close(h, gram);
+  const int vs = span_open(h, 1, h->stream, &h->st.pred_var_ms);
   const MatView Vv{blk, T, N, ldl};
   if (h->cfg.kernel_type == 1) {
     double* P = h->covP.as<double>();
@@ -1269,7 +1269,7 @@ int block_covariance(nngp_handle* h, int64_t T, bool solved, const double* var, 
   const dim3 mg((unsigned)((T + 31) / 32), (unsigned)((T + 31) / 32));
   mirror_lower_kernel<<<mg, dim3(32, 8), 0, h->stream>>>(C, ldc, (int)T, var);
   h->st.kernel_launches++;
-  timers.back().stop();
+  span_close(h, vs);
   CK(cudaGetLastError());
   return NNGP_OK;
 }
@@ -1522,10 +1522,9 @@ void nngp_destroy(nngp_handle* h) {
                     &h->blk, &h->mean_d, &h->var_d, &h->ssq, &h->sync_ints, &h->Mmat, &h->Kdd, &h->blk2, &h->cov, &h->covP, &h->cross, &h->partial, &h->mean_partial, &h->ka, &h->kb, &h->kqa, &h->kqb, &h->kout, &h->stage, &h->Linv, &h->Linvfull, &h->panel_inv, &h->panel_sync, &h->zkeep, &h->L2, &h->y, &h->app_x, &h->app_y, &h->sel_mean, &h->sel_var, &h->sel_score, &h->sel_key,
                     &h->sel_state, &h->sel_okey, &h->sel_oidx, &h->sel_max, &h->Wq, &h->wscale, &h->Aq, &h->ascale, &h->slscratch, &h->slsync})
     release(*b);
-  for (auto& r : h->pending) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
+  discard_spans(h);
   for (auto e : h->ev_pool) cudaEventDestroy(e);
   for (auto e : h->rep_events) cudaEventDestroy(e);
-  for (auto& sp : h->sliced_spans) { cudaEventDestroy(sp.first); cudaEventDestroy(sp.second); }
   if (h->panel_stream) cudaStreamDestroy(h->panel_stream);
   if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
   if (h->stream) cudaStreamDestroy(h->stream);
@@ -1568,7 +1567,7 @@ int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2, i
   CKR(ensure(h, h->ka, (size_t)M * ldx * 8));
   CKR(ensure(h, h->kqa, (size_t)M * 8));
   CKR(ensure(h, h->kout, (size_t)M * ldo * 8));
-  CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
+  CKR(begin_call(h));
   CKR(upload_matrix(h, x1, M, D, h->ka.as<double>(), ldx));
   CKR(check_finite_async(h, h->ka.as<double>(), ldx, M, D));
   row_sqnorm_kernel<<<(unsigned)((M * 32 + 255) / 256), 256, 0, h->stream>>>(h->ka.as<double>(), ldx, (int)M, (int)D, sw2, sb2, h->kqa.as<double>(), h->flags.as<int>() + 1);
@@ -1595,12 +1594,7 @@ int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2, i
     h->st.kernel_launches++;
   }
   CKR(download(h, h->kout.as<double>(), M, Nn, ldo, k_out));
-  int flags[2];
-  CK(cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  flush_class_events(h);
-  if (flags[1]) return input_error(h, flags[1], "nngp_kernel", "the inputs");
-  return NNGP_OK;
+  return end_call(h, "nngp_kernel", "the inputs");
 }
 
 // -------------------------------------------------------------------------------------------------
@@ -1622,15 +1616,15 @@ static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train
   double* alpha = h->alpha.as<double>();
   double* q = h->q.as<double>();
 
-  StageTimer t_total(h, &h->st.fit_total_ms), t_h2d(h, &h->st.h2d_ms);
-  CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
+  CKR(begin_call(h));
+  const int total = span_open(h, 1, h->stream, &h->st.fit_total_ms), h2d = span_open(h, 1, h->stream, &h->st.h2d_ms);
   CKR(upload_matrix(h, x_train, N, D, X, h->ldx));
   CKR(upload_matrix(h, y_train, N, 1, alpha, 1));
   CK(cudaMemcpyAsync(h->y.p, alpha, (size_t)N * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
-  t_h2d.stop();
+  span_close(h, h2d);
   CKR(check_finite_async(h, alpha, 1, N, 1));
 
-  StageTimer t_gram(h, &h->st.fit_gram_ms);
+  const int gram = span_open(h, 1, h->stream, &h->st.fit_gram_ms);
   CKR(derive_q(h, N, 0));
   const bool ntk = h->cfg.kernel_type == 1;
   if (!ntk) {
@@ -1640,15 +1634,15 @@ static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train
   }
   diag_reg_kernel<<<1, 1024, 0, h->stream>>>(L, h->ldl, (int)N, h->cfg.diag_reg, h->cfg.diag_reg_absolute, h->lam_d.as<double>());
   h->st.kernel_launches++;
-  t_gram.stop();
+  span_close(h, gram);
 
-  StageTimer t_chol(h, &h->st.fit_chol_ms);
+  const int chol = span_open(h, 1, h->stream, &h->st.fit_chol_ms);
   // y^T goes into row N of the factor buffer: the factorisation turns it into z^T = (L^-1 y)^T
   CK(cudaMemcpyAsync(L + N * h->ldl, alpha, (size_t)N * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
   CKR(run_potrf(h, L, h->ldl, N, 1, h->Linv.as<double>()));   // also leaves inv(L_JJ) of every diagonal block in Linv
-  t_chol.stop();
+  span_close(h, chol);
 
-  StageTimer t_solve(h, &h->st.fit_solve_ms);
+  const int solve = span_open(h, 1, h->stream, &h->st.fit_solve_ms);
   lml_terms_kernel<<<1, 1024, 0, h->stream>>>(L, h->ldl, (int)N, L + N * h->ldl, h->lam_d.as<double>() + 1);
   h->st.kernel_launches++;
   CK(cudaMemcpyAsync(h->zkeep.p, L + N * h->ldl, (size_t)N * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
@@ -1662,20 +1656,16 @@ static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train
     h->st.kernel_launches++;
     CKR(run_predict_solve(h, Mm, h->ldl, N, L, h->ldl, N, nullptr, nullptr));   // Mm <- (L^-1 K_dd L^-T)^T = M
   }
-  t_solve.stop();
-  t_total.stop();
+  span_close(h, solve);
+  span_close(h, total);
 
-  int flags[2];
-  CK(cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream));
   CK(cudaMemcpyAsync(&h->lambda, h->lam_d.p, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CK(cudaMemcpyAsync(h->lml_terms, h->lam_d.as<double>() + 1, 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  t_total.collect(); t_h2d.collect(); t_gram.collect(); t_chol.collect(); t_solve.collect();
-  flush_class_events(h);
-  if (flags[1]) return input_error(h, flags[1], "nngp_fit", "x_train / y_train");
-  if (flags[0])
+  int pivot = 0;
+  CKR(end_call(h, "nngp_fit", "x_train / y_train", &pivot));
+  if (pivot)
     return fail(h, NNGP_ENOTPD, "nngp_fit: K + lambda*I is not positive definite (pivot %d of %lld, lambda=%.6g)",
-                flags[0] - 1, (long long)N, h->lambda);
+                pivot - 1, (long long)N, h->lambda);
   return NNGP_OK;
 }
 
@@ -1783,9 +1773,9 @@ static int append_incremental(nngp_handle* h, int64_t M) {
   const int64_t N = h->N, D = h->D, Nn = N + M;
   const int64_t ldo = h->ldl, ldn = round_up(Nn, 16);
   drop_fit(h);   // a half-extended model is not a model (nngp_append_fit publishes the extended one)
-  StageTimer t_total(h, &h->st.fit_total_ms);
+  CKR(begin_call(h));
+  const int total = span_open(h, 1, h->stream, &h->st.fit_total_ms);
   double* Ln = h->L2.as<double>();
-  CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
   // old factor (lower part incl. diagonal blocks) and old z into the new pitch
   CK(cudaMemcpy2DAsync(Ln, ldn * sizeof(double), h->L.p, ldo * sizeof(double), (size_t)N * sizeof(double), N,
                        cudaMemcpyDeviceToDevice, h->stream));
@@ -1803,16 +1793,16 @@ static int append_incremental(nngp_handle* h, int64_t M) {
   CKR(derive_q(h, Nn, N));
   CKR(check_finite_async(h, h->y.as<double>() + N, 1, M, 1));
 
-  StageTimer t_gram(h, &h->st.fit_gram_ms);
+  const int gram = span_open(h, 1, h->stream, &h->st.fit_gram_ms);
   double* L21 = Ln + N * ldn;        // rows N..Nn-1, columns 0..N-1
   double* S = Ln + N * ldn + N;      // the Schur complement block
   CKR(run_gram(h, X + N * h->ldx, h->ldx, M, q + N, X, h->ldx, N, q, D, L21, ldn, 0));                     // K21
   CKR(run_gram(h, X + N * h->ldx, h->ldx, M, q + N, X + N * h->ldx, h->ldx, M, q + N, D, S, ldn, 1));       // K22 (lower)
   diag_reg_kernel<<<1, 1024, 0, h->stream>>>(S, ldn, (int)M, h->cfg.diag_reg, 1, h->lam_d.as<double>());
   h->st.kernel_launches++;
-  t_gram.stop();
+  span_close(h, gram);
 
-  StageTimer t_chol(h, &h->st.fit_chol_ms);
+  const int chol = span_open(h, 1, h->stream, &h->st.fit_chol_ms);
   CKR(run_predict_solve(h, L21, ldn, M, Ln, ldn, N, nullptr, nullptr));                                    // L21 = K21 L11^-T
   {  // [S; y_new^T] -= [L21; z^T] L21^T   (K = N, zero-filled up to a multiple of 16 by the tensor map bounds)
     MatView Av{Ln, Nn + 1, N, ldn};
@@ -1825,27 +1815,23 @@ static int append_incremental(nngp_handle* h, int64_t M) {
   h->N = Nn; h->ldl = ldn;
   CKR(ensure_model(h, Nn, D));   // (the old inverses are no longer needed)
   CKR(run_trtri_diag(h));
-  t_chol.stop();
+  span_close(h, chol);
 
-  StageTimer t_solve(h, &h->st.fit_solve_ms);
+  const int solve = span_open(h, 1, h->stream, &h->st.fit_solve_ms);
   double* zrow = Ln + Nn * ldn;
   lml_terms_kernel<<<1, 1024, 0, h->stream>>>(Ln, ldn, (int)Nn, zrow, h->lam_d.as<double>() + 1);
   h->st.kernel_launches++;
   CK(cudaMemcpyAsync(h->zkeep.p, zrow, (size_t)Nn * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
   CKR(run_trsv_bwd(h, Ln, ldn, Nn, zrow, h->alpha.as<double>(), h->Linv.as<double>()));
-  t_solve.stop();
-  t_total.stop();
+  span_close(h, solve);
+  span_close(h, total);
 
-  int flags[2];
-  CK(cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream));
   CK(cudaMemcpyAsync(h->lml_terms, h->lam_d.as<double>() + 1, 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  t_total.collect(); t_gram.collect(); t_chol.collect(); t_solve.collect();
-  flush_class_events(h);
-  if (flags[1]) return input_error(h, flags[1], "nngp_append_fit", "x_new / y_new");
-  if (flags[0])
+  int pivot = 0;
+  CKR(end_call(h, "nngp_append_fit", "x_new / y_new", &pivot));
+  if (pivot)
     return fail(h, NNGP_ENOTPD, "nngp_append_fit: the extended K + lambda*I is not positive definite (pivot %lld of %lld)",
-                (long long)(N + flags[0] - 1), (long long)Nn);
+                (long long)(N + pivot - 1), (long long)Nn);
   return NNGP_OK;
 }
 
@@ -1936,15 +1922,13 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
   const int col_tiles = (int)((N + GEMM_BN - 1) / GEMM_BN);
   CKR(ensure_predict_workspace(h, N, D, T, want_var));
   if (cov_out) CKR(ensure_cov_workspace(h, N, T));
-  CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
+  CKR(begin_call(h));
 
   double* xt = h->xt.as<double>();
   double* blk = h->blk.as<double>();
-  StageTimer t_total(h, &h->st.pred_total_ms);
-  std::vector<StageTimer> timers;
-  timers.reserve(10 * ((T + TB - 1) / TB) + 8);
-  std::vector<std::pair<cudaEvent_t, cudaEvent_t>> h2d_spans;   // per block, on the copy stream
-  cudaEvent_t ev_xt_free = nullptr;
+  const int total = span_open(h, 1, h->stream, &h->st.pred_total_ms);
+  // ev_landed: a chunk is on the device (one event serves every chunk: a stream wait binds the record before it)
+  cudaEvent_t ev_landed = call_event(h), ev_xt_free = nullptr;
   for (int64_t t0 = 0; t0 < T; t0 += TB) {
     const int64_t rows = std::min<int64_t>(TB, T - t0);
     // Upload and Gram are pipelined in chunks of CH rows: the copy stream runs ahead, the main stream starts the
@@ -1953,17 +1937,14 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
     // independent, so chunking does not change a bit of the result.
     const int64_t CH = 16384;
     const int nchunks = (int)((rows + CH - 1) / CH);
-    cudaEvent_t ev_h2d_a = get_event(h), ev_h2d_b = get_event(h);
-    std::vector<cudaEvent_t> ev_chunk((size_t)nchunks);
-    for (auto& e : ev_chunk) e = get_event(h);
     if (ev_xt_free) CK(cudaStreamWaitEvent(h->copy_stream, ev_xt_free, 0));   // previous block's Gram has read xt
-    CK(cudaEventRecord(ev_h2d_a, h->copy_stream));
-    timers.emplace_back(h, &h->st.pred_gram_ms);
+    const int h2d = span_open(h, 1, h->copy_stream, &h->st.h2d_ms);
+    const int gram = span_open(h, 1, h->stream, &h->st.pred_gram_ms);
     for (int c = 0; c < nchunks; ++c) {
       const int64_t c0 = (int64_t)c * CH, cr = std::min<int64_t>(CH, rows - c0);
       CKR(upload_matrix(h, x_test + (t0 + c0) * D, cr, D, xt + c0 * ldx, ldx, h->copy_stream));
-      CK(cudaEventRecord(ev_chunk[(size_t)c], h->copy_stream));
-      CK(cudaStreamWaitEvent(h->stream, ev_chunk[(size_t)c], 0));
+      CK(cudaEventRecord(ev_landed, h->copy_stream));
+      CK(cudaStreamWaitEvent(h->stream, ev_landed, 0));
       CKR(check_finite_async(h, xt + c0 * ldx, ldx, cr, D));
       double* qt_c = h->qt.as<double>() + c0;
       double* mp_c = h->mean_partial.as<double>() + c0 * 2 * col_tiles;
@@ -1974,12 +1955,10 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
       mean_reduce_kernel<<<(unsigned)((cr + 255) / 256), 256, 0, h->stream>>>(mp_c, 2 * col_tiles, (int)cr, h->mean_d.as<double>() + t0 + c0);
       h->st.kernel_launches++;
     }
-    timers.back().stop();
-    CK(cudaEventRecord(ev_h2d_b, h->copy_stream));
-    h2d_spans.push_back({ev_h2d_a, ev_h2d_b});
-    if (!ev_xt_free) ev_xt_free = get_event(h);
+    span_close(h, gram);
+    span_close(h, h2d);
+    if (!ev_xt_free) ev_xt_free = call_event(h);
     CK(cudaEventRecord(ev_xt_free, h->stream));   // the next block's upload may overlap this block's solve
-    for (auto e : ev_chunk) h->ev_pool.push_back(e);
 
     if (want_var) {
       LayerSig sig;
@@ -1987,36 +1966,17 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
       q_final_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, h->stream>>>(h->qt.as<double>(), (int)rows, h->cfg.depth - 1, sig, h->kss.as<double>());
       h->st.kernel_launches++;
       bool solved = false;
-      CKR(block_variance(h, T, rows, h->var_d.as<double>() + t0, timers, &solved));
-      if (cov_out) CKR(block_covariance(h, T, solved, h->var_d.as<double>(), h->cov.as<double>(), round_up(T, 2), timers));
+      CKR(block_variance(h, T, rows, h->var_d.as<double>() + t0, &solved));
+      if (cov_out) CKR(block_covariance(h, T, solved, h->var_d.as<double>(), h->cov.as<double>(), round_up(T, 2)));
     }
   }
-  timers.emplace_back(h, &h->st.d2h_ms);
+  const int d2h = span_open(h, 1, h->stream, &h->st.d2h_ms);
   CKR(download(h, h->mean_d.as<double>(), T, 1, 1, mean_out));
   if (var_out) CKR(download(h, h->var_d.as<double>(), T, 1, 1, var_out));
   if (cov_out) CKR(download(h, h->cov.as<double>(), T, T, round_up(T, 2), cov_out));
-  timers.back().stop();
-  t_total.stop();
-  int flags[2];
-  CK(cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CK(cudaGetLastError());
-  t_total.collect();
-  for (auto& t : timers) t.collect();
-  if (ev_xt_free) h->ev_pool.push_back(ev_xt_free);
-  for (auto& sp : h->sliced_spans) {
-    float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, sp.first, sp.second) == cudaSuccess) h->st.sliced_ms += ms;
-    h->ev_pool.push_back(sp.first); h->ev_pool.push_back(sp.second);
-  }
-  h->sliced_spans.clear();
-  for (auto& sp : h2d_spans) {
-    float ms = 0.f;
-    if (h->cfg.stats_level >= 1 && cudaEventElapsedTime(&ms, sp.first, sp.second) == cudaSuccess) h->st.h2d_ms += ms;
-    h->ev_pool.push_back(sp.first); h->ev_pool.push_back(sp.second);
-  }
-  flush_class_events(h);
-  if (flags[1]) return input_error(h, flags[1], cov_out ? "nngp_predict_cov" : "nngp_predict", "x_test");
+  span_close(h, d2h);
+  span_close(h, total);
+  CKR(end_call(h, cov_out ? "nngp_predict_cov" : "nngp_predict", "x_test"));
   h->st.queries += T;
   return NNGP_OK;
 }
@@ -2077,14 +2037,10 @@ int nngp_get_state(nngp_handle* h, double* x_out, double* l_out, double* alpha_o
 // The tail of nngp_set_state / nngp_state_import_end: X, L and alpha are on the device.  X gets the checks of a fit
 // (the handle stays unfitted if it fails them); q and inv(L_JJ) are derived, then the state is published.
 static int finish_import(nngp_handle* h, double lambda, bool have_M, const char* who) {
-  CK(cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream));
+  CKR(begin_call(h));
   CKR(derive_q(h, h->N, 0));
   CKR(run_trtri_diag(h));
-  int flags[2];
-  CK(cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  CK(cudaGetLastError());
-  if (flags[1]) return input_error(h, flags[1], who, "x");
+  CKR(end_call(h, who, "x"));
   h->lambda = lambda;
   return publish_state(h, false, have_M);
 }
@@ -2238,6 +2194,7 @@ int nngp_diag_gemm_probe(nngp_handle* h, int64_t M, int64_t N, int64_t K, int32_
   cudaMemsetAsync(B.p, 0, (size_t)N * ld * 8, h->stream);
   cudaMemsetAsync(C.p, 0, (size_t)M * ldc * 8, h->stream);
   MatView Av{A.as<double>(), M, K, ld}, Bv{B.as<double>(), N, K, ld};
+  discard_spans(h);   // (spans of a failed earlier call)
   rc = run_gemm_sub(h, Av, 0, 0, Bv, 0, 0, M, N, K, C.as<double>(), ldc, 0);  // warm-up
   cudaEvent_t a = get_event(h), b = get_event(h);
   cudaEventRecord(a, h->stream);
@@ -2247,7 +2204,7 @@ int nngp_diag_gemm_probe(nngp_handle* h, int64_t M, int64_t N, int64_t K, int32_
   float ms = 0.f;
   cudaEventElapsedTime(&ms, a, b);
   h->ev_pool.push_back(a); h->ev_pool.push_back(b);
-  flush_class_events(h);
+  settle_spans(h);
   h->tmaps.clear();  // the scratch operands are about to be freed
   release(A); release(B); release(C);
   if (rc != NNGP_OK) return rc;
@@ -2262,21 +2219,18 @@ int nngp_diag_potrf(nngp_handle* h, double* a, int64_t N) {
   const int64_t ld = round_up(N, 16);
   DevBuf A, W;   // the matrix and the inverses of its diagonal blocks
   CKR(ensure(h, A, (size_t)N * ld * 8));
-  int rc = NNGP_OK;
-  cudaMemsetAsync(h->flags.p, 0, 2 * sizeof(int), h->stream);
-  rc = upload_matrix(h, a, N, N, A.as<double>(), ld);
+  int rc = begin_call(h);
+  if (rc == NNGP_OK) rc = upload_matrix(h, a, N, N, A.as<double>(), ld);
   if (rc == NNGP_OK) rc = ensure(h, W, (size_t)round_up(N, NB) * NB * sizeof(double));
   if (rc == NNGP_OK) rc = run_potrf(h, A.as<double>(), ld, N, 0, W.as<double>());
   if (rc == NNGP_OK) rc = download(h, A.as<double>(), N, N, ld, a);
-  int flags[2] = {0, 0};
-  cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream);
-  cudaError_t e = cudaStreamSynchronize(h->stream);
-  flush_class_events(h);
+  int pivot = 0;
+  if (rc == NNGP_OK) rc = end_call(h, "nngp_diag_potrf", "a", &pivot);
+  cudaStreamSynchronize(h->stream);   // (also after a failure: A and W are freed next)
   h->tmaps.clear();
   release(A); release(W);
   if (rc != NNGP_OK) return rc;
-  if (e != cudaSuccess) return fail(h, NNGP_ECUDA, "potrf failed: %s", cudaGetErrorString(e));
-  if (flags[0]) return fail(h, NNGP_ENOTPD, "nngp_diag_potrf: not positive definite (pivot %d)", flags[0] - 1);
+  if (pivot) return fail(h, NNGP_ENOTPD, "nngp_diag_potrf: not positive definite (pivot %d)", pivot - 1);
   return NNGP_OK;
 }
 
