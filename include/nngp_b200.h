@@ -133,8 +133,42 @@ typedef struct nngp_handle nngp_handle;
  * relative) -- train.py:161-172. */
 NNGP_API void nngp_default_config(nngp_config* cfg);
 
-/* Create a handle on one GPU.  [replaces: closure construction, train.py:161-172] */
+/* Create a handle on one GPU.  [replaces: closure construction, train.py:161-172]
+ * Same as nngp_create_with_activation(cfg, NULL, out): every hidden step is a ReLU. */
 NNGP_API int nngp_create(const nngp_config* cfg, nngp_handle** out);
+
+/*
+ * The activation of the hidden steps: one activation for every step of the chain Dense (act Dense)* (per_layer
+ * sigmas still apply).  For the step that maps the previous Dense layer's pre-activation covariance (q1, q2, k) to the
+ * next one, with s = sqrt(max(q1 q2 - k^2, 0)) and theta = atan2(s, k):
+ *   k'   = sigma_w^2 E[phi(u) phi(v)] + sigma_b^2,   q' = sigma_w^2 E[phi(u)^2] + sigma_b^2,
+ *   ntk' = k' + sigma_w^2 ntk E[phi'(u) phi'(v)]     (kernel_type 'ntk')
+ * NNGP_ACT_RELU   max(x, 0)                       the default; a, b, c are ignored
+ * NNGP_ACT_ABRELU a min(x, 0) + b max(x, 0)       [nt 0.6.1 stax.ABRelu; LeakyRelu(alpha) = (alpha, 1), Abs = (-1, 1)]
+ *                 E[phi phi] = (a-b)^2/(2 pi) s + kdot k,  kdot = (a^2+b^2)/2 - (a-b)^2 theta/(2 pi)
+ * NNGP_ACT_ERF    a erf(b x) + c                  [nt 0.6.1 stax.Erf]; b != 0; with Q = b^2 q, K = b^2 k,
+ *                 P = (1 + 2 Q1)(1 + 2 Q2) - 4 K^2:  E[phi phi] = a^2 (2/pi) atan2(2K, sqrt P) + c^2,
+ *                 kdot = a^2 b^2 (4/pi) / sqrt P
+ * a, b and c must be finite; kind must be one of the three.  Erf also needs b^2, a^2 b^2 and c^2 to be finite normal
+ * (or zero) doubles, and every hidden layer's diagonal bound sigma_w^2 (a^2 + c^2) + sigma_b^2 (E[phi^2] <= a^2 + c^2)
+ * to satisfy the Erf input range below.  Anything else is NNGP_EINVAL with a message.
+ * Erf input range: on top of nngp_kernel's, every row's layer-0 diagonal q must have b^2 q < 2^508 (NNGP_EINVAL
+ * otherwise); within it the Erf kernel needs no range guard (DESIGN.md 5.12).
+ * ABRelu input range: every step forms q q', so the diagonal entering every step, sigma_w^2 (a^2+b^2)/2 q +
+ * sigma_b^2 after the previous one, must stay below 2^512 like the layer-0 one; that bound is carried back to a
+ * limit on the layer-0 q (NNGP_EINVAL above it, and at creation if sigma_b^2 alone reaches it).
+ * act == NULL or kind == NNGP_ACT_RELU is exactly nngp_create.  A handle with n_gpus > 1 uses the activation on
+ * every GPU.
+ */
+#define NNGP_ACT_RELU 0
+#define NNGP_ACT_ABRELU 1
+#define NNGP_ACT_ERF 2
+typedef struct nngp_activation {
+  int32_t kind;      /* NNGP_ACT_*                          */
+  int32_t reserved;  /* 0                                   */
+  double a, b, c;    /* ABRelu (a, b); Erf (a, b, c)        */
+} nngp_activation;
+NNGP_API int nngp_create_with_activation(const nngp_config* cfg, const nngp_activation* act, nngp_handle** out);
 NNGP_API void nngp_destroy(nngp_handle* h);
 
 /* Message of the last failing call on this handle (or of a failed nngp_create when
@@ -152,8 +186,8 @@ NNGP_API void* nngp_get_stream(nngp_handle* h);
  * x1: M x D, x2: N2 x D (NULL => x2 = x1, N2 ignored), k_out: M x N2.
  *
  * Accepted input range (nngp_kernel, nngp_fit, nngp_append_fit, nngp_predict): every element finite, and every
- * row's layer-0 diagonal q = sigma_w^2 |x|^2 / D + sigma_b^2 below 2^512, so that q q' is a finite double;
- * anything else is NNGP_EINVAL.  nngp_set_state and nngp_state_import_end hold the imported X to the same range
+ * row's layer-0 diagonal q = sigma_w^2 |x|^2 / D + sigma_b^2 below 2^512, so that q q' is a finite double (with an
+ * Erf(a, b, c) activation also b^2 q below 2^508, see nngp_activation); anything else is NNGP_EINVAL.  nngp_set_state and nngp_state_import_end hold the imported X to the same range
  * (NNGP_EINVAL, the handle is left without a fitted model).  There is no lower bound: rows down to the subnormal range (and zero rows) are
  * accepted, but an entry whose q, q q' or k^2 is subnormal carries fewer significant bits.
  */
@@ -201,7 +235,7 @@ NNGP_API int nngp_predict_cov(nngp_handle* h, const double* x_test, int64_t T, d
  * nngp_get_state copies X (N x D), L (N x N row-major lower factor, upper triangle
  * zero) and alpha (N); any pointer may be NULL to skip it.
  * nngp_set_state installs a state produced by nngp_get_state on a handle with the
- * same config. */
+ * same config and the same activation (nngp_create_with_activation): the state does not record either. */
 NNGP_API int nngp_get_dims(nngp_handle* h, int64_t* N, int64_t* D, double* lambda_out);
 NNGP_API int nngp_get_state(nngp_handle* h, double* x_out, double* l_out, double* alpha_out);
 NNGP_API int nngp_set_state(nngp_handle* h, const double* x, const double* l, const double* alpha, int64_t N,
@@ -280,7 +314,8 @@ NNGP_API int nngp_sliced_product(nngp_handle* h, const double* a, int64_t M, int
  * nngp_state_packed_size reports its length; nngp_state_pack copies elements [offset, offset+count) into `dst`
  * (host or device memory); on the receiving side nngp_state_import_begin sizes the buffers,
  * nngp_state_unpack stores a range, nngp_state_import_end derives the rest (layer-0 diagonal, diagonal-block
- * inverses, replicas) and marks the handle fitted.  Every call is complete when it returns. */
+ * inverses, replicas) and marks the handle fitted.  Every call is complete when it returns.  The receiving handle
+ * needs the same config and activation as the one that packed the state. */
 NNGP_API int nngp_state_packed_size(nngp_handle* h, int64_t* n_doubles);
 NNGP_API int nngp_state_pack(nngp_handle* h, int64_t offset, int64_t count, double* dst);
 NNGP_API int nngp_state_import_begin(nngp_handle* h, int64_t N, int64_t D);

@@ -7,6 +7,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cfloat>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -60,6 +61,8 @@ inline int64_t round_up(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
 struct nngp_handle {
   nngp_config cfg;
   double lsw2[NNGP_MAX_LAYERS], lsb2[NNGP_MAX_LAYERS];   // sigma_w^2 / sigma_b^2 of Dense layer l (uniform: all alike)
+  ActCoef act{};         // activation of every hidden step (make_act_coef)
+  double q_limit = 0.0;  // layer-0 diagonals must stay below this (row_sqnorm_kernel's range flag)
   int device = 0;
   // cfg.n_gpus > 1: replicas of the fitted state on the other GPUs (each a complete single-GPU handle with its own
   // streams and workspace; nngp_predict runs them on one host thread each).  `owner` is set on a replica.
@@ -107,6 +110,7 @@ struct nngp_handle {
   DevBuf cov, covP;
   // nngp_kernel workspace
   DevBuf ka, kb, kqa, kqb, kout;
+  DevBuf qtab;    // Erf, depth > 2: the per-row diagonal tables of the operands of the current Gram launch (run_gram)
   DevBuf stage;   // nngp_state_pack / _unpack with host memory on the other side: one range at a time
   // nngp_active_select workspace
   DevBuf sel_mean, sel_var, sel_score, sel_key, sel_state, sel_okey, sel_oidx, sel_max;
@@ -266,7 +270,7 @@ struct MatView {  // a whole device matrix a tensor map is built over
 };
 
 // ---- GEMM launches ----------------------------------------------------------------------------
-template <int EPI>
+template <int EPI, int ACT = ACT_RELU>
 int launch_gemm(nngp_handle* h, const MatView& A, int a_row0, int a_col0, const MatView& B, int b_row0, int b_col0,
                 GemmParams p, int grid_z = 1) {
   if (p.M <= 0 || p.N <= 0) return NNGP_OK;
@@ -278,7 +282,7 @@ int launch_gemm(nngp_handle* h, const MatView& A, int a_row0, int a_col0, const 
   if (grid.y > 65535) return fail(h, NNGP_EINVAL, "internal: GEMM row range too large (%d rows)", p.M);
   // (ROWDOT counts as a GEMM-class launch)
   const int span = span_open(h, 2, h->cur, EPI == EPI_GRAM ? &h->st.gram_ms : &h->st.gemm_ms);
-  gemm_nt_kernel<EPI><<<grid, GEMM_THREADS, GEMM_SMEM_BYTES, h->cur>>>(tmA, tmB, p);
+  gemm_nt_kernel<EPI, ACT><<<grid, GEMM_THREADS, GEMM_SMEM_BYTES, h->cur>>>(tmA, tmB, p);
   span_close(h, span);
   CK(cudaGetLastError());
   h->st.kernel_launches++;
@@ -298,6 +302,15 @@ int launch_gemm(nngp_handle* h, const MatView& A, int a_row0, int a_col0, const 
   return NNGP_OK;
 }
 
+// sigma_w^2 / sigma_b^2 of the Dense layer that follows activation step s
+LayerSig layer_sig(const nngp_handle* h) {
+  LayerSig sig;
+  for (int i = 0; i < 16; ++i) { sig.sw2[i] = h->lsw2[std::min(i + 1, NNGP_MAX_LAYERS - 1)]; sig.sb2[i] = h->lsb2[std::min(i + 1, NNGP_MAX_LAYERS - 1)]; }
+  return sig;
+}
+
+size_t act_table_bytes(const nngp_handle* h, int64_t rows);   // (device buffer sizes, below)
+
 // K(A rows, B rows) -> out (M x N, ld ldo).  A: M x D (lda), B: N x D (ldb); qa/qb layer-0 diagonals.
 // In NTK mode (cfg.kernel_type == 1) `out` receives Theta and `out2` (optional) the NNGP kernel K -- unless
 // `nngp_only`: then `out` receives K in either mode.
@@ -305,6 +318,7 @@ int run_gram(nngp_handle* h, const double* A, int64_t lda, int64_t M, const doub
              int64_t N, const double* qb, int64_t D, double* out, int64_t ldo, int lower, double* out2 = nullptr,
              const double* alpha = nullptr, double* mean_partial = nullptr, bool nngp_only = false) {
   GemmParams p{};
+  p.act = h->act;
   p.alpha = alpha; p.mean_partial = mean_partial;
   p.ntk = h->cfg.kernel_type == 1 && !nngp_only ? 1 : 0;
   p.C2 = out2;
@@ -318,7 +332,29 @@ int run_gram(nngp_handle* h, const double* A, int64_t lda, int64_t M, const doub
     p.lsb2[i] = h->lsb2[std::min(i + 1, NNGP_MAX_LAYERS - 1)];
   }
   MatView a{A, M, D, lda}, b{B, N, D, ldb};
-  return launch_gemm<EPI_GRAM>(h, a, 0, 0, b, 0, 0, p);
+  if (h->act.kind == ACT_ERF && p.steps > 1 && M > 0 && N > 0) {
+    // the diagonals of layers 1..steps-1 of both operands (one table when both are the same rows), on the stream of
+    // the launch that reads them
+    const bool same = qa == qb && M == N;
+    if (h->qtab.cap < act_table_bytes(h, same ? M : M + N))
+      return fail(h, NNGP_EINVAL, "internal: diagonal tables sized for fewer than %lld rows", (long long)(same ? M : M + N));
+    double* ta = h->qtab.as<double>();
+    double* tb = same ? ta : ta + (int64_t)(p.steps - 1) * M;
+    const LayerSig sig = layer_sig(h);
+    q_final_kernel<<<(unsigned)((M + 255) / 256), 256, 0, h->cur>>>(qa, (int)M, p.steps, sig, h->act, ta, nullptr);
+    h->st.kernel_launches++;
+    if (!same) {
+      q_final_kernel<<<(unsigned)((N + 255) / 256), 256, 0, h->cur>>>(qb, (int)N, p.steps, sig, h->act, tb, nullptr);
+      h->st.kernel_launches++;
+    }
+    p.tab1 = ta; p.tld1 = M;
+    p.tab2 = tb; p.tld2 = N;
+  }
+  switch (h->act.kind) {
+    case ACT_ABRELU: return launch_gemm<EPI_GRAM, ACT_ABRELU>(h, a, 0, 0, b, 0, 0, p);
+    case ACT_ERF: return launch_gemm<EPI_GRAM, ACT_ERF>(h, a, 0, 0, b, 0, 0, p);
+    default: return launch_gemm<EPI_GRAM>(h, a, 0, 0, b, 0, 0, p);
+  }
 }
 
 // C(M x N at `C`, ldc) -= Aop[a_row0:+M, a_col0:+K] * Bop[b_row0:+N, b_col0:+K]^T ; K % 16 == 0.
@@ -413,6 +449,17 @@ int ensure_sliced_block(nngp_handle* h, int64_t N, int64_t rows) {
   return sliced_grid(h, sb, N, &grid, &rounds);
 }
 
+// Erf, depth > 2: the diagonal tables of layers 1..depth-2 for a Gram launch over `rows` distinct operand rows
+// (run_gram; every caller sizes them for its largest launch)
+size_t act_table_bytes(const nngp_handle* h, int64_t rows) {
+  const int64_t steps = h->cfg.depth - 1;
+  return h->act.kind == ACT_ERF && steps >= 2 ? (size_t)(steps - 1) * rows * sizeof(double) : 0;
+}
+int ensure_act_tables(nngp_handle* h, int64_t rows) {
+  const size_t bytes = act_table_bytes(h, rows);
+  return bytes ? ensure(h, h->qtab, bytes) : NNGP_OK;
+}
+
 // the training rows X and their layer-0 diagonals q
 int ensure_inputs(nngp_handle* h, int64_t N, int64_t D) {
   CKR(ensure(h, h->X, (size_t)N * round_up(D, 2) * sizeof(double)));
@@ -425,6 +472,7 @@ int ensure_model(nngp_handle* h, int64_t N, int64_t D) {
   const int64_t ldl = round_up(N, 16), ldq = round_up(N, SL_BK);
   const int s = h->cfg.variance_slices;
   CKR(ensure_inputs(h, N, D));
+  CKR(ensure_act_tables(h, N));
   CKR(ensure(h, h->L, (size_t)(N + 1) * ldl * sizeof(double)));
   CKR(ensure(h, h->alpha, (size_t)ldl * sizeof(double)));
   CKR(ensure(h, h->Linv, (size_t)round_up(N, NB) * NB * sizeof(double)));
@@ -453,6 +501,7 @@ int ensure_fit_workspace(nngp_handle* h, int64_t N) {
 int ensure_append_workspace(nngp_handle* h, int64_t N, int64_t D) {
   CKR(ensure(h, h->app_x, (size_t)N * D * sizeof(double)));
   CKR(ensure(h, h->app_y, (size_t)N * sizeof(double)));
+  CKR(ensure_act_tables(h, N));   // (the incremental append's K21: the M new rows against the N - M old ones)
   if (!can_append_incrementally(h)) return NNGP_OK;
   CKR(ensure(h, h->L2, (size_t)(N + 1) * round_up(N, 16) * sizeof(double)));
   return ensure(h, h->panel_inv, (size_t)round_up(N, NB) * NB * sizeof(double));
@@ -477,6 +526,7 @@ int ensure_predict_workspace(nngp_handle* h, int64_t N, int64_t D, int64_t T, bo
   CKR(ensure(h, h->blk, (size_t)TB * ldl * sizeof(double)));
   CKR(ensure(h, h->mean_partial, (size_t)TB * 2 * ((N + GEMM_BN - 1) / GEMM_BN) * sizeof(double)));  // per 32 columns
   CKR(ensure(h, h->mean_d, (size_t)T * sizeof(double)));
+  CKR(ensure_act_tables(h, TB + N));   // (a chunk of the block against the training rows; the covariance: TB rows)
   if (!want_var) return NNGP_OK;
   CKR(ensure(h, h->var_d, (size_t)T * sizeof(double)));
   CKR(ensure_solve_workspace(h, TB));
@@ -1019,6 +1069,10 @@ int check_finite_async(nngp_handle* h, const double* x, int64_t ld, int64_t rows
 // flags[1] after check_finite_async (bit 0) and row_sqnorm_kernel with range_flag (bit 1) -> the caller's error
 int input_error(nngp_handle* h, int flag, const char* who, const char* what) {
   if (flag & 1) return fail(h, NNGP_EINVAL, "%s: non-finite value in %s", who, what);
+  if (h->act.kind != ACT_RELU)
+    return fail(h, NNGP_EINVAL,
+                "%s: %s out of range: a row's layer-0 kernel diagonal q = sigma_w^2 |x|^2 / D + sigma_b^2 must stay below "
+                "%.17g (every layer's diagonal below 2^512; Erf: b^2 q below 2^508)", who, what, h->q_limit);
   return fail(h, NNGP_EINVAL,
               "%s: %s out of range: a row's layer-0 kernel diagonal sigma_w^2 |x|^2 / D + sigma_b^2 reaches 2^512 "
               "(the kernel needs q q' < 2^1024)", who, what);
@@ -1050,7 +1104,7 @@ int end_call(nngp_handle* h, const char* who, const char* what, int* pivot = nul
 int derive_q(nngp_handle* h, int64_t rows, int64_t new0) {
   const double* X = h->X.as<double>();
   CKR(check_finite_async(h, X + new0 * h->ldx, h->ldx, rows - new0, h->D));
-  row_sqnorm_kernel<<<(unsigned)((rows * 32 + 255) / 256), 256, 0, h->stream>>>(X, h->ldx, (int)rows, (int)h->D, h->lsw2[0], h->lsb2[0], h->q.as<double>(), h->flags.as<int>() + 1);
+  row_sqnorm_kernel<<<(unsigned)((rows * 32 + 255) / 256), 256, 0, h->stream>>>(X, h->ldx, (int)rows, (int)h->D, h->lsw2[0], h->lsb2[0], h->q.as<double>(), h->flags.as<int>() + 1, h->q_limit);
   h->st.kernel_launches++;
   return NNGP_OK;
 }
@@ -1297,7 +1351,64 @@ void nngp_default_config(nngp_config* cfg) {
 
 const char* nngp_last_error(const nngp_handle* h) { return h ? h->err.c_str() : g_create_error.c_str(); }
 
-static int create_single(const nngp_config* cfg, nngp_handle** out) {
+// Checks the activation of a new handle (cfg already checked) and derives its step coefficients and the limit of the
+// layer-0 diagonals (nngp_activation in the header).  NULL / NNGP_ACT_RELU: ReLU, the limit 2^512.
+static int make_act_coef(const nngp_config* cfg, const nngp_activation* act, ActCoef* c, double* q_limit) {
+  const double inv_2pi = 0.15915494309189533577, two_over_pi = 0.63661977236758134308;
+  *c = ActCoef{};
+  c->kind = ACT_RELU; c->c0 = 0.5; c->c1 = inv_2pi;
+  *q_limit = Q_LIMIT;
+  if (!act || act->kind == NNGP_ACT_RELU) return NNGP_OK;
+  const char* who = "nngp_create_with_activation";
+  if (act->kind != NNGP_ACT_ABRELU && act->kind != NNGP_ACT_ERF)
+    return fail(nullptr, NNGP_EINVAL, "%s: unknown activation kind %d (NNGP_ACT_RELU, _ABRELU or _ERF)", who, act->kind);
+  const double a = act->a, b = act->b, cc = act->c;
+  if (!std::isfinite(a) || !std::isfinite(b) || !std::isfinite(cc))
+    return fail(nullptr, NNGP_EINVAL, "%s: a, b and c must be finite (got %g, %g, %g)", who, a, b, cc);
+  if (act->kind == NNGP_ACT_ABRELU) {
+    c->kind = ACT_ABRELU;
+    c->c0 = (a * a + b * b) * 0.5;
+    c->c1 = (a - b) * (a - b) * inv_2pi;
+    if (!std::isfinite(c->c0) || !std::isfinite(c->c1))
+      return fail(nullptr, NNGP_EINVAL, "%s: ABRelu(%g, %g): a^2 + b^2 overflows", who, a, b);
+    // Every step forms q q', so the diagonal entering each step must stay below 2^512 like the layer-0 one.  Later
+    // diagonals are q_l = sigma_w_l^2 c0 q_(l-1) + sigma_b_l^2: carry that bound back to a limit on the layer-0 q.
+    double lim = Q_LIMIT;
+    for (int l = cfg->depth - 1; l >= 1; --l) {
+      const double w = cfg->per_layer ? cfg->sigma_w_layers[l] : cfg->sigma_w;
+      const double sb = cfg->per_layer ? cfg->sigma_b_layers[l] : cfg->sigma_b;
+      lim = std::min(Q_LIMIT, (lim - sb * sb) / (w * w * c->c0));
+      if (!(lim > 0.0))
+        return fail(nullptr, NNGP_EINVAL, "%s: ABRelu(%g, %g): the diagonal of Dense layer %d reaches 2^512 for every "
+                    "input", who, a, b, l);
+    }
+    *q_limit = lim;
+    return NNGP_OK;
+  }
+  const double b2 = b * b;
+  if (!(b2 >= DBL_MIN) || !std::isfinite(b2))
+    return fail(nullptr, NNGP_EINVAL, "%s: Erf needs b != 0 with b^2 a finite normal double (got b = %g)", who, b);
+  c->kind = ACT_ERF;
+  c->b2x2 = 2.0 * b2;
+  c->e = a * a * two_over_pi;
+  c->c2 = cc * cc;
+  c->kd = a * a * b2 * (2.0 * two_over_pi);
+  if (!std::isfinite(c->e) || !std::isfinite(c->c2) || !std::isfinite(c->kd))
+    return fail(nullptr, NNGP_EINVAL, "%s: Erf(%g, %g, %g): a^2, c^2 or a^2 b^2 overflows", who, a, b, cc);
+  *q_limit = std::min(Q_LIMIT, ERF_Q_LIMIT / b2);
+  // the diagonal entering every later step is sigma_w^2 E[phi^2] + sigma_b^2 <= sigma_w^2 (a^2 + c^2) + sigma_b^2
+  for (int l = 1; l < std::min(cfg->depth, NNGP_MAX_LAYERS); ++l) {
+    const double w = cfg->per_layer ? cfg->sigma_w_layers[l] : cfg->sigma_w;
+    const double sb = cfg->per_layer ? cfg->sigma_b_layers[l] : cfg->sigma_b;
+    const double bound = w * w * (a * a + cc * cc) + sb * sb;
+    if (!(bound < Q_LIMIT) || !(b2 * bound < ERF_Q_LIMIT))
+      return fail(nullptr, NNGP_EINVAL, "%s: Erf(%g, %g, %g): the diagonal of Dense layer %d can reach %g; it needs "
+                  "b^2 q < 2^508", who, a, b, cc, l, bound);
+  }
+  return NNGP_OK;
+}
+
+static int create_single(const nngp_config* cfg, const nngp_activation* act, nngp_handle** out) {
   nngp_handle* h = nullptr;
   if (!cfg || !out) return fail(h, NNGP_EINVAL, "nngp_create: null argument");
   *out = nullptr;
@@ -1313,6 +1424,9 @@ static int create_single(const nngp_config* cfg, nngp_handle** out) {
       if (!(cfg->sigma_w_layers[l] > 0.0) || !(cfg->sigma_b_layers[l] >= 0.0))
         return fail(h, NNGP_EINVAL, "nngp_create: layer %d needs sigma_w > 0, sigma_b >= 0", l);
   }
+  ActCoef coef;
+  double q_limit;
+  CKR(make_act_coef(cfg, act, &coef, &q_limit));
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     cudaGetLastError();
@@ -1334,6 +1448,8 @@ static int create_single(const nngp_config* cfg, nngp_handle** out) {
     return fail(h, NNGP_EINVAL, "nngp_create: variance_slices applies to kernel_type 0 ('nngp') only");
   nngp_handle* nh = new nngp_handle();
   nh->cfg = *cfg;
+  nh->act = coef;
+  nh->q_limit = q_limit;
   if (nh->cfg.variance_slices > 0) nh->cfg.latency_mode = 1;   // the digit planes are those of the explicit inverse
   for (int l = 0; l < NNGP_MAX_LAYERS; ++l) {
     const int ll = std::min(l, std::max(cfg->depth - 1, 0));
@@ -1375,6 +1491,8 @@ static int create_single(const nngp_config* cfg, nngp_handle** out) {
   }
   h->encode = reinterpret_cast<PFN_encodeTiled>(fn);
   cudaError_t e1 = cudaFuncSetAttribute(gemm_nt_kernel<EPI_GRAM>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES);
+  if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(gemm_nt_kernel<EPI_GRAM, ACT_ABRELU>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES);
+  if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(gemm_nt_kernel<EPI_GRAM, ACT_ERF>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES);
   cudaError_t e2 = cudaFuncSetAttribute(gemm_nt_kernel<EPI_SUB>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES);
   if (e2 == cudaSuccess) e2 = cudaFuncSetAttribute(gemm_nt_kernel<EPI_ROWDOT>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES);
   cudaError_t e3 = cudaFuncSetAttribute(trsm_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TF_SMEM_BYTES);
@@ -1394,7 +1512,9 @@ static int create_single(const nngp_config* cfg, nngp_handle** out) {
   return NNGP_OK;
 }
 
-int nngp_create(const nngp_config* cfg, nngp_handle** out) {
+int nngp_create(const nngp_config* cfg, nngp_handle** out) { return nngp_create_with_activation(cfg, nullptr, out); }
+
+int nngp_create_with_activation(const nngp_config* cfg, const nngp_activation* act, nngp_handle** out) {
   nngp_handle* h = nullptr;
   if (!cfg || !out) return fail(h, NNGP_EINVAL, "nngp_create: null argument");
   *out = nullptr;
@@ -1402,7 +1522,7 @@ int nngp_create(const nngp_config* cfg, nngp_handle** out) {
   if (G > NNGP_MAX_GPUS) return fail(h, NNGP_EINVAL, "nngp_create: n_gpus=%d exceeds NNGP_MAX_GPUS=%d", G, NNGP_MAX_GPUS);
   nngp_config c0 = *cfg;
   c0.n_gpus = 1;
-  if (G == 1) return create_single(&c0, out);
+  if (G == 1) return create_single(&c0, act, out);
   int ids[NNGP_MAX_GPUS];
   bool any = false;
   for (int g = 0; g < G; ++g) any = any || cfg->device_ids[g] >= 0;
@@ -1412,12 +1532,12 @@ int nngp_create(const nngp_config* cfg, nngp_handle** out) {
       if (ids[g] == ids[k] || ids[g] < 0)
         return fail(h, NNGP_EINVAL, "nngp_create: device_ids must be %d distinct CUDA ordinals", G);
   c0.device = ids[0];
-  CKR(create_single(&c0, &h));
+  CKR(create_single(&c0, act, &h));
   for (int g = 1; g < G; ++g) {
     nngp_config cg = c0;
     cg.device = ids[g];
     nngp_handle* p = nullptr;
-    const int rc = create_single(&cg, &p);
+    const int rc = create_single(&cg, act, &p);
     if (rc != NNGP_OK) { nngp_destroy(h); return rc; }   // g_create_error holds the message
     p->owner = h;
     h->peers.push_back(p);
@@ -1519,7 +1639,7 @@ void nngp_destroy(nngp_handle* h) {
   cudaSetDevice(h->device);
   if (h->stream) cudaStreamSynchronize(h->stream);
   for (DevBuf* b : {&h->X, &h->q, &h->L, &h->alpha, &h->flags, &h->lam_d, &h->xt, &h->qt, &h->kss,
-                    &h->blk, &h->mean_d, &h->var_d, &h->ssq, &h->sync_ints, &h->Mmat, &h->Kdd, &h->blk2, &h->cov, &h->covP, &h->cross, &h->partial, &h->mean_partial, &h->ka, &h->kb, &h->kqa, &h->kqb, &h->kout, &h->stage, &h->Linv, &h->Linvfull, &h->panel_inv, &h->panel_sync, &h->zkeep, &h->L2, &h->y, &h->app_x, &h->app_y, &h->sel_mean, &h->sel_var, &h->sel_score, &h->sel_key,
+                    &h->blk, &h->mean_d, &h->var_d, &h->ssq, &h->sync_ints, &h->Mmat, &h->Kdd, &h->blk2, &h->cov, &h->covP, &h->cross, &h->partial, &h->mean_partial, &h->ka, &h->kb, &h->kqa, &h->kqb, &h->kout, &h->qtab, &h->stage, &h->Linv, &h->Linvfull, &h->panel_inv, &h->panel_sync, &h->zkeep, &h->L2, &h->y, &h->app_x, &h->app_y, &h->sel_mean, &h->sel_var, &h->sel_score, &h->sel_key,
                     &h->sel_state, &h->sel_okey, &h->sel_oidx, &h->sel_max, &h->Wq, &h->wscale, &h->Aq, &h->ascale, &h->slscratch, &h->slsync})
     release(*b);
   discard_spans(h);
@@ -1567,10 +1687,11 @@ int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2, i
   CKR(ensure(h, h->ka, (size_t)M * ldx * 8));
   CKR(ensure(h, h->kqa, (size_t)M * 8));
   CKR(ensure(h, h->kout, (size_t)M * ldo * 8));
+  CKR(ensure_act_tables(h, x2 ? M + Nn : M));
   CKR(begin_call(h));
   CKR(upload_matrix(h, x1, M, D, h->ka.as<double>(), ldx));
   CKR(check_finite_async(h, h->ka.as<double>(), ldx, M, D));
-  row_sqnorm_kernel<<<(unsigned)((M * 32 + 255) / 256), 256, 0, h->stream>>>(h->ka.as<double>(), ldx, (int)M, (int)D, sw2, sb2, h->kqa.as<double>(), h->flags.as<int>() + 1);
+  row_sqnorm_kernel<<<(unsigned)((M * 32 + 255) / 256), 256, 0, h->stream>>>(h->ka.as<double>(), ldx, (int)M, (int)D, sw2, sb2, h->kqa.as<double>(), h->flags.as<int>() + 1, h->q_limit);
   h->st.kernel_launches++;
   const double* bptr = h->ka.as<double>();
   const double* qb = h->kqa.as<double>();
@@ -1579,7 +1700,7 @@ int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const double* x2, i
     CKR(ensure(h, h->kqb, (size_t)Nn * 8));
     CKR(upload_matrix(h, x2, Nn, D, h->kb.as<double>(), ldx));
     CKR(check_finite_async(h, h->kb.as<double>(), ldx, Nn, D));
-    row_sqnorm_kernel<<<(unsigned)((Nn * 32 + 255) / 256), 256, 0, h->stream>>>(h->kb.as<double>(), ldx, (int)Nn, (int)D, sw2, sb2, h->kqb.as<double>(), h->flags.as<int>() + 1);
+    row_sqnorm_kernel<<<(unsigned)((Nn * 32 + 255) / 256), 256, 0, h->stream>>>(h->kb.as<double>(), ldx, (int)Nn, (int)D, sw2, sb2, h->kqb.as<double>(), h->flags.as<int>() + 1, h->q_limit);
     h->st.kernel_launches++;
     bptr = h->kb.as<double>();
     qb = h->kqb.as<double>();
@@ -1948,7 +2069,7 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
       CKR(check_finite_async(h, xt + c0 * ldx, ldx, cr, D));
       double* qt_c = h->qt.as<double>() + c0;
       double* mp_c = h->mean_partial.as<double>() + c0 * 2 * col_tiles;
-      row_sqnorm_kernel<<<(unsigned)((cr * 32 + 255) / 256), 256, 0, h->stream>>>(xt + c0 * ldx, ldx, (int)cr, (int)D, sw2, sb2, qt_c, h->flags.as<int>() + 1);
+      row_sqnorm_kernel<<<(unsigned)((cr * 32 + 255) / 256), 256, 0, h->stream>>>(xt + c0 * ldx, ldx, (int)cr, (int)D, sw2, sb2, qt_c, h->flags.as<int>() + 1, h->q_limit);
       h->st.kernel_launches++;
       CKR(run_gram(h, xt + c0 * ldx, ldx, cr, qt_c, h->X.as<double>(), ldx, N, h->q.as<double>(), D, blk + c0 * ldl, ldl, 0,
                    (ntk && want_var) ? h->blk2.as<double>() + c0 * ldl : nullptr, h->alpha.as<double>(), mp_c));
@@ -1961,9 +2082,7 @@ static int predict_impl(nngp_handle* h, const double* x_test, int64_t T, double*
     CK(cudaEventRecord(ev_xt_free, h->stream));   // the next block's upload may overlap this block's solve
 
     if (want_var) {
-      LayerSig sig;
-      for (int i = 0; i < 16; ++i) { sig.sw2[i] = h->lsw2[std::min(i + 1, NNGP_MAX_LAYERS - 1)]; sig.sb2[i] = h->lsb2[std::min(i + 1, NNGP_MAX_LAYERS - 1)]; }
-      q_final_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, h->stream>>>(h->qt.as<double>(), (int)rows, h->cfg.depth - 1, sig, h->kss.as<double>());
+      q_final_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, h->stream>>>(h->qt.as<double>(), (int)rows, h->cfg.depth - 1, layer_sig(h), h->act, nullptr, h->kss.as<double>());
       h->st.kernel_launches++;
       bool solved = false;
       CKR(block_variance(h, T, rows, h->var_d.as<double>() + t0, &solved));

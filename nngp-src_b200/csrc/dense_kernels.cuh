@@ -1,5 +1,5 @@
 // dense_kernels.cuh -- the small kernels around the DMMA GEMM core:
-//   row_sqnorm / q_final          layer-0 kernel diagonal and K(x,x)            (K2, K9)
+//   row_sqnorm                    layer-0 kernel diagonal (K2; K(x,x) is q_final_kernel in gemm_nt.cuh, K9)
 //   diag_reg                      lambda = diag_reg * trace(K)/N ; K += lambda I (K4)
 //   potf2_64_block                64x64 diagonal-block Cholesky, 4 x 4 register blocks            (K5 panel)
 //   trtri_diag                    inv(L_JJ) of every diagonal block: operand of the solves' diagonal step (K10)
@@ -25,10 +25,14 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // q[r] = sw2 * sum_j x[r][j]^2 / D + sb2 ; one warp per row.
-// range_flag (optional): |= 2 when some q >= 2^512 (or overflows): the Gram epilogue forms q q', which must stay finite.
+// range_flag (optional): |= 2 when some q >= q_limit (or overflows): the Gram epilogue forms q q', which must stay
+// finite (Q_LIMIT); Erf(a, b, c) also forms b^2 q (P of erf_step), held below ERF_Q_LIMIT: q_limit = min(Q_LIMIT,
+// ERF_Q_LIMIT / b^2).
 constexpr double Q_LIMIT = 0x1p+512;
+constexpr double ERF_Q_LIMIT = 0x1p+508;
 __global__ void row_sqnorm_kernel(const double* __restrict__ x, long long ldx, int rows, int D, double sw2,
-                                  double sb2, double* __restrict__ q, int* __restrict__ range_flag = nullptr) {
+                                  double sb2, double* __restrict__ q, int* __restrict__ range_flag = nullptr,
+                                  double q_limit = Q_LIMIT) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp >= rows) return;
@@ -42,24 +46,14 @@ __global__ void row_sqnorm_kernel(const double* __restrict__ x, long long ldx, i
   if (lane == 0) {
     const double v = sw2 * (s / (double)D) + sb2;
     q[warp] = v;
-    if (range_flag && !(v < Q_LIMIT)) atomicOr(range_flag, 2);
+    if (range_flag && !(v < q_limit)) atomicOr(range_flag, 2);
   }
 }
 
-// kss[r] = layer-(depth-1) diagonal: q <- sw2_s*q/2 + sb2_s for the Dense layer that follows arc-cosine step s.
+// sigma_w^2 / sigma_b^2 of the Dense layer that follows activation step s (q_final_kernel, gemm_nt.cuh)
 struct LayerSig {
   double sw2[16], sb2[16];   // entry min(s, 15)
 };
-__global__ void q_final_kernel(const double* __restrict__ q, int rows, int steps, LayerSig sig, double* __restrict__ kss) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= rows) return;
-  double v = q[i];
-  for (int s = 0; s < steps; ++s) {
-    const int li = s < 16 ? s : 15;
-    v = sig.sw2[li] * (0.5 * v) + sig.sb2[li];
-  }
-  kss[i] = v;
-}
 
 // Single CTA: lambda = reg * (absolute ? 1 : trace(K)/N); K[i][i] += lambda.  lambda -> *lambda_out.
 __global__ void diag_reg_kernel(double* __restrict__ K, long long ld, int N, double reg, int absolute,

@@ -21,6 +21,7 @@
 // permutation of the k index shared by A and B, see mma_mainloop) touches, per half-warp, every
 // bank exactly once => 2 wavefronts for 256 B: conflict-free.
 #pragma once
+#include "dense_kernels.cuh"
 #include "ptx.cuh"
 
 namespace nngp {
@@ -40,6 +41,17 @@ constexpr int GEMM_SMEM_BYTES =
     GEMM_STAGES * (GEMM_A_STAGE_BYTES + GEMM_B_STAGE_BYTES) + 2 * GEMM_STAGES * 8 + 1024;
 
 enum GemmEpilogue : int { EPI_GRAM = 0, EPI_SUB = 1, EPI_ROWDOT = 2, EPI_DIAG = 3 };
+
+// Activation of every hidden step (== NNGP_ACT_*, include/nngp_b200.h), and the coefficients its steps use, derived
+// once from (a, b, c) on the host (make_act_coef in capi.cu).
+enum GramAct : int { ACT_RELU = 0, ACT_ABRELU = 1, ACT_ERF = 2 };
+struct ActCoef {
+  int kind;
+  double c0, c1;   // ReLU / ABRelu: (a^2 + b^2) / 2 and (a - b)^2 / (2 pi)   (ReLU: 1/2 and 1/(2 pi))
+  double b2x2;     // Erf: 2 b^2
+  double e, c2;    // Erf: a^2 (2/pi) and c^2
+  double kd;       // Erf: a^2 b^2 (4/pi)
+};
 
 struct GemmParams {
   int M, N;            // valid output extent (rows of the A range, rows of the B range)
@@ -76,6 +88,12 @@ struct GemmParams {
   const double* kss;   // [M] K(x,x)
   double* var;         // [M] or nullptr (plain solve)
   int J, col_blocks;   // which 64-column block this launch solves, of how many
+  // EPI_GRAM: the activation's coefficients (gemm_nt_kernel<EPI_GRAM, ACT>).  Erf reads the diagonals entering steps
+  // 1..steps-1 from per-row tables (q_final_kernel): tab1[(s - 1) * tld1 + r] for the A rows, tab2 alike for B.
+  ActCoef act;
+  const double* tab1;
+  const double* tab2;
+  long long tld1, tld2;
 };
 
 // Epilogue of the diagonal step of  V = K_* L^-T  (shared by trsm_fused_kernel and gemm_nt_kernel<EPI_DIAG>, which
@@ -237,6 +255,91 @@ __device__ __forceinline__ void arccos_step_ntk(double& k, double& ntk, double q
   ntk = k + sw2 * (ntk * dot_sigma);
 }
 
+// ABRelu(a, b), phi(x) = a min(x, 0) + b max(x, 0) [nt 0.6.1 stax.ABRelu]: the arc-cosine step with two coefficients,
+//   kdot = c0 - c1 theta,  E[phi(u) phi(v)] = c1 s + kdot k,  E[phi(u)^2] = c0 q;  c0 = (a^2+b^2)/2, c1 = (a-b)^2/(2 pi)
+// (ReLU is c0 = 1/2, c1 = 1/(2 pi): arccos_step).  Same theta, same range argument as ReLU.  Returns kdot.
+template <bool GUARD>
+__device__ __forceinline__ double abrelu_step(double& k, double q1, double q2, double sw2, double sb2, double c0, double c1) {
+  const double s2 = clamp_nonneg(q1 * q2 - k * k);
+  const double s = sqrt(s2);
+  const double theta = atan2_pos<GUARD>(s, s2, k);
+  const double kdot = c0 - c1 * theta;
+  const double r = c1 * s + kdot * k;
+  k = sw2 * r + sb2;
+  return kdot;
+}
+
+// Erf(a, b, c), phi(x) = a erf(b x) + c [nt 0.6.1 stax.Erf].  With Q = b^2 q, K = b^2 k and
+//   P = (1 + 2 Q1)(1 + 2 Q2) - 4 K^2 = 1 + 2 (Q1 + Q2) + 4 b^4 s^2        (the second form cancels nothing)
+//   E[phi(u) phi(v)] = a^2 (2/pi) arcsin(2K / sqrt((1 + 2 Q1)(1 + 2 Q2))) + c^2 = a^2 (2/pi) atan2(2K, sqrt P) + c^2
+//   kdot = E[phi'(u) phi'(v)] = a^2 b^2 (4/pi) / sqrt P
+// sqrt P >= 1, so nothing divides by a small number, and atan2_pos takes atan(|2K| / sqrt P) itself wherever
+// |2K| < sqrt P (its t = min / max): a small kernel value keeps its relative accuracy against a small diagonal.  The
+// accepted input range, b^2 q < 2^508 on every layer (row_sqnorm_kernel's limit and make_act_coef), keeps P below
+// 2^1019 and 4 K^2 below 2^1018, so atan2_pos needs no range guard: there is no guarded Erf path.
+__device__ __forceinline__ double erf_expect(double k2, double sp, const ActCoef& a) {   // k2 = 2K, sp = sqrt P
+  const double th = atan2_pos<false>(fabs(k2), k2 * k2, sp);
+  return fma(a.e, copysign(th, k2), a.c2);
+}
+
+// E[phi(u)^2] of Erf at variance q: the step above at k = q1 = q2 = q (s = 0), P = 1 + 4Q
+__device__ __forceinline__ double erf_diag(double q, const ActCoef& a) {
+  return erf_expect(a.b2x2 * q, sqrt(fma(a.b2x2, q + q, 1.0)), a);
+}
+
+template <bool NTK>
+__device__ __forceinline__ void erf_step(double& k, double& ntk, double q1, double q2, double sw2, double sb2,
+                                         const ActCoef& a) {
+  const double s2 = clamp_nonneg(q1 * q2 - k * k);
+  const double bs = a.b2x2 * sqrt(s2);                               // 2 b^2 s
+  const double sp = sqrt(fma(bs, bs, fma(a.b2x2, q1 + q2, 1.0)));    // sqrt P
+  const double kn = sw2 * erf_expect(a.b2x2 * k, sp, a) + sb2;
+  if (NTK) ntk = kn + sw2 * (ntk * (a.kd * rcp_newton(sp)));
+  k = kn;
+}
+
+// One hidden step of activation ACT on an entry (and its NTK when NTK), followed by the next Dense layer
+template <int ACT, bool GUARD, bool NTK>
+__device__ __forceinline__ void gram_step(double& k, double& ntk, double q1, double q2, double sw2, double sb2,
+                                          const ActCoef& a) {
+  if constexpr (ACT == ACT_ERF) {
+    erf_step<NTK>(k, ntk, q1, q2, sw2, sb2, a);
+  } else if constexpr (ACT == ACT_ABRELU) {
+    const double kdot = abrelu_step<GUARD>(k, q1, q2, sw2, sb2, a.c0, a.c1);
+    if (NTK) ntk = k + sw2 * (ntk * kdot);
+  } else if constexpr (NTK) {
+    arccos_step_ntk<GUARD>(k, ntk, q1, q2, sw2, sb2);
+  } else {
+    k = arccos_step<GUARD>(k, q1, q2, sw2, sb2);
+  }
+}
+
+// The diagonal of the Dense layer that follows a step: q' = sw2 E[phi(u)^2] + sb2
+template <int ACT>
+__device__ __forceinline__ double next_diag(double q, const ActCoef& a, double sw2, double sb2) {
+  if constexpr (ACT == ACT_ERF) return sw2 * erf_diag(q, a) + sb2;
+  else if constexpr (ACT == ACT_ABRELU) return sw2 * (a.c0 * q) + sb2;
+  else return sw2 * (0.5 * q) + sb2;
+}
+
+// Per row: the diagonals of the Dense layers after each of the `steps` activation steps.  tab (optional) receives those
+// entering steps 1..steps-1, tab[(s - 1) * rows + r] (what the Erf Gram epilogue reads instead of evaluating E[phi^2]
+// per entry), kss (optional) the one after the last step, K(x,x).
+__global__ void q_final_kernel(const double* __restrict__ q, int rows, int steps, LayerSig sig, ActCoef act,
+                               double* __restrict__ tab, double* __restrict__ kss) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= rows) return;
+  double v = q[i];
+  for (int s = 0; s < steps; ++s) {
+    const int li = s < 16 ? s : 15;
+    if (tab != nullptr && s > 0) tab[(long long)(s - 1) * rows + i] = v;
+    // (ReLU: c0 = 1/2 exactly -- the same bits as next_diag<ACT_RELU>)
+    v = act.kind == ACT_ERF ? next_diag<ACT_ERF>(v, act, sig.sw2[li], sig.sb2[li])
+                            : next_diag<ACT_ABRELU>(v, act, sig.sw2[li], sig.sb2[li]);
+  }
+  if (kss != nullptr) kss[i] = v;
+}
+
 // Operand ring, producer and consumer in one loop.  Every warp: wait for a stage, run its 4 x (4 x 4) DMMAs on
 // the warp's 32 x 32 tile, release the stage.  Thread 0 additionally re-arms the stage it has just finished with
 // k-tile kt + STAGES once all 8 warps have released it.  `stage` / `phase` persist across calls (persistent kernels).
@@ -384,6 +487,27 @@ __device__ __forceinline__ bool q_in_range(double q1, const double (&q2)[W]) {
 #ifndef NNGP_GRAM_ILP
 #define NNGP_GRAM_ILP 4   // entries advanced through the layers together (2, 4 or 8): independent dependency chains
 #endif                    // (sqrt, reciprocal, two Horner halves each) for the scheduler to interleave; 8 spills
+// The diagonals entering step s + 1 (not needed after the last step): ReLU / ABRelu advance them in registers, Erf
+// loads them from the per-row tables (an arcsine per entry and step would double the epilogue's transcendental work).
+template <int ACT, int W>
+__device__ __forceinline__ void advance_diags(double& qa, double (&qb)[W], const GemmParams& p, int s, int r,
+                                              int col_base, int n0, double sw2, double sb2) {
+  if constexpr (ACT == ACT_ERF) {
+    qa = __ldg(p.tab1 + s * p.tld1 + r);
+#pragma unroll
+    for (int j = 0; j < W / 2; ++j) {
+      const int c = col_base + 8 * (n0 + j);
+      qb[2 * j] = (c < p.N) ? __ldg(p.tab2 + s * p.tld2 + c) : 0.0;
+      qb[2 * j + 1] = (c + 1 < p.N) ? __ldg(p.tab2 + s * p.tld2 + c + 1) : 0.0;
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < W; ++j) qb[j] = next_diag<ACT>(qb[j], p.act, sw2, sb2);
+    qa = next_diag<ACT>(qa, p.act, sw2, sb2);
+  }
+}
+
+template <int ACT>
 __device__ __forceinline__ void gram_epilogue(const double (&acc)[4][4][2], const GemmParams& p, int tile_n, int row_base,
                                               int col_base, int wn, int t) {
   constexpr int W = NNGP_GRAM_ILP;          // entries per group
@@ -406,22 +530,20 @@ __device__ __forceinline__ void gram_epilogue(const double (&acc)[4][4][2], cons
           qb[2 * j + 1] = (c + 1 < p.N) ? __ldg(p.q2 + c + 1) : 0.0;
         }
         double qa = q1r;
+        // (Erf has no guarded variant: its input range keeps every step inside atan2_pos' unguarded domain)
         if (!p.ntk) {
+          double unused = 0.0;
           for (int s = 0; s < p.steps; ++s) {
             const int li = s < GEMM_MAX_LAYERS ? s : GEMM_MAX_LAYERS - 1;
             const double sw2 = p.lsw2[li], sb2 = p.lsb2[li];
-            if (q_in_range<W>(qa, qb)) {
+            if (ACT == ACT_ERF || q_in_range<W>(qa, qb)) {
 #pragma unroll
-              for (int j = 0; j < W; ++j) k[j] = arccos_step<false>(k[j], qa, qb[j], sw2, sb2);
+              for (int j = 0; j < W; ++j) gram_step<ACT, false, false>(k[j], unused, qa, qb[j], sw2, sb2, p.act);
             } else {
 #pragma unroll
-              for (int j = 0; j < W; ++j) k[j] = arccos_step<true>(k[j], qa, qb[j], sw2, sb2);
+              for (int j = 0; j < W; ++j) gram_step<ACT, true, false>(k[j], unused, qa, qb[j], sw2, sb2, p.act);
             }
-            if (s + 1 < p.steps) {              // the diagonals of the next layer (not needed after the last one)
-#pragma unroll
-              for (int j = 0; j < W; ++j) qb[j] = sw2 * (0.5 * qb[j]) + sb2;
-              qa = sw2 * (0.5 * qa) + sb2;
-            }
+            if (s + 1 < p.steps) advance_diags<ACT, W>(qa, qb, p, s, r, col_base, n0, sw2, sb2);
           }
         } else {
           double n[W];
@@ -430,18 +552,14 @@ __device__ __forceinline__ void gram_epilogue(const double (&acc)[4][4][2], cons
           for (int s = 0; s < p.steps; ++s) {
             const int li = s < GEMM_MAX_LAYERS ? s : GEMM_MAX_LAYERS - 1;
             const double sw2 = p.lsw2[li], sb2 = p.lsb2[li];
-            if (q_in_range<W>(qa, qb)) {
+            if (ACT == ACT_ERF || q_in_range<W>(qa, qb)) {
 #pragma unroll
-              for (int j = 0; j < W; ++j) arccos_step_ntk<false>(k[j], n[j], qa, qb[j], sw2, sb2);
+              for (int j = 0; j < W; ++j) gram_step<ACT, false, true>(k[j], n[j], qa, qb[j], sw2, sb2, p.act);
             } else {
 #pragma unroll
-              for (int j = 0; j < W; ++j) arccos_step_ntk<true>(k[j], n[j], qa, qb[j], sw2, sb2);
+              for (int j = 0; j < W; ++j) gram_step<ACT, true, true>(k[j], n[j], qa, qb[j], sw2, sb2, p.act);
             }
-            if (s + 1 < p.steps) {
-#pragma unroll
-              for (int j = 0; j < W; ++j) qb[j] = sw2 * (0.5 * qb[j]) + sb2;
-              qa = sw2 * (0.5 * qa) + sb2;
-            }
+            if (s + 1 < p.steps) advance_diags<ACT, W>(qa, qb, p, s, r, col_base, n0, sw2, sb2);
           }
           if (p.C2) {
 #pragma unroll
@@ -486,7 +604,8 @@ __device__ __forceinline__ void gram_epilogue(const double (&acc)[4][4][2], cons
 #ifndef NNGP_GEMM_MINBLOCKS
 #define NNGP_GEMM_MINBLOCKS 2
 #endif
-template <int EPI>
+// ACT: the activation of the EPI_GRAM epilogue (GramAct); the other epilogues only exist with the default.
+template <int EPI, int ACT = ACT_RELU>
 __global__ void __launch_bounds__(GEMM_THREADS, NNGP_GEMM_MINBLOCKS)
 gemm_nt_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const GemmParams p) {
@@ -669,7 +788,7 @@ gemm_nt_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       if (r < p.M) p.partial[(long long)tile_n * p.M + r] = red[threadIdx.x] + red[GEMM_BM + threadIdx.x];
     }
   } else {
-    gram_epilogue(acc, p, tile_n, row_base_e, col_base_e, wn, t);
+    gram_epilogue<ACT>(acc, p, tile_n, row_base_e, col_base_e, wn, t);
   }
 }
 

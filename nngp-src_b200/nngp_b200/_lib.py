@@ -8,6 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+from dataclasses import dataclass
 from pathlib import Path
 
 import numpy as np
@@ -40,6 +41,31 @@ class NngpConfig(C.Structure):
         ("variance_slices", C.c_int32),
         ("reserved0", C.c_int32),
     ]
+
+
+class NngpActivation(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("reserved", C.c_int32), ("a", C.c_double), ("b", C.c_double), ("c", C.c_double)]
+
+
+ACT_KINDS = {"relu": 0, "abrelu": 1, "erf": 2}     # NNGP_ACT_*
+
+
+@dataclass(frozen=True)
+class Activation:
+    """The activation of every hidden step (``nngp_activation``): 'relu', 'abrelu' -- a min(x, 0) + b max(x, 0) -- or
+    'erf' -- a erf(b x) + c.  Built by ``stax.Relu`` / ``LeakyRelu`` / ``Abs`` / ``ABRelu`` / ``Erf``."""
+    kind: str = "relu"
+    a: float = 0.0
+    b: float = 1.0
+    c: float = 0.0
+
+    def as_struct(self) -> NngpActivation:
+        if self.kind not in ACT_KINDS:
+            raise ValueError(f"nngp_b200: unknown activation {self.kind!r} ({sorted(ACT_KINDS)})")
+        return NngpActivation(ACT_KINDS[self.kind], 0, float(self.a), float(self.b), float(self.c))
+
+
+RELU = Activation()
 
 
 class NngpStats(C.Structure):
@@ -75,6 +101,7 @@ EXPORTS = {
     "nngp_state_import_end": (C.c_int, [_P, C.c_double]),
     "nngp_default_config": (None, [C.POINTER(NngpConfig)]),
     "nngp_create": (C.c_int, [C.POINTER(NngpConfig), C.POINTER(_P)]),
+    "nngp_create_with_activation": (C.c_int, [C.POINTER(NngpConfig), C.POINTER(NngpActivation), C.POINTER(_P)]),
     "nngp_destroy": (None, [_P]),
     "nngp_last_error": (C.c_char_p, [_P]),
     "nngp_get_stream": (_P, [_P]),
@@ -205,11 +232,14 @@ def _npz_path(path):
 
 
 class Handle:
-    """RAII wrapper of ``nngp_handle*`` (one GPU, not re-entrant)."""
+    """RAII wrapper of ``nngp_handle*`` (one GPU, not re-entrant).  ``activation``: an ``Activation`` for every hidden
+    step (None: ReLU, ``nngp_create``)."""
 
     def __init__(self, depth=2, sigma_w=1.0, sigma_b=0.0, diag_reg=1e-3, diag_reg_absolute=False,
                  device=-1, max_block_bytes=0, stats_level=1, kernel_type="nngp", n_gpus=1, device_ids=None,
-                 latency_mode=False, variance_slices=0):
+                 latency_mode=False, variance_slices=0, activation=None):
+        self.activation = RELU if activation is None else activation
+        act = self.activation.as_struct()
         self._lib = load()
         cfg = NngpConfig()
         self._lib.nngp_default_config(C.byref(cfg))
@@ -244,7 +274,7 @@ class Handle:
         cfg.variance_slices = int(variance_slices)
         self.cfg = cfg
         h = C.c_void_p()
-        rc = self._lib.nngp_create(C.byref(cfg), C.byref(h))
+        rc = self._lib.nngp_create_with_activation(C.byref(cfg), C.byref(act), C.byref(h))
         if rc != NNGP_OK:
             _raise(self._lib, None, rc)
         self._h = h
@@ -455,14 +485,21 @@ class Handle:
             sw, sb = self.cfg.sigma_w, self.cfg.sigma_b
         np.savez(_npz_path(path), x=st["x"], l=st["l"], alpha=st["alpha"], lam=st["lambda"], depth=self.cfg.depth,
                  sigma_w=sw, sigma_b=sb, diag_reg=self.cfg.diag_reg,
-                 diag_reg_absolute=self.cfg.diag_reg_absolute, kernel_type="ntk" if self.is_ntk else "nngp", **extra)
+                 diag_reg_absolute=self.cfg.diag_reg_absolute, kernel_type="ntk" if self.is_ntk else "nngp",
+                 act_kind=self.activation.kind, act_abc=np.array([self.activation.a, self.activation.b, self.activation.c]),
+                 **extra)
 
     @classmethod
     def load(cls, path, **kw) -> "Handle":
         z = np.load(_npz_path(path))
         kt = str(z["kernel_type"]) if "kernel_type" in z.files else "nngp"
+        act = RELU                                    # (files written before activations existed are ReLU models)
+        if "act_kind" in z.files:
+            a, b, c = (float(v) for v in z["act_abc"])
+            act = Activation(str(z["act_kind"]), a, b, c)
         h = cls(depth=int(z["depth"]), sigma_w=z["sigma_w"], sigma_b=z["sigma_b"],
-                diag_reg=float(z["diag_reg"]), diag_reg_absolute=bool(z["diag_reg_absolute"]), kernel_type=kt, **kw)
+                diag_reg=float(z["diag_reg"]), diag_reg_absolute=bool(z["diag_reg_absolute"]), kernel_type=kt,
+                activation=act, **kw)
         h.set_state(z["x"], z["l"], z["alpha"], float(z["lam"]), m=z["m"] if kt == "ntk" else None)
         return h
 

@@ -63,7 +63,8 @@ def new_handle(spec, diag_reg=0.0, diag_reg_absolute=False, kernel_type="nngp") 
     return _lib.Handle(depth=spec.depth, sigma_w=spec.sigma_w, sigma_b=spec.sigma_b, diag_reg=diag_reg,
                        diag_reg_absolute=diag_reg_absolute, device=_device, max_block_bytes=_max_block_bytes,
                        stats_level=_stats_level, kernel_type=kernel_type, n_gpus=_n_gpus, device_ids=_device_ids,
-                       latency_mode=_latency_mode, variance_slices=_variance_slices if kernel_type == "nngp" else 0)
+                       latency_mode=_latency_mode, variance_slices=_variance_slices if kernel_type == "nngp" else 0,
+                       activation=spec.activation)
 
 
 def as_matrix(x, name="x"):

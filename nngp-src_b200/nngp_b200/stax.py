@@ -4,9 +4,10 @@ Reference call sites: ``stax.serial(stax.Dense(512), stax.Relu(), stax.Dense(1))
 neuroestimator/estimator/estimator.py:27-30, active/active_train.py:40-43 (and the commented
 ``W_std=1.5, b_std=0.05`` variant at active/active_train.py:44-49).
 
-Only what defines the infinite-width NNGP kernel is kept: a chain Dense (Relu Dense)* collapses to a
-``KernelSpec(depth, W_std, b_std)`` and ``kernel_fn`` evaluates it with the sm_100a Gram+arc-cosine
-kernel through the C ABI.  ``init_fn`` / ``apply_fn`` (finite-width networks) and every other layer type
+Only what defines the infinite-width NNGP kernel is kept: a chain Dense (Act Dense)* with one activation
+throughout (Relu, LeakyRelu, Abs, ABRelu or Erf) collapses to a ``KernelSpec(depth, W_std, b_std, activation)``
+and ``kernel_fn`` evaluates it with the sm_100a Gram kernel (the activation's steps in its epilogue) through the
+C ABI.  ``init_fn`` / ``apply_fn`` (finite-width networks) and every other layer type
 raise ``NotImplementedError`` -- never a silent CPU fallback.
 """
 from __future__ import annotations
@@ -20,9 +21,10 @@ from . import _lib, runtime
 
 @dataclass(frozen=True)
 class KernelSpec:
-    depth: int           # number of Dense layers; depth-1 ReLU arc-cosine steps
+    depth: int           # number of Dense layers; depth-1 activation steps
     sigma_w: object      # W_std: a float when every Dense layer has the same, else a tuple with one value per layer
     sigma_b: object      # b_std (None -> 0): likewise
+    activation: _lib.Activation = _lib.RELU   # of every step
 
 
 class _Layer(tuple):
@@ -45,19 +47,43 @@ def Dense(out_dim, W_std=1.0, b_std=None, batch_axis=0, channel_axis=-1, paramet
     return _Layer("dense", out_dim=int(out_dim), W_std=float(W_std), b_std=0.0 if b_std is None else float(b_std))
 
 
+def _act_layer(act):
+    return _Layer("act", activation=act)
+
+
 def Relu(do_backprop=False, do_stabilize=False):
-    return _Layer("relu")
+    return _act_layer(_lib.RELU)
+
+
+def ABRelu(a, b, do_stabilize=False):
+    """a min(x, 0) + b max(x, 0)   [nt 0.6.1 stax.ABRelu]"""
+    return _act_layer(_lib.Activation("abrelu", float(a), float(b)))
+
+
+def LeakyRelu(alpha, do_stabilize=False):
+    """ABRelu(alpha, 1)   [nt 0.6.1 stax.LeakyRelu]"""
+    return ABRelu(alpha, 1.0)
+
+
+def Abs(do_stabilize=False):
+    """ABRelu(-1, 1)   [nt 0.6.1 stax.Abs]"""
+    return ABRelu(-1.0, 1.0)
+
+
+def Erf(a=1., b=1., c=0.):
+    """a erf(b x) + c   [nt 0.6.1 stax.Erf]"""
+    return _act_layer(_lib.Activation("erf", float(a), float(b), float(c)))
 
 
 def _unsupported(name):
     def ctor(*_a, **_k):
-        raise NotImplementedError(f"nngp_b200.stax.{name} is not on the reference's NNGP path "
-                                  "(only Dense/Relu/serial are used: train.py:161-164)")
+        raise NotImplementedError(f"nngp_b200.stax.{name} is not implemented (the kernels exist for Dense and the "
+                                  "Relu / LeakyRelu / Abs / ABRelu / Erf activations)")
     ctor.__name__ = name
     return ctor
 
 
-for _n in ("Conv", "Erf", "Gelu", "ABRelu", "LeakyRelu", "Abs", "Flatten", "AvgPool", "GlobalAvgPool", "FanOut",
+for _n in ("Conv", "Gelu", "Flatten", "AvgPool", "GlobalAvgPool", "FanOut",
            "FanInSum", "LayerNorm", "Dropout", "Identity", "parallel"):
     globals()[_n] = _unsupported(_n)
 
@@ -90,21 +116,25 @@ class KernelFn:
 
 
 def serial(*layers):
-    """Collapse Dense (Relu Dense)* into one KernelSpec; returns (init_fn, apply_fn, kernel_fn)."""
+    """Collapse Dense (Act Dense)* into one KernelSpec; returns (init_fn, apply_fn, kernel_fn)."""
     if not layers or any(not isinstance(l, _Layer) for l in layers):
-        raise NotImplementedError("nngp_b200.stax.serial: expects layers built by nngp_b200.stax.Dense / Relu")
+        raise NotImplementedError("nngp_b200.stax.serial: expects layers built by nngp_b200.stax.Dense / an activation")
     kinds = [l.kind for l in layers]
     if kinds[0] != "dense" or kinds[-1] != "dense" or any(
             kinds[i] == kinds[i + 1] for i in range(len(kinds) - 1)):
-        raise NotImplementedError(f"nngp_b200.stax.serial: only Dense (Relu Dense)* chains are supported, got {kinds}")
+        raise NotImplementedError(f"nngp_b200.stax.serial: only Dense (Act Dense)* chains are supported, got {kinds}")
+    acts = {l.params["activation"] for l in layers if l.kind == "act"}
+    if len(acts) > 1:
+        raise NotImplementedError(f"nngp_b200.stax.serial: one activation for every hidden layer, got {sorted(map(str, acts))}")
+    act = acts.pop() if acts else _lib.RELU
     dense = [l for l in layers if l.kind == "dense"]
     w = tuple(l.params["W_std"] for l in dense)
     b = tuple(l.params["b_std"] for l in dense)
     if len(set(w)) == 1 and len(set(b)) == 1:
-        spec = KernelSpec(depth=len(dense), sigma_w=w[0], sigma_b=b[0])
+        spec = KernelSpec(depth=len(dense), sigma_w=w[0], sigma_b=b[0], activation=act)
     else:                                   # layers differ [nt allows it]: per-layer values (nngp_config.per_layer)
         if len(dense) > 16:
             raise NotImplementedError("nngp_b200.stax.serial: per-layer W_std / b_std support at most 16 Dense layers")
-        spec = KernelSpec(depth=len(dense), sigma_w=w, sigma_b=b)
+        spec = KernelSpec(depth=len(dense), sigma_w=w, sigma_b=b, activation=act)
     init_fn, apply_fn, _ = dense[0]
     return init_fn, apply_fn, KernelFn(spec)
