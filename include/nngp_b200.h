@@ -96,7 +96,10 @@ typedef struct nngp_config {
                                  (tcgen05.mma kind::i8, accumulators in TMEM): both operands are split row-wise into s
                                  signed 7-bit digit planes, the s(s+1)/2 - 1 exact int32 plane products with p + q < s (all but
                                  the weakest, plane s-1 of K_* times plane 0 of L^-1) are recombined in FP64.  s = 7 keeps the posterior variance within ~1e-8 relative of the
-                                 FP64 path at cond(K + lambda I) = 1e7 (s = 8: 1e-10); the mean is untouched.  N <= 2^19 / s. */
+                                 FP64 path at cond(K + lambda I) = 1e7 (s = 8: 1e-10); the mean is untouched.  N <= 2^19 / s.
+                                 Every row scale is carried as an integer exponent, so rows of any finite magnitude,
+                                 down to the smallest subnormal, are split exactly; an entry of the product that falls
+                                 below 2^-1022 is rounded once into the subnormal range. */
   int32_t reserved0;
 } nngp_config;
 
@@ -201,6 +204,9 @@ NNGP_API int nngp_kernel(nngp_handle* h, const double* x1, int64_t M, const doub
  *   active/ActiveLearner.py:27-28  [nt: predict.gp_inference/_get_cho_solve/
  *   _add_diagonal_regularizer -> scipy cho_factor/cho_solve]
  * x_train: N x D, y_train: N (used raw, never centred).
+ * alpha must come out finite: when (K + lambda I)^-1 y overflows the double range (a lambda near the bottom of the
+ * normal range against O(1) labels) the fit is NNGP_EINVAL with a message instead of a model whose means are inf or
+ * NaN; nngp_append_fit checks its alpha the same way.
  */
 NNGP_API int nngp_fit(nngp_handle* h, const double* x_train, const double* y_train, int64_t N, int64_t D);
 
@@ -304,6 +310,8 @@ NNGP_API int nngp_num_gpus(const nngp_handle* h);
  * `lower` != 0 treats B as lower triangular (entries with k > row ignored, N == K); `lower` == 2 also drops the plane
  * pair (slices-1, 0), exactly as the variance path does for B = L^-1 (whose rows are dominated by their diagonal entry).  v_out [M, N] receives the product,
  * rowsq_out [M] (optional) the row sums of V^2 in the order the variance uses.  Independent of any fitted model.
+ * Any finite rows are accepted: each row of A and B is scaled by its own power of two (down to rows whose largest
+ * magnitude is the smallest subnormal), and each entry is the folded plane sum times 2^(ea + eb - 12), rounded once.
  * [no reference counterpart: the reference's only matrix product is XLA's dot, train.py:157-158]              */
 NNGP_API int nngp_sliced_product(nngp_handle* h, const double* a, int64_t M, int64_t K, const double* b, int64_t N,
                                  int32_t lower, int32_t slices, double* v_out, double* rowsq_out);

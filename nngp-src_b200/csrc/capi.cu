@@ -93,8 +93,8 @@ struct nngp_handle {
   DevBuf Linvfull;  // latency mode: the explicit inverse factor L^-1 (N x N, lower, row-major, ld = ldl)
   bool have_inv = false;
   // cfg.variance_slices: int8 digit planes of L^-1 ([s][wq_rb][wq_ldq]) + 2^(e-6) of its rows; planes of the current
-  // K_* row block, their row scales, and the per-CTA running-sum tiles of sliced_gemm_kernel
-  DevBuf Wq, wscale, Aq, ascale, slscratch, slsync;
+  // K_* row block, their row exponents, and the per-CTA running-sum tiles of sliced_gemm_kernel
+  DevBuf Wq, wexp, Aq, aexp, slscratch, slsync;
   bool have_wq = false;
   int64_t wq_ldq = 0, wq_rb = 0;
   DevBuf L2;      // second factor buffer: target of the incremental (fixed-lambda) append, then swapped with L
@@ -438,13 +438,13 @@ size_t partial_bytes(const nngp_handle* h, int64_t N, int64_t rows) {
   return (size_t)n * sizeof(double);
 }
 
-// run_sliced_variance over `rows` rows: K_* digit planes and row scales of a sub-block, partials, launch workspace
+// run_sliced_variance over `rows` rows: K_* digit planes and row exponents of a sub-block, partials, launch workspace
 int ensure_sliced_block(nngp_handle* h, int64_t N, int64_t rows) {
   const int64_t sb = sliced_rows(h, N, rows);
   int grid;
   int64_t rounds;
   CKR(ensure(h, h->Aq, (size_t)h->cfg.variance_slices * sb * round_up(N, SL_BK)));
-  CKR(ensure(h, h->ascale, (size_t)sb * sizeof(double)));
+  CKR(ensure(h, h->aexp, (size_t)sb * sizeof(int)));
   CKR(ensure(h, h->partial, partial_bytes(h, N, rows)));
   return sliced_grid(h, sb, N, &grid, &rounds);
 }
@@ -483,7 +483,7 @@ int ensure_model(nngp_handle* h, int64_t N, int64_t D) {
     return fail(h, NNGP_EINVAL, "variance_slices = %d: int32 plane sums need N <= %lld (N = %lld)", s,
                 (long long)((1LL << 19) / s), (long long)N);
   CKR(ensure(h, h->Wq, (size_t)s * round_up(N, SL_BN) * ldq));
-  return ensure(h, h->wscale, (size_t)N * sizeof(double));
+  return ensure(h, h->wexp, (size_t)N * sizeof(int));
 }
 
 // Only the handle that fits N rows: y, z = L^-1 y, the panel counters of the (N + 1)-row factorisation, K_dd ('ntk')
@@ -890,11 +890,11 @@ int get_tmap_u8(nngp_handle* h, const void* base, uint64_t rows, uint64_t ldq, u
   return NNGP_OK;
 }
 
-// digit planes of `rows` rows of A (columns [0, ncols), or [0, row] when tri) -> planes[s][rpad][ldq], scale[rows]
+// digit planes of `rows` rows of A (columns [0, ncols), or [0, row] when tri) -> planes[s][rpad][ldq], row exponents exps[rows]
 int slice_matrix(nngp_handle* h, const double* A, int64_t lda, int64_t rows, int64_t ncols, int tri, int s, int64_t rpad,
-                 int64_t ldq, int8_t* planes, double* scale) {
+                 int64_t ldq, int8_t* planes, int* exps) {
   slice_rows_kernel<<<(unsigned)rpad, SL_SLICE_THREADS, 0, h->stream>>>(A, lda, (int)rows, (int)ncols, tri, s, planes,
-                                                                       rpad * ldq, (int)ldq, scale);
+                                                                       rpad * ldq, (int)ldq, exps);
   h->st.kernel_launches++;
   CK(cudaGetLastError());
   return NNGP_OK;
@@ -914,14 +914,14 @@ double sliced_macs(int64_t row_tiles, int64_t col_tiles, int64_t K, int tri, int
 
 // V = A W^T from the digit planes: vpart[2 col_tiles][rows] row sums of V^2 per 128-column half tile and/or V itself
 // (ra: rows per K_* plane, a multiple of 256)
-int launch_sliced(nngp_handle* h, const int8_t* qa, int64_t ra, const double* sa, const int8_t* qw, int64_t rb,
-                  const double* sw, int64_t ldq, int s, int tri, int64_t rows, int64_t N, int64_t K, double* vpart, double* V,
+int launch_sliced(nngp_handle* h, const int8_t* qa, int64_t ra, const int* ea, const int8_t* qw, int64_t rb,
+                  const int* ew, int64_t ldq, int s, int tri, int64_t rows, int64_t N, int64_t K, double* vpart, double* V,
                   int64_t ldv, int skip_weak) {
   SlicedParams p{};
   p.s = s; p.rows = (int)rows; p.N = (int)N; p.K = (int)K; p.tri = tri; p.skip_weak = skip_weak;
   p.row_tiles = (int)((rows + SL_BM - 1) / SL_BM);
   p.col_tiles = (int)((N + SL_BN - 1) / SL_BN);
-  p.ra = ra; p.rb = rb; p.rscale = sa; p.cscale = sw; p.vpart = vpart; p.V = V; p.ldv = ldv;
+  p.ra = ra; p.rb = rb; p.rexp = ea; p.cexp = ew; p.vpart = vpart; p.V = V; p.ldv = ldv;
   if ((int64_t)s * ra >= (1LL << 31) || (int64_t)s * rb >= (1LL << 31))
     return fail(h, NNGP_EINVAL, "internal: digit-plane row range too large");
   // Two row tiles per CTA tile (SL_RT): 32 KiB of operands per MMA set instead of 48.  (Single row tiles -- twice as
@@ -970,8 +970,8 @@ int launch_sliced(nngp_handle* h, const int8_t* qa, int64_t ra, const double* sa
 int build_w_planes(nngp_handle* h) {
   const int s = h->cfg.variance_slices;
   const int64_t N = h->N;
-  const int64_t ldq = round_up(N, SL_BK), rb = round_up(N, SL_BN);   // (Wq, wscale: sized by ensure_model)
-  CKR(slice_matrix(h, h->Linvfull.as<double>(), h->ldl, N, N, 1, s, rb, ldq, h->Wq.as<int8_t>(), h->wscale.as<double>()));
+  const int64_t ldq = round_up(N, SL_BK), rb = round_up(N, SL_BN);   // (Wq, wexp: sized by ensure_model)
+  CKR(slice_matrix(h, h->Linvfull.as<double>(), h->ldl, N, N, 1, s, rb, ldq, h->Wq.as<int8_t>(), h->wexp.as<int>()));
   CK(cudaStreamSynchronize(h->stream));
   h->wq_ldq = ldq; h->wq_rb = rb; h->have_wq = true;
   return NNGP_OK;
@@ -988,9 +988,9 @@ int run_sliced_variance(nngp_handle* h, const double* B, int64_t ldb, int64_t ro
   const int span = span_open(h, 0, h->stream, &h->st.sliced_ms);
   for (int64_t r0 = 0; r0 < rows; r0 += sb) {
     const int64_t nr = std::min<int64_t>(sb, rows - r0), ra = round_up(nr, SL_RT * SL_BM);
-    CKR(slice_matrix(h, B + r0 * ldb, ldb, nr, N, 0, s, ra, ldq, h->Aq.as<int8_t>(), h->ascale.as<double>()));
-    CKR(launch_sliced(h, h->Aq.as<int8_t>(), ra, h->ascale.as<double>(), h->Wq.as<int8_t>(), h->wq_rb,
-                      h->wscale.as<double>(), ldq, s, 1, nr, N, N, h->partial.as<double>(), nullptr, 0, 1));
+    CKR(slice_matrix(h, B + r0 * ldb, ldb, nr, N, 0, s, ra, ldq, h->Aq.as<int8_t>(), h->aexp.as<int>()));
+    CKR(launch_sliced(h, h->Aq.as<int8_t>(), ra, h->aexp.as<int>(), h->Wq.as<int8_t>(), h->wq_rb,
+                      h->wexp.as<int>(), ldq, s, 1, nr, N, N, h->partial.as<double>(), nullptr, 0, 1));
     var_from_partial_kernel<<<(unsigned)((nr + 255) / 256), 256, 0, h->stream>>>(kss + r0, h->partial.as<double>(), 2 * col_tiles, (int)nr, var + r0);
     h->st.kernel_launches++;
   }
@@ -1057,11 +1057,13 @@ int download(nngp_handle* h, const double* dsrc, int64_t rows, int64_t cols, int
   return NNGP_OK;
 }
 
-int check_finite_async(nngp_handle* h, const double* x, int64_t ld, int64_t rows, int64_t cols) {
+// flags[1] |= bit when a value of x is not finite: bit 1 for caller input, FLAG_ALPHA for the solved alpha
+constexpr int FLAG_ALPHA = 4;
+int check_finite_async(nngp_handle* h, const double* x, int64_t ld, int64_t rows, int64_t cols, int bit = 1) {
   const int64_t total = rows * cols;
   int grid = (int)std::min<int64_t>((total + 255) / 256, 8 * h->sm_count);
   if (grid < 1) grid = 1;
-  finite_check_kernel<<<grid, 256, 0, h->stream>>>(x, ld, rows, (int)cols, h->flags.as<int>() + 1);
+  finite_check_kernel<<<grid, 256, 0, h->stream>>>(x, ld, rows, (int)cols, h->flags.as<int>() + 1, bit);
   h->st.kernel_launches++;
   return NNGP_OK;
 }
@@ -1088,7 +1090,9 @@ int begin_call(nngp_handle* h) {
 }
 
 // Enqueues the flags read-back (after the caller's own), waits for the main stream and settles the spans.  flags[1]
-// becomes input_error(who, what); flags[0], the potrf pivot + 1 (0: none), goes to *pivot.
+// becomes input_error(who, what); flags[0], the potrf pivot + 1 (0: none), goes to *pivot; FLAG_ALPHA of a factor
+// without a failed pivot means that alpha = (K + lambda I)^-1 y overflowed (lambda near the bottom of the normal
+// range against O(1) labels): an error, not a model whose means are inf or NaN.
 int end_call(nngp_handle* h, const char* who, const char* what, int* pivot = nullptr) {
   int flags[2];
   CK(cudaMemcpyAsync(flags, h->flags.p, sizeof flags, cudaMemcpyDeviceToHost, h->stream));
@@ -1096,7 +1100,11 @@ int end_call(nngp_handle* h, const char* who, const char* what, int* pivot = nul
   CK(cudaGetLastError());
   settle_spans(h);
   if (pivot) *pivot = flags[0];
-  return flags[1] ? input_error(h, flags[1], who, what) : NNGP_OK;
+  if (flags[1] & ~FLAG_ALPHA) return input_error(h, flags[1], who, what);
+  if ((flags[1] & FLAG_ALPHA) && !flags[0])
+    return fail(h, NNGP_EINVAL, "%s: alpha = (K + lambda I)^-1 y overflows the double range (lambda = %.6g): scale y "
+                "down or raise diag_reg", who, h->lambda);
+  return NNGP_OK;
 }
 
 // Rows [new0, rows) of X are new input: check them finite, and derive q of all `rows` rows with the range flag.
@@ -1599,17 +1607,17 @@ int nngp_sliced_product(nngp_handle* h, const double* a, int64_t M, int64_t K, c
   if (rc == NNGP_OK) rc = ensure(h, dB, (size_t)N * K * 8);
   if (rc == NNGP_OK) rc = ensure(h, qa, (size_t)slices * ra * ldq);
   if (rc == NNGP_OK) rc = ensure(h, qb, (size_t)slices * rb * ldq);
-  if (rc == NNGP_OK) rc = ensure(h, sa, (size_t)M * 8);
-  if (rc == NNGP_OK) rc = ensure(h, sb, (size_t)N * 8);
+  if (rc == NNGP_OK) rc = ensure(h, sa, (size_t)M * sizeof(int));
+  if (rc == NNGP_OK) rc = ensure(h, sb, (size_t)N * sizeof(int));
   if (rc == NNGP_OK && v_out) rc = ensure(h, dV, (size_t)M * N * 8);
   if (rc == NNGP_OK) rc = ensure(h, vp, (size_t)2 * col_tiles * M * 8);
   if (rc == NNGP_OK) rc = ensure(h, rs, (size_t)M * 8);
   auto run = [&]() -> int {
     CK(cudaMemcpyAsync(dA.p, a, (size_t)M * K * 8, cudaMemcpyDefault, h->stream));
     CK(cudaMemcpyAsync(dB.p, b, (size_t)N * K * 8, cudaMemcpyDefault, h->stream));
-    CKR(slice_matrix(h, dA.as<double>(), K, M, K, 0, slices, ra, ldq, qa.as<int8_t>(), sa.as<double>()));
-    CKR(slice_matrix(h, dB.as<double>(), K, N, K, lower ? 1 : 0, slices, rb, ldq, qb.as<int8_t>(), sb.as<double>()));
-    CKR(launch_sliced(h, qa.as<int8_t>(), ra, sa.as<double>(), qb.as<int8_t>(), rb, sb.as<double>(), ldq, slices, lower ? 1 : 0,
+    CKR(slice_matrix(h, dA.as<double>(), K, M, K, 0, slices, ra, ldq, qa.as<int8_t>(), sa.as<int>()));
+    CKR(slice_matrix(h, dB.as<double>(), K, N, K, lower ? 1 : 0, slices, rb, ldq, qb.as<int8_t>(), sb.as<int>()));
+    CKR(launch_sliced(h, qa.as<int8_t>(), ra, sa.as<int>(), qb.as<int8_t>(), rb, sb.as<int>(), ldq, slices, lower ? 1 : 0,
                       M, N, K, vp.as<double>(), v_out ? dV.as<double>() : nullptr, N, lower == 2 ? 1 : 0));
     if (v_out) CK(cudaMemcpyAsync(v_out, dV.p, (size_t)M * N * 8, cudaMemcpyDefault, h->stream));
     if (rowsq_out) {
@@ -1640,7 +1648,7 @@ void nngp_destroy(nngp_handle* h) {
   if (h->stream) cudaStreamSynchronize(h->stream);
   for (DevBuf* b : {&h->X, &h->q, &h->L, &h->alpha, &h->flags, &h->lam_d, &h->xt, &h->qt, &h->kss,
                     &h->blk, &h->mean_d, &h->var_d, &h->ssq, &h->sync_ints, &h->Mmat, &h->Kdd, &h->blk2, &h->cov, &h->covP, &h->cross, &h->partial, &h->mean_partial, &h->ka, &h->kb, &h->kqa, &h->kqb, &h->kout, &h->qtab, &h->stage, &h->Linv, &h->Linvfull, &h->panel_inv, &h->panel_sync, &h->zkeep, &h->L2, &h->y, &h->app_x, &h->app_y, &h->sel_mean, &h->sel_var, &h->sel_score, &h->sel_key,
-                    &h->sel_state, &h->sel_okey, &h->sel_oidx, &h->sel_max, &h->Wq, &h->wscale, &h->Aq, &h->ascale, &h->slscratch, &h->slsync})
+                    &h->sel_state, &h->sel_okey, &h->sel_oidx, &h->sel_max, &h->Wq, &h->wexp, &h->Aq, &h->aexp, &h->slscratch, &h->slsync})
     release(*b);
   discard_spans(h);
   for (auto e : h->ev_pool) cudaEventDestroy(e);
@@ -1768,6 +1776,7 @@ static int fit_impl(nngp_handle* h, const double* x_train, const double* y_train
   h->st.kernel_launches++;
   CK(cudaMemcpyAsync(h->zkeep.p, L + N * h->ldl, (size_t)N * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
   CKR(run_trsv_bwd(h, L, h->ldl, N, L + N * h->ldl, alpha, h->Linv.as<double>()));  // alpha = L^-T z
+  CKR(check_finite_async(h, alpha, 1, N, 1, FLAG_ALPHA));
   if (ntk) {  // M = L^-1 K_dd L^-T : two row-wise solves around a transpose (M is symmetric)
     double* Kd = h->Kdd.as<double>();
     double* Mm = h->Mmat.as<double>();
@@ -1944,6 +1953,7 @@ static int append_incremental(nngp_handle* h, int64_t M) {
   h->st.kernel_launches++;
   CK(cudaMemcpyAsync(h->zkeep.p, zrow, (size_t)Nn * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
   CKR(run_trsv_bwd(h, Ln, ldn, Nn, zrow, h->alpha.as<double>(), h->Linv.as<double>()));
+  CKR(check_finite_async(h, h->alpha.as<double>(), 1, Nn, 1, FLAG_ALPHA));
   span_close(h, solve);
   span_close(h, total);
 

@@ -791,7 +791,7 @@ __global__ void state_pack_kernel(StatePackView v, long long offset, long long c
 
 // finite check: *flag |= 1 for any non-finite in x (rows x cols, ld)
 __global__ void finite_check_kernel(const double* __restrict__ x, long long ld, long long rows, int cols,
-                                    int* __restrict__ flag) {
+                                    int* __restrict__ flag, int bit) {
   const long long total = rows * cols;
   int bad = 0;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
@@ -800,7 +800,7 @@ __global__ void finite_check_kernel(const double* __restrict__ x, long long ld, 
     const int c = (int)(i - r * cols);
     if (!isfinite(x[r * ld + c])) bad = 1;
   }
-  if (bad) atomicOr(flag, 1);
+  if (bad) atomicOr(flag, bit);
 }
 
 // Register-resident DMMA issue-rate microbenchmark: 8 warps per CTA, 16 independent accumulators.

@@ -4,7 +4,10 @@
 // sm_100a has no FP64 tcgen05 kind; its FP64 tensor path (DMMA) peaks at 37 TFLOP/s while kind::i8 runs ~120x the
 // MAC rate.  Every row of both operands is therefore written as
 //        a[k] = 2^(e-6) * sum_p d_p[k] 2^(-7p),   d_p[k] integer, |d_p[k]| <= 64   (one exponent e per row)
-// (slice_rows_kernel; the digits are exact: each step subtracts the rounded value and rescales by 128).  The
+// (slice_rows_kernel; the digits are exact: each step subtracts the rounded value and rescales by 128).  Every finite
+// row is covered, down to a largest magnitude of 2^-1074: the kernel keeps the integer exponent e of each row, scales
+// the row up by two power-of-two factors (2^(6-e) alone overflows for e < -1017) and the epilogue applies both rows'
+// exponents at once, V = S 2^(ea+eb-12) rounded once (sl_ldexp), so no scale 2^(e-6) has to be a double.  The
 // product of two digit planes is an exact int32 GEMM (|sum| <= (g+1) * 2^12 * K < 2^31 for K <= 65536), planes with
 // the same p + q = g share the scale 2^(-7g), and keeping the groups g < s gives V to 2^(-7s) of
 // |row a|_max |row b|_max K -- s = 7: posterior variance within 1e-8 of the FP64 path at cond 1e7
@@ -55,8 +58,8 @@ struct SlicedParams {
   int row_tiles, col_tiles;
   int tri;                 // W lower triangular: column tile j needs K < 256 (j + 1) only
   long long ra, rb;        // rows per plane in the stacked plane arrays of K_* / W
-  const double* rscale;    // [rows]  2^(e-6) of the K_* rows
-  const double* cscale;    // [N]     2^(e-6) of the W rows
+  const int* rexp;         // [rows]  exponent e of the K_* rows (the row is 2^(e-6) times its digits)
+  const int* cexp;         // [N]     exponent e of the W rows
   double* scratch;         // gridDim.x x 2 x 256 x 128 running sums
   double* vpart;           // [2 col_tiles][rows] sum over each 128-column half tile of V^2 (may be null)
   double* V;               // [rows][ldv] the product itself (diagnostics / tests)     (may be null)
@@ -69,10 +72,29 @@ struct SlicedParams {
 };
 
 // ---- digit planes ---------------------------------------------------------------------------------------------
-// One CTA per (padded) row.  planes[p][row][ldq] int8, zero outside [0, ncols) and for rows >= rows.
+__device__ __forceinline__ double sl_pow2(int n) {   // 2^n, n in [-1022, 1023]
+  return __longlong_as_double((long long)(n + 1023) << 52);
+}
+
+// x 2^n rounded once, for the folded plane sums x (0, or |x| in [2^-56, 2^32): s <= 9 groups of int32 sums in 2^-7
+// steps) and n = ea + eb - 12 anywhere in [-2158, 2036].  Inside the normal exponent range it is the one product
+// x 2^n; outside, the first factor keeps the product normal and exact (|x 2^(n+k)| >= 2^-1022) and the second rounds.
+// Below n = -1988 the first factor stops at 2^-1022, which only matters where |x 2^n| < 2^-1956: the result is 0
+// either way.
+__device__ __forceinline__ double sl_ldexp(double x, int n) {
+  if (n > 1023) return (x * sl_pow2(1023)) * sl_pow2(min(n - 1023, 1023));
+  if (n < -1022) {
+    const int k = min(-966 - n, 1022);
+    return (x * sl_pow2(max(n + k, -1022))) * sl_pow2(-k);
+  }
+  return x * sl_pow2(n);
+}
+
+// One CTA per (padded) row.  planes[p][row][ldq] int8, zero outside [0, ncols) and for rows >= rows; exp_out[row]
+// the row's exponent e (|a| < 2^e; 0 for a zero row).
 __global__ void __launch_bounds__(SL_SLICE_THREADS)
 slice_rows_kernel(const double* __restrict__ A, long long lda, int rows, int ncols, int tri, int s,
-                  int8_t* __restrict__ planes, long long plane_stride, int ldq, double* __restrict__ scale_out) {
+                  int8_t* __restrict__ planes, long long plane_stride, int ldq, int* __restrict__ exp_out) {
   __shared__ double red[SL_SLICE_THREADS / 32];
   __shared__ int e_sh;
   const int row = blockIdx.x;
@@ -91,15 +113,17 @@ slice_rows_kernel(const double* __restrict__ A, long long lda, int rows, int nco
     int e = 0;
     if (m > 0.0) (void)frexp(m, &e);          // m = f 2^e, f in [0.5, 1)  =>  |a| 2^(6-e) < 64
     e_sh = e;
-    if (row < rows) scale_out[row] = ldexp(1.0, e - 6);
+    if (row < rows) exp_out[row] = e;
   }
   __syncthreads();
-  const double up = ldexp(1.0, 6 - e_sh);
+  // |a| 2^(6-e) < 64 in two exact steps: 2^(6-e) is not a double for e < -1017 (e >= -1073, so the second is <= 2^56)
+  const int k = 6 - e_sh;
+  const double up = sl_pow2(min(k, 1023)), up2 = sl_pow2(max(k - 1023, 0));
   int8_t* out = planes + (long long)row * ldq;
   for (int c0 = threadIdx.x * 4; c0 < ldq; c0 += SL_SLICE_THREADS * 4) {
     double t[4];
 #pragma unroll
-    for (int j = 0; j < 4; ++j) t[j] = (c0 + j < nc) ? a[c0 + j] * up : 0.0;
+    for (int j = 0; j < 4; ++j) t[j] = (c0 + j < nc) ? a[c0 + j] * up * up2 : 0.0;
     for (int p = 0; p < s; ++p) {
       uint32_t w = 0;
 #pragma unroll
@@ -303,7 +327,7 @@ sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         const bool first = (g == p.s - 1);
         for (int h = 0; h < ntile; ++h) {
           const int grow = (t.ip * SL_RT + h) * SL_BM + row;
-          const double rs = (grow < p.rows) ? p.rscale[grow] : 0.0;
+          const int re = (grow < p.rows) ? p.rexp[grow] - 12 : 0;
           const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + h * SL_BN + half * (SL_BN / 2);
           double* sch = sc + (h * SL_BN + half * (SL_BN / 2)) * SL_BM;
           for (int c0 = 0; c0 < SL_BN / 2; c0 += 32) {
@@ -322,7 +346,7 @@ sliced_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                 const int col = t.jt * SL_BN + half * (SL_BN / 2) + c0 + j;
                 const double c = (double)(int)r[j];
                 const double sv = first ? c : fma(sch[(c0 + j) * SL_BM], 0.0078125, c);
-                const double v = (col < p.N) ? sv * rs * __ldg(p.cscale + col) : 0.0;
+                const double v = (col < p.N && grow < p.rows) ? sl_ldexp(sv, re + __ldg(p.cexp + col)) : 0.0;
                 sum[h] = fma(v, v, sum[h]);
                 if (p.V && grow < p.rows && col < p.N) p.V[(long long)grow * p.ldv + col] = v;
               }

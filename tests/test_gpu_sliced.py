@@ -21,6 +21,8 @@ def lib():
 
 
 def _split_rows(a, s, tri=False):
+    """Digit planes of the rows of ``a`` and their exponents e (|row| < 2^e, 0 for a zero row): the scale-up by 2^(6-e)
+    is exact for every finite row, down to the smallest subnormal (np.ldexp does not form 2^(6-e) on its own)."""
     a = np.tril(a) if tri else a
     amax = np.max(np.abs(a), axis=1)
     _, e = np.frexp(amax)
@@ -36,7 +38,8 @@ def _split_rows(a, s, tri=False):
 
 def _digit_restatement(a, b, s, tri, skip_weak=False):
     """What sliced_gemm_kernel computes, in numpy: exact integer plane products (FP64 matmuls of small integers),
-    groups p + q = g folded by Horner in 2^-7, two row scales.  ``skip_weak``: without the pair (s-1, 0), as the
+    groups p + q = g folded by Horner in 2^-7, both row exponents applied at once (one rounding, also where the
+    product or a row scale 2^(e-6) leaves the normal range).  ``skip_weak``: without the pair (s-1, 0), as the
     variance path runs it."""
     pa, ea = _split_rows(a, s)
     pb, eb = _split_rows(b, s, tri)
@@ -46,17 +49,45 @@ def _digit_restatement(a, b, s, tri, skip_weak=False):
         c = sum(pa[p] @ pb[g - p].T for p in range(last + 1))
         assert np.max(np.abs(c)) < 2 ** 31
         acc = c if acc is None else acc * 0.0078125 + c
-    return acc * np.ldexp(1.0, ea - 6)[:, None] * np.ldexp(1.0, eb - 6)[None, :]
+    return np.ldexp(acc, ea[:, None] + eb[None, :] - 12)
 
 
-@pytest.mark.parametrize("m,k,n,tri,s", [(128, 128, 256, False, 1), (200, 300, 500, False, 7), (1, 40, 3, False, 6),
-                                         (515, 1280, 1280, True, 7), (2500, 2304, 2304, True, 9), (300, 4096, 700, False, 5)])
-def test_sliced_product_is_bit_exact_against_the_digit_restatement(lib, m, k, n, tri, s):
+# largest magnitudes of the rows placed at the bottom of the range: 2^-1017 is the last exponent whose scale-up 2^(6-e)
+# is a double, 2^-1068 the last whose row scale 2^(e-6) is, 2^-1074 the smallest subnormal
+TINY_ROWS = (-1017, -1018, -1030, -1068, -1070, -1074)
+
+
+def _set_tiny_rows(x, rng, first):
+    """Rows first.. of x get largest magnitude exactly 2^E for E in TINY_ROWS (signed entries, some exact zeros)."""
+    for i, e in enumerate(TINY_ROWS):
+        u = rng.uniform(-1.0, 1.0, size=x.shape[1])
+        u[rng.random(x.shape[1]) < 0.1] = 0.0
+        u[i % x.shape[1]] = -1.0 if i % 2 else 1.0
+        x[first + i] = np.ldexp(u, e)
+
+
+@pytest.mark.parametrize("m,k,n,tri,s,tiny", [
+    pytest.param(128, 128, 256, False, 1, False, id="128-128-256-False-1"),
+    pytest.param(200, 300, 500, False, 7, False, id="200-300-500-False-7"),
+    pytest.param(1, 40, 3, False, 6, False, id="1-40-3-False-6"),
+    pytest.param(515, 1280, 1280, True, 7, False, id="515-1280-1280-True-7"),
+    pytest.param(2500, 2304, 2304, True, 9, False, id="2500-2304-2304-True-9"),
+    pytest.param(300, 4096, 700, False, 5, False, id="300-4096-700-False-5"),
+    # rows of A (and of B when it is rectangular) whose largest magnitude is 2^-1017 .. 2^-1074, among normal rows
+    pytest.param(200, 300, 500, False, 7, True, id="200-300-500-False-7-subnormal_rows"),
+    pytest.param(515, 1280, 1280, True, 7, True, id="515-1280-1280-True-7-subnormal_rows"),
+    pytest.param(300, 700, 260, False, 9, True, id="300-700-260-False-9-subnormal_rows"),
+])
+def test_sliced_product_is_bit_exact_against_the_digit_restatement(lib, m, k, n, tri, s, tiny):
     rng = np.random.default_rng(m + n + s)
     a = rng.normal(size=(m, k)) * np.exp(3 * rng.normal(size=(m, 1)))       # row scales over ~10 decades
     b = rng.normal(size=(n, k)) * np.exp(3 * rng.normal(size=(n, 1)))
     if m > 100:
         a[7] = 0.0                                                            # an all-zero row: exponent 0, digits 0
+    if tiny:
+        _set_tiny_rows(a, rng, 20)
+        if not tri:
+            _set_tiny_rows(b, rng, 30)
     if tri:
         b = np.tril(b)
     h = lib.Handle()
@@ -65,8 +96,14 @@ def test_sliced_product_is_bit_exact_against_the_digit_restatement(lib, m, k, n,
     assert np.array_equal(v, ref)
     assert np.allclose(rowsq, np.einsum("ij,ij->i", v, v), rtol=1e-13, atol=0)
     if s >= 7:      # and the digits carry the product: error relative to |row a|max |row b|max K
-        scale = np.max(np.abs(a), axis=1)[:, None] * np.max(np.abs(b), axis=1)[None, :] * k + 1e-300
-        assert np.max(np.abs(v - a @ b.T) / scale) < 2.0 ** (-7 * s + 8)
+        # (the exact product of the rows brought to [0.5, 1) by their exponents, where V is a normal double)
+        _, ea = np.frexp(np.max(np.abs(a), axis=1))
+        _, eb = np.frexp(np.max(np.abs(np.tril(b) if tri else b), axis=1))
+        an, bn = np.ldexp(a, -ea[:, None]), np.ldexp(b, -eb[:, None])
+        scale = np.max(np.abs(an), axis=1)[:, None] * np.max(np.abs(bn), axis=1)[None, :] * k + 1e-300
+        normal = np.abs(v) >= np.finfo(np.float64).tiny
+        err = np.abs(np.ldexp(v, -(ea[:, None] + eb[None, :])) - an @ bn.T) / scale
+        assert np.max(np.where(normal, err, 0.0)) < 2.0 ** (-7 * s + 8)
     v2 = h.sliced_product(a, b, slices=s, lower=tri)
     assert np.array_equal(v, v2)
     h.close()
